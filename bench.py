@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the path-tracing hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload C2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload C2] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one full render of the workload (default BASELINE.json configs[1]: Cornell box
@@ -19,6 +19,8 @@ Rank 0 prints ONE JSON line (contract in the task statement):
             threads (row strips, nproc-1 threads), on a bounded sample
 
 `--impl reference` times that CPU port alone, on the same workload/metric (rank 0 only).
+`--dump-outputs DIR` writes the image and statistics of the last timed step as .npy files (dump_outputs): the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree (it may be read-only)
 
 WORKLOADS = {
     # BASELINE.json configs (SURVEY.md §8d for the concrete inputs)
@@ -101,13 +104,14 @@ def executed_events(workload, ropts, spp):
         "print(json.dumps({'paths': st.samples['total'], 'rays': st.rays, 'node_visits': st.nodeVisits, 'prim_tests': st.primTests}))\n"
     )
     try:
-        r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, RT_B200_LIB=lib), capture_output=True, text=True, timeout=600)
+        r = subprocess.run([sys.executable, "-B", "-c", code], env=dict(os.environ, RT_B200_LIB=lib), capture_output=True, text=True, timeout=600)
         return json.loads(r.stdout.strip().splitlines()[-1])
     except Exception:
         return None
 
 
 ORACLE_BUILD = None
+ORACLE_BUILD_DIR = None  # temporary directory of the host-tuned oracle build, removed when the process ends
 
 
 def cpu_reference_run(sd, opts, target_seconds, threads):
@@ -121,9 +125,12 @@ def cpu_reference_run(sd, opts, target_seconds, threads):
     import oracle_binding
     from oracle_binding import OracleCamera
 
-    global ORACLE_BUILD
+    global ORACLE_BUILD, ORACLE_BUILD_DIR
     if ORACLE_BUILD is None:  # first use: the host-tuned build (-O3 -march=native, made on this host), else the portable one
-        native = None if os.environ.get("RT_ORACLE_LIB") else oracle_binding.build_native_oracle()
+        native = None
+        if not os.environ.get("RT_ORACLE_LIB"):
+            ORACLE_BUILD_DIR = tempfile.TemporaryDirectory(prefix="rt_oracle_")  # never into the tree: it may be read-only
+            native = oracle_binding.build_native_oracle(ORACLE_BUILD_DIR.name)
         if native:
             os.environ["RT_ORACLE_LIB"] = native
         ORACLE_BUILD = "-O3 -march=native, built on this host" if (native or os.environ.get("RT_ORACLE_LIB")) else "-O3 (portable build)"
@@ -224,6 +231,29 @@ def measured_traffic(workload, world, overridden):
     return t.get("dram_bytes_total")
 
 
+DUMP_BYTES = 64_000_000  # what --dump-outputs may write in all, shared by the workloads of the run
+
+
+def dump_outputs(out_dir, workload, rgb8, stats, budget):
+    """Writes DIR/<workload>_<name>.npy: `image`, the RGB8 framebuffer (H, W, 3) as float32, and `stats`, float64
+    [pixels, samples_total, samples_min, samples_max, bounces_total, bounces_min, bounces_max, rays] (rt_stats order).
+    An image whose float32 copy does not fit `budget` is stored as `image_sample` (n, 3) float32 of the pixels at
+    `image_sample_index` (flat y * W + x, ascending, float64), drawn with a fixed seed: the same pixels on every run."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    path = lambda name: os.path.join(out_dir, f"{workload}_{name}.npy")  # noqa: E731
+    budget -= 4096  # the stats array and the .npy headers
+    pixels = rgb8.reshape(-1, 3)
+    if pixels.size * 4 <= budget:
+        np.save(path("image"), rgb8.astype(np.float32))
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(len(pixels), budget // (3 * 4 + 8), replace=False))
+        np.save(path("image_sample"), pixels[idx].astype(np.float32))
+        np.save(path("image_sample_index"), idx.astype(np.float64))
+    np.save(path("stats"), np.asarray(stats, np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -238,7 +268,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-threads", type=int, default=None,
                     help="threads of the CPU port (default: host cores - 1 like the reference; 1 = the scalar figure SURVEY 8d asks for)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<workload>_<name>.npy "
+                         "(the image as float32, the render statistics as float64), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm sizes its sample from its own timings, so its output varies")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # `python bench.py --gpus N` without a launcher: become the one-process-per-GPU job the contract describes
         port = 29500 + os.getpid() % 2000
@@ -402,6 +439,17 @@ def bench_workload(args, workload, rank, world, local_rank, emit, env):
     total_ms = float(t.item())
     paths_per_step, rays_per_step = int(sums[1].item()), int(sums[3].item())
     kernel_launches_per_step = int(st_local.kernel_launches)
+    if args.dump_outputs:  # the image and statistics of the last timed step, outside every timed region
+        if world > 1:
+            torch.cuda.synchronize()
+            if peer_writes:
+                dist.barrier()                                     # every rank's pixels are in rank 0's framebuffer
+            else:
+                gather_owned_blocks(fb)
+        if rank == 0:
+            stats = [sums[0], sums[1], mins[0], maxs[0], sums[2], mins[1], maxs[1], sums[3]]
+            dump_outputs(args.dump_outputs, workload, fb.cpu().numpy(), [int(x.item()) for x in stats],
+                         DUMP_BYTES // len(args.workload.split(",")))
 
     # ---- end-to-end through the public API, host buffers, every step: flatten + build + H2D +
     #      render + gather + D2H ----

@@ -38,15 +38,18 @@ def build_oracle() -> str:
     return so
 
 
-def build_native_oracle() -> Optional[str]:
-    """`make native`: the oracle compiled with -march=native ON THIS HOST (bench.py's CPU baseline, BASELINE.md section 3).
+def build_native_oracle(out_dir: str) -> Optional[str]:
+    """`make native`: the oracle compiled with -march=native ON THIS HOST (bench.py's CPU baseline, BASELINE.md section 3),
+    written to `out_dir` so that the tree itself may be read-only.
     None when there is no compiler here or the build fails; the portable build is used then."""
     d = os.path.join(ROOT, "oracle")
+    out_dir = os.path.abspath(out_dir)
     try:
-        subprocess.check_call(["make", "-C", d, "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=300)
+        subprocess.check_call(["make", "-C", d, "native", f"NATIVE_DIR={out_dir}"], stdout=subprocess.DEVNULL,
+                              stderr=subprocess.DEVNULL, timeout=300)
     except Exception:
         return None
-    so = os.path.join(d, "_native", "liboracle.so")
+    so = os.path.join(out_dir, "liboracle.so")
     return so if os.path.exists(so) else None
 
 

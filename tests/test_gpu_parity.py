@@ -294,6 +294,25 @@ def test_render_is_deterministic_and_seeded(gpu):
     assert not np.array_equal(a["linear"], c["linear"])
 
 
+def test_bench_dump_outputs_are_what_the_public_api_renders(gpu, tmp_path):
+    """bench.py --dump-outputs writes the framebuffer and statistics of its last timed step: the image and the statistics
+    Camera.render gives for the same workload and options, after exactly --steps timed steps."""
+    import subprocess
+    import sys
+
+    bench = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
+    cmd = [sys.executable, bench, "--steps", "2", "--warmup", "1", "--samples", "16", "--width", "96", "--no-cpu-baseline",
+           "--dump-outputs", str(tmp_path)]
+    out = subprocess.run(cmd, stdout=subprocess.PIPE, timeout=600, check=True).stdout.decode()
+    line = json.loads(out.strip().splitlines()[-1])
+    assert line["steps"] == 2 and len(line["step_ms"]) == 2
+    g = gpu_render(SCENES["C2-cornell"](), {"width": 96, "samples": 16, "aTolerance": 0})
+    assert np.array_equal(np.load(tmp_path / "C2_image.npy"), g["rgb8"].astype(np.float32))
+    s = g["stats"]
+    assert np.load(tmp_path / "C2_stats.npy").tolist() == [s.pixels, s.samples["total"], s.samples["min"], s.samples["max"],
+                                                          s.bounces["total"], s.bounces["min"], s.bounces["max"], s.rays]
+
+
 def test_region_writes_only_region_pixels(gpu):  # camera.ts:388-431, camera.test.ts:381-396
     sd = SCENES["C2-cornell"]()
     opts = {"width": 80, "samples": 4, "aTolerance": 0, "seed": 3}

@@ -262,7 +262,7 @@ sums = torch.tensor([int(tile_owner_mask(W, H, rank, world).sum()), 10 * (rank +
 mins = torch.tensor([rank + 3], dtype=torch.int64); maxs = torch.tensor([rank + 7], dtype=torch.int64)
 merge_stats(sums, mins, maxs)
 from mcp_raytracer_b200.distributed import SharedFramebuffer
-shared = SharedFramebuffer(W, H, device=0)     # no GPU here: creation fails on rank 0 and EVERY rank learns to fall back
+shared = SharedFramebuffer(W, H, device=0)     # no visible GPU: creation fails on rank 0 and EVERY rank learns to fall back
 assert shared.ok is False and shared.ptr == 0
 shared.close()
 if rank == 0:
@@ -291,10 +291,34 @@ def test_bench_reference_arm_prints_one_contract_line():
         assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
 
 
+def test_bench_dump_outputs_fit_the_budget_and_are_deterministic(tmp_path):
+    """bench.dump_outputs: the whole image when its float32 copy fits, else the same seeded sample of pixels on every run."""
+    import bench
+
+    rng = np.random.default_rng(1)
+    small = rng.integers(0, 256, (30, 40, 3), dtype=np.uint8)
+    bench.dump_outputs(str(tmp_path / "a"), "C2", small, [1200, 4800, 4, 4, 9000, 1, 7, 13800], 64_000_000)
+    assert np.array_equal(np.load(tmp_path / "a" / "C2_image.npy"), small.astype(np.float32))
+    st = np.load(tmp_path / "a" / "C2_stats.npy")
+    assert st.dtype == np.float64 and st.tolist() == [1200, 4800, 4, 4, 9000, 1, 7, 13800]
+    big = rng.integers(0, 256, (300, 400, 3), dtype=np.uint8)
+    budget = 300 * 400 * 3 * 4 // 2
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), "C4", big, [0] * 8, budget)
+        assert sum(f.stat().st_size for f in (tmp_path / d).iterdir()) <= budget
+        assert not (tmp_path / d / "C4_image.npy").exists()
+    idx = np.load(tmp_path / "b" / "C4_image_sample_index.npy")
+    sample = np.load(tmp_path / "b" / "C4_image_sample.npy")
+    assert idx.dtype == np.float64 and sample.dtype == np.float32 and len(idx) > 10000 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(sample, big.reshape(-1, 3)[idx.astype(np.int64)].astype(np.float32))
+    assert np.array_equal(idx, np.load(tmp_path / "c" / "C4_image_sample_index.npy"))
+
+
 def test_gloo_world_size_2_gather_and_stats(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text(_WORKER)
-    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT="29613", WORLD_SIZE="2")
+    # the workers see no CUDA device, also on a GPU machine: the fallback of SharedFramebuffer is what they check
+    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT="29613", WORLD_SIZE="2", CUDA_VISIBLE_DEVICES="")
     procs = [subprocess.Popen([sys.executable, str(script), ROOT], env=dict(env, RANK=str(r)), stdout=subprocess.PIPE,
                               stderr=subprocess.STDOUT) for r in range(2)]
     outs = [p.communicate(timeout=180)[0].decode() for p in procs]
