@@ -252,6 +252,39 @@ rt_status rt_camera_render_progressive(rt_camera* cam, const rt_region* region, 
 rt_status rt_camera_trace_primary(rt_camera* cam, const rt_region* region, int32_t* obj_id,
                                   float* t, float* normal, uint8_t* front_face);
 
+/* ---- opt-in denoiser (not in the reference) ----
+ * The spatial filter of SVGF (Schied et al., HPG 2017) without its temporal part, guided by first-hit feature buffers: the
+ * colour is demodulated by the feature albedo, filtered by `iterations` a-trous passes (step 2^k, 5x5 B3-spline taps) whose
+ * weights stop at normal, depth and luminance edges (the luminance stop scaled by the per-pixel variance of the render's
+ * moments), and remodulated.  FP32; the filter reads only pixels inside the region.  tests/denoise_reference.py is its
+ * specification.  rt_denoise_opts: iterations 0..8 are taken as given (0 = demodulate and remodulate only); a sigma of 0
+ * selects its default (luminance 4, normal 128, depth 1); opts == NULL = all defaults (5 iterations). */
+typedef struct rt_denoise_opts {
+  int32_t iterations;
+  float sigma_luminance, sigma_normal, sigma_depth;
+} rt_denoise_opts;
+
+/* First-hit features averaged over the camera rays of samples 0..n_samples-1 (n_samples >= 1) — the rays the render kernels
+ * draw for those samples (jitter when samples > 1, defocus when the aperture is open).  HOST outputs, each optional, only
+ * region pixels written: albedo [H][W][3] (the root material's feature albedo: Lambert / Metal colour, 1 for Glass and
+ * Light, Mixed = weighted mean of its children, Layered = its inner material; 1 on a miss), normal [H][W][3] (mean of the
+ * face-forwarded normals, renormalised when more than one ray hit; 0 when none did), depth [H][W] (mean Euclidean hit
+ * distance over the rays that hit, -1 when none did).  Synchronous. */
+rt_status rt_camera_render_features(rt_camera* cam, const rt_region* region, int32_t n_samples,
+                                    float* albedo, float* normal, float* depth);
+/* The filter on explicit HOST inputs [H][W][...] of one whole image (width x height): colour [3], albedo [3], normal [3],
+ * depth [1] as rt_camera_render_features writes them, moments [8] as rt_camera_render_moments writes them; out [H][W][3]
+ * must not alias an input.  A pixel whose inputs are not finite is passed through unchanged and is no neighbour's tap.
+ * device -1 = current.  Synchronous. */
+rt_status rt_denoise(int32_t device, int32_t width, int32_t height, const float* color, const float* albedo, const float* normal,
+                     const float* depth, const float* moments, const rt_denoise_opts* opts, float* out);
+/* Render with moments, features of the first min(samples, 8) samples, and the filter, all on the device; one copy back.
+ * rgb8 / linear_rgb as rt_camera_render_region (the filtered image).  stats = the render's, except device_ms and
+ * kernel_launches, which cover every kernel of the call.  RT_ERR_UNSUPPORTED for partitioned cameras (part_count > 1) and
+ * render modes other than RT_MODE_DEFAULT.  Synchronous. */
+rt_status rt_camera_render_denoised(rt_camera* cam, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear_rgb,
+                                    const rt_denoise_opts* opts, rt_stats* stats);
+
 /* ---- one process, N GPUs: replaces the worker pool of generateImageBuffer(parallel: true)
  *      (src/raytracer.ts:60-90: N worker_threads over row strips of a SharedArrayBuffer, RenderStats.merge) ----
  * The scene is compiled once and uploaded to `n_devices` GPUs (devices == NULL: ordinals 0..n-1; n_devices <= 0:

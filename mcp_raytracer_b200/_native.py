@@ -10,7 +10,7 @@ import os
 import subprocess
 from typing import Optional
 
-from .scene_data import rt_camera_info, rt_region, rt_render_opts, rt_scene_desc, rt_stats
+from .scene_data import rt_camera_info, rt_denoise_opts, rt_region, rt_render_opts, rt_scene_desc, rt_stats
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
@@ -25,6 +25,7 @@ EXPORTS = [
     "rt_multi_create", "rt_multi_destroy", "rt_multi_get_info", "rt_multi_render_region",
     "rt_shared_buffer_create", "rt_shared_buffer_open", "rt_shared_buffer_release",
     "rt_debug_scatter", "rt_debug_get_ray", "rt_debug_light_pdf", "rt_debug_light_random_vec", "rt_debug_diffuse_bounce",
+    "rt_camera_render_features", "rt_denoise", "rt_camera_render_denoised",
 ]
 
 STATUS_NAMES = {
@@ -90,6 +91,9 @@ def lib() -> C.CDLL:
     L.rt_debug_light_pdf.argtypes = [vp, i32, i32, vp, vp, vp]
     L.rt_debug_light_random_vec.argtypes = [vp, i32, i32, vp, vp, vp]
     L.rt_debug_diffuse_bounce.argtypes = [vp, i32, vp, vp, vp, vp]
+    L.rt_camera_render_features.argtypes = [vp, C.POINTER(rt_region), i32, vp, vp, vp]
+    L.rt_denoise.argtypes = [i32, i32, i32, vp, vp, vp, vp, vp, C.POINTER(rt_denoise_opts), vp]
+    L.rt_camera_render_denoised.argtypes = [vp, C.POINTER(rt_region), vp, C.c_size_t, vp, C.POINTER(rt_denoise_opts), C.POINTER(rt_stats)]
     _lib = L
     return L
 

@@ -23,7 +23,7 @@ import numpy as np
 
 from . import _native
 from .scene_data import (
-    FlatScene, RaytracerError, merge_render_options, render_opts_struct, rt_camera_info, rt_region, rt_stats,
+    FlatScene, RaytracerError, denoise_opts_struct, merge_render_options, render_opts_struct, rt_camera_info, rt_region, rt_stats,
 )
 from .scenes import generateSceneData
 
@@ -236,6 +236,35 @@ class Camera:
                                                           nrm.ctypes.data, ff.ctypes.data))
         return ids, t, nrm, ff
 
+    # -- opt-in denoiser (not in the reference) --
+    def renderFeatures(self, nSamples: int, region: Optional[Dict[str, int]] = None) -> Dict[str, np.ndarray]:
+        """First-hit features averaged over the camera rays of samples 0..nSamples-1 (rt_camera_render_features):
+        albedo [H,W,3], normal [H,W,3], depth [H,W] (-1 where no ray hit).  Pixels outside `region` are 0."""
+        W, H = self.imageWidth, self.imageHeight
+        reg = _region_struct(region, W, H)
+        alb = np.zeros((H, W, 3), np.float32)
+        nrm = np.zeros((H, W, 3), np.float32)
+        dep = np.zeros((H, W), np.float32)
+        self._check(_native.lib().rt_camera_render_features(self._h, C.byref(reg), int(nSamples), alb.ctypes.data, nrm.ctypes.data,
+                                                            dep.ctypes.data))
+        return {"albedo": alb, "normal": nrm, "depth": dep}
+
+    def renderDenoised(self, pixelData: Optional[np.ndarray], linear: Optional[np.ndarray] = None, region: Optional[Dict[str, int]] = None,
+                       options: Optional[Dict[str, Any]] = None) -> RenderStats:
+        """Render, then denoise on the device (rt_camera_render_denoised): `pixelData` / `linear` receive the filtered image.
+        options: {iterations, sigmaLuminance, sigmaNormal, sigmaDepth}; absent = defaults."""
+        W, H = self.imageWidth, self.imageHeight
+        if pixelData is not None and (pixelData.dtype != np.uint8 or not pixelData.flags["C_CONTIGUOUS"]):
+            raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
+        if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3 or not linear.flags["C_CONTIGUOUS"]):
+            raise RaytracerError("linear buffer must be float32 [H][W][3]")
+        reg = _region_struct(region, W, H)
+        opts = denoise_opts_struct(options)
+        st = rt_stats()
+        self._check(_native.lib().rt_camera_render_denoised(
+            self._h, C.byref(reg), pixelData.ctypes.data if pixelData is not None else None, pixelData.nbytes if pixelData is not None else 0,
+            linear.ctypes.data if linear is not None else None, C.byref(opts), C.byref(st)))
+        return RenderStats.from_struct(st)
 
     # -- per-function parity hooks (rt_debug_*): one device function of the render path on explicit inputs --
     DEBUG_UNIFORMS = 16
@@ -363,6 +392,28 @@ def createCameraFromSceneData(sceneData: Dict[str, Any], renderOptions: Optional
 def generateScene(sceneConfig: Dict[str, Any]) -> Camera:
     """src/scenes/scenes.ts:52-55"""
     return createCameraFromSceneData(generateSceneData(sceneConfig), sceneConfig.get("render"))
+
+
+def denoise(color, albedo, normal, depth, moments, options: Optional[Dict[str, Any]] = None, device: int = -1) -> np.ndarray:
+    """The denoiser on explicit arrays (rt_denoise): color/albedo/normal [H,W,3], depth [H,W], moments [H,W,8] as
+    `Camera.renderRegion(..., moments=)` and `Camera.renderFeatures` return them.  Returns the filtered colour [H,W,3]."""
+    c = np.ascontiguousarray(color, np.float32)
+    if c.ndim != 3 or c.shape[2] != 3:
+        raise RaytracerError("color must be [H][W][3]")
+    H, W = c.shape[:2]
+    shapes = {"albedo": (H, W, 3), "normal": (H, W, 3), "depth": (H, W), "moments": (H, W, 8)}
+    arrs = {}
+    for name, a in (("albedo", albedo), ("normal", normal), ("depth", depth), ("moments", moments)):
+        arrs[name] = np.ascontiguousarray(a, np.float32)
+        if arrs[name].shape != shapes[name]:
+            raise RaytracerError(f"{name} must have shape {shapes[name]}, not {arrs[name].shape}")
+    opts = denoise_opts_struct(options)
+    out = np.zeros((H, W, 3), np.float32)
+    st = _native.lib().rt_denoise(int(device), W, H, c.ctypes.data, arrs["albedo"].ctypes.data, arrs["normal"].ctypes.data,
+                                  arrs["depth"].ctypes.data, arrs["moments"].ctypes.data, C.byref(opts), out.ctypes.data)
+    if st != 0:
+        raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
+    return out
 
 
 def measureFp32Peak(device: int = -1):

@@ -29,6 +29,9 @@ int render_adaptive_blocks(const DevScene& S, const RenderParams& R, int sms, in
 cudaError_t launch_trace_primary(const DevScene& S, const RenderParams& R, int* obj_id, float* t, float* normal,
                                  uint8_t* front, cudaStream_t st);
 cudaError_t launch_fp32_peak(float* out, int blocks, int iters, cudaStream_t st);
+cudaError_t launch_render_features(const DevScene& S, const RenderParams& R, int n_samples, float* albedo, float* normal, float* depth,
+                                   cudaStream_t st);
+cudaError_t launch_denoise(const DenoiseParams& D, cudaStream_t st, int* launches);
 cudaError_t launch_render_wavefront(const DevScene& S, const RenderParams& R, WfHost& H, int sms, cudaStream_t st, int* launches);
 cudaError_t launch_finalize_stats(const unsigned long long* raw, rt_stats* out, int launches, cudaStream_t st);
 // per-function parity hooks (rt_debug.cuh)
@@ -172,6 +175,10 @@ struct rt_camera {
   float* d_t = nullptr;
   float* d_normal = nullptr;
   uint8_t* d_front = nullptr;
+  float* d_falb = nullptr;   // feature buffers (rt_camera_render_features)
+  float* d_fnrm = nullptr;
+  float* d_fdepth = nullptr;
+  float* d_dn = nullptr;     // denoiser scratch: dn_floats_per_pixel floats per pixel
   unsigned long long* d_stats = nullptr;
   // work queue of the render kernel: [0] = next item, [1..] = finished chunks per tile
   int* d_queue = nullptr;
@@ -219,7 +226,8 @@ static void free_camera(rt_camera* c) {
   cudaStreamSynchronize(c->stream); // the blocks go back to the cache: nothing of this camera may still be in flight
   for (void* p : c->allocs) dev_free(p);
   dev_free(c->d_rgb8); dev_free(c->d_linear); dev_free(c->d_moments); dev_free(c->d_ids);
-  dev_free(c->d_t); dev_free(c->d_normal); dev_free(c->d_front); dev_free(c->d_stats); dev_free(c->d_queue); dev_free(c->d_scratch); dev_free(c->d_pixstate); dev_free(c->d_adrec);
+  dev_free(c->d_t); dev_free(c->d_normal); dev_free(c->d_front); dev_free(c->d_falb); dev_free(c->d_fnrm); dev_free(c->d_fdepth);
+  dev_free(c->d_dn); dev_free(c->d_stats); dev_free(c->d_queue); dev_free(c->d_scratch); dev_free(c->d_pixstate); dev_free(c->d_adrec);
   wf_release(c);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -438,7 +446,7 @@ static rt_status camera_from_host(std::shared_ptr<HostScene> hs, const rt_render
   UP(c->hs->p0, &d.p0); UP(c->hs->p1, &d.p1); UP(c->hs->p2, &d.p2); UP(c->hs->p3, &d.p3);
   UP(c->hs->slot_info, &d.slot_info); UP(c->hs->exact, &d.exact);
   UP(c->hs->matA, &d.matA); UP(c->hs->matB, &d.matB); UP(c->hs->matE, &d.matE);
-  UP(c->hs->lights, &d.lights);
+  UP(c->hs->lights, &d.lights); UP(c->hs->matF, &d.matF);
 #undef UP
   d.n_nodes = (int)c->hs->nodes.size();
   d.n_slots = (int)c->hs->p0.size();
@@ -916,6 +924,171 @@ rt_status rt_camera_trace_primary(rt_camera* c, const rt_region* region, int32_t
   }
   CU(cudaStreamSynchronize(c->stream));
   return RT_OK;
+}
+
+// ---- denoiser (rt_denoise.cuh) ----
+// Scratch of the filter per pixel: two (colour, variance) ping-pong float4, the (normal, depth) float4, the depth gradient.
+static const size_t kDnFloatsPerPixel = 14;
+static void dn_scratch(DenoiseParams& D, float* base, size_t npx) {
+  D.buf[0] = reinterpret_cast<F4*>(base);
+  D.buf[1] = reinterpret_cast<F4*>(base + npx * 4);
+  D.feat = reinterpret_cast<F4*>(base + npx * 8);
+  D.grad = base + npx * 12;
+}
+// rt_denoise_opts -> filter constants (NULL = all defaults; a zero sigma = its default; iterations are taken as given)
+static rt_status dn_options(const rt_denoise_opts* o, DenoiseParams& D) {
+  const rt_denoise_opts defaults{5, 0.f, 0.f, 0.f};
+  if (!o) o = &defaults;
+  if (o->iterations < 0 || o->iterations > 8) return fail(RT_ERR_INVALID_ARGUMENT, "denoise iterations must be 0..8");
+  if (!(o->sigma_luminance >= 0.f) || !(o->sigma_normal >= 0.f) || !(o->sigma_depth >= 0.f) || !std::isfinite(o->sigma_luminance) ||
+      !std::isfinite(o->sigma_normal) || !std::isfinite(o->sigma_depth))
+    return fail(RT_ERR_INVALID_ARGUMENT, "denoise sigmas must be finite and >= 0");
+  D.iterations = o->iterations;
+  D.sigma_l = o->sigma_luminance > 0.f ? o->sigma_luminance : 4.f;
+  D.sigma_n = o->sigma_normal > 0.f ? o->sigma_normal : 128.f;
+  D.sigma_z = o->sigma_depth > 0.f ? o->sigma_depth : 1.f;
+  return RT_OK;
+}
+
+static rt_status features_prepare(rt_camera* c, size_t npx) {
+  if (!c->d_falb) CU(dev_alloc(&c->d_falb, npx * 12));
+  if (!c->d_fnrm) CU(dev_alloc(&c->d_fnrm, npx * 12));
+  if (!c->d_fdepth) CU(dev_alloc(&c->d_fdepth, npx * 4));
+  return RT_OK;
+}
+
+rt_status rt_camera_render_features(rt_camera* c, const rt_region* region, int32_t n_samples, float* albedo, float* normal, float* depth) {
+  RT_GUARD_BEGIN
+  if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
+  if (n_samples < 1) return fail(RT_ERR_INVALID_ARGUMENT, "n_samples must be >= 1");
+  DeviceGuard g(c->device);
+  const int W = c->hs->image_width, H = c->hs->image_height;
+  const size_t npx = (size_t)W * H;
+  RenderParams P;
+  rt_status st = clip_region(c, region, P);
+  if (st != RT_OK) return st;
+  if ((st = features_prepare(c, npx)) != RT_OK) return st;
+  CU(launch_render_features(c->ds, P, n_samples, c->d_falb, c->d_fnrm, c->d_fdepth, c->stream));
+  const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
+  if (rw > 0 && rh > 0) {
+    const size_t off = (size_t)P.y0 * W + P.x0;
+    if (albedo) CU(cudaMemcpy2DAsync(albedo + off * 3, (size_t)W * 12, c->d_falb + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
+    if (normal) CU(cudaMemcpy2DAsync(normal + off * 3, (size_t)W * 12, c->d_fnrm + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
+    if (depth) CU(cudaMemcpy2DAsync(depth + off, (size_t)W * 4, c->d_fdepth + off, (size_t)W * 4, (size_t)rw * 4, rh, cudaMemcpyDeviceToHost, c->stream));
+  }
+  CU(cudaStreamSynchronize(c->stream));
+  return RT_OK;
+  RT_GUARD_END
+}
+
+rt_status rt_denoise(int32_t device, int32_t width, int32_t height, const float* color, const float* albedo, const float* normal,
+                     const float* depth, const float* moments, const rt_denoise_opts* opts, float* out) {
+  RT_GUARD_BEGIN
+  if (!color || !albedo || !normal || !depth || !moments || !out) return fail(RT_ERR_INVALID_ARGUMENT, "null argument");
+  if (width <= 0 || height <= 0) return fail(RT_ERR_INVALID_ARGUMENT, "width and height must be > 0");
+  DenoiseParams D{};
+  rt_status st = dn_options(opts, D);
+  if (st != RT_OK) return st;
+  const int ndev = rt_device_count();
+  if (ndev <= 0) return fail(RT_ERR_NO_DEVICE, "no CUDA device visible; this library has no CPU fallback");
+  if (device < 0) { if (cudaGetDevice(&device) != cudaSuccess) device = 0; }
+  if (device >= ndev) return fail(RT_ERR_INVALID_ARGUMENT, "device ordinal out of range");
+  DeviceGuard g(device);
+  if (!g.ok) return fail(RT_ERR_CUDA, "cudaSetDevice failed");
+  const size_t npx = (size_t)width * height;
+  struct Blocks { // back to the device cache once nothing of this call is in flight
+    float* in = nullptr;
+    float* scratch = nullptr;
+    ~Blocks() { cudaStreamSynchronize(0); dev_free(in); dev_free(scratch); }
+  } b;
+  CU(dev_alloc(&b.in, npx * 18 * sizeof(float)));
+  CU(dev_alloc(&b.scratch, npx * kDnFloatsPerPixel * sizeof(float)));
+  float* d_col = b.in;
+  float* d_alb = b.in + npx * 3;
+  float* d_nrm = b.in + npx * 6;
+  float* d_mom = b.in + npx * 9;
+  float* d_dep = b.in + npx * 17;
+  CU(cudaMemcpyAsync(d_col, color, npx * 12, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_alb, albedo, npx * 12, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_nrm, normal, npx * 12, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_mom, moments, npx * 32, cudaMemcpyHostToDevice, 0));
+  CU(cudaMemcpyAsync(d_dep, depth, npx * 4, cudaMemcpyHostToDevice, 0));
+  D.width = width;
+  D.x0 = 0; D.y0 = 0; D.x1 = width; D.y1 = height;
+  D.color = d_col; D.albedo = d_alb; D.normal = d_nrm; D.depth = d_dep; D.moments = d_mom;
+  dn_scratch(D, b.scratch, npx);
+  D.out = d_col;
+  D.rgb8 = nullptr;
+  int launches = 0;
+  CU(launch_denoise(D, 0, &launches));
+  CU(cudaMemcpyAsync(out, d_col, npx * 12, cudaMemcpyDeviceToHost, 0));
+  CU(cudaStreamSynchronize(0));
+  return RT_OK;
+  RT_GUARD_END
+}
+
+rt_status rt_camera_render_denoised(rt_camera* c, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
+                                    const rt_denoise_opts* opts, rt_stats* stats) {
+  RT_GUARD_BEGIN
+  if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
+  DenoiseParams D{};
+  rt_status st = dn_options(opts, D);
+  if (st != RT_OK) return st;
+  const int W = c->hs->image_width, H = c->hs->image_height;
+  const size_t npx = (size_t)W * H;
+  if (rgb8 && rgb8_len < npx * 3) return fail(RT_ERR_BUFFER_TOO_SMALL, "rgb8 buffer smaller than width*height*3");
+  // the filter reads the neighbours of a pixel, which other parts render; modes other than default are not radiance
+  if (c->opts.part_count > 1) return fail(RT_ERR_UNSUPPORTED, "denoised renders are not partitioned");
+  if (c->hs->cam.mode != RT_MODE_DEFAULT) return fail(RT_ERR_UNSUPPORTED, "denoised renders need the default render mode");
+  DeviceGuard g(c->device);
+  RenderParams P;
+  st = clip_region(c, region, P);
+  if (st != RT_OK) return st;
+  if (rgb8 && !c->d_rgb8) CU(dev_alloc(&c->d_rgb8, npx * 3));
+  if (!c->d_linear) CU(dev_alloc(&c->d_linear, npx * 3 * sizeof(float)));
+  if (!c->d_moments) CU(dev_alloc(&c->d_moments, npx * 8 * sizeof(float)));
+  if ((st = features_prepare(c, npx)) != RT_OK) return st;
+  if (!c->d_dn) CU(dev_alloc(&c->d_dn, npx * kDnFloatsPerPixel * sizeof(float)));
+  P.rgb8 = nullptr; // RGB8 is written from the filtered image
+  P.linear = c->d_linear;
+  P.moments = c->d_moments;
+  int launches = 0;
+  CU(cudaEventRecord(c->ev0, c->stream));
+  st = enqueue_render(c, P, nullptr, &launches);
+  if (st != RT_OK) return st;
+  const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
+  if (rw > 0 && rh > 0) {
+    const int n_feat = std::max(1, std::min(c->hs->cam.samples, 8));
+    CU(launch_render_features(c->ds, P, n_feat, c->d_falb, c->d_fnrm, c->d_fdepth, c->stream));
+    D.width = W;
+    D.x0 = P.x0; D.y0 = P.y0; D.x1 = P.x1; D.y1 = P.y1;
+    D.color = c->d_linear; D.albedo = c->d_falb; D.normal = c->d_fnrm; D.depth = c->d_fdepth; D.moments = c->d_moments;
+    dn_scratch(D, c->d_dn, npx);
+    D.out = c->d_linear;
+    D.rgb8 = rgb8 ? c->d_rgb8 : nullptr;
+    int dn_launches = 0;
+    CU(launch_denoise(D, c->stream, &dn_launches));
+    launches += 1 + dn_launches;
+  }
+  CU(cudaEventRecord(c->ev1, c->stream));
+  unsigned long long raw[kStatCount];
+  CU(cudaMemcpyAsync(raw, c->d_stats, sizeof(raw), cudaMemcpyDeviceToHost, c->stream));
+  if (rw > 0 && rh > 0) {
+    const size_t off = (size_t)P.y0 * W + P.x0;
+    if (rgb8) CU(cudaMemcpy2DAsync(rgb8 + off * 3, (size_t)W * 3, c->d_rgb8 + off * 3, (size_t)W * 3, (size_t)rw * 3, rh, cudaMemcpyDeviceToHost, c->stream));
+    if (linear) CU(cudaMemcpy2DAsync(linear + off * 3, (size_t)W * 12, c->d_linear + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
+  }
+  CU(cudaStreamSynchronize(c->stream));
+  if (stats) {
+    std::memset(stats, 0, sizeof(*stats));
+    unpack_stats(raw, stats);
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+    stats->device_ms = ms;
+    stats->kernel_launches = launches;
+  }
+  return RT_OK;
+  RT_GUARD_END
 }
 
 rt_status rt_measure_fp32_peak(int32_t device, double* tflops, double* sm_clock_mhz) {

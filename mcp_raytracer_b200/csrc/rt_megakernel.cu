@@ -351,16 +351,18 @@ RT_DEV bool path_step_shadow(const DevScene& S, const SmemList& L, const ListSme
   return path_post_shadow<KIND>(S, L, &sm, mw, ps, g, t, slot, wc);
 }
 
+// writeColorToBuffer (camera.ts:455-472) of one channel: sqrt gamma, then the Uint8ClampedArray store
+// (NaN/negative -> 0, >255 -> 255).  Shared by write_pixel and the denoiser's output (rt_denoise.cuh).
+RT_DEV uint8_t gamma_rgb8(float c) {
+  const double v = floor(255.999 * sqrt((double)c));
+  return !(v > 0.0) ? 0 : (v >= 255.0 ? 255 : (uint8_t)v);
+}
 // finalColor (camera.ts:326-340, default mode) + writeColorToBuffer (camera.ts:455-472)
 RT_DEV void write_pixel(const RenderParams& R, size_t pi, V3 fc) {
   if (R.rgb8) {
-    const float c[3] = {fc.x, fc.y, fc.z};
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-      double v = floor(255.999 * sqrt((double)c[k]));
-      // Uint8ClampedArray store: NaN/negative -> 0, >255 -> 255
-      R.rgb8[pi * 3 + k] = !(v > 0.0) ? 0 : (v >= 255.0 ? 255 : (uint8_t)v);
-    }
+    R.rgb8[pi * 3] = gamma_rgb8(fc.x);
+    R.rgb8[pi * 3 + 1] = gamma_rgb8(fc.y);
+    R.rgb8[pi * 3 + 2] = gamma_rgb8(fc.z);
   }
   if (R.linear) { R.linear[pi * 3] = fc.x; R.linear[pi * 3 + 1] = fc.y; R.linear[pi * 3 + 2] = fc.z; }
 }
@@ -2002,3 +2004,4 @@ cudaError_t launch_fp32_peak(float* out, int blocks, int iters, cudaStream_t st)
 
 #include "rt_wavefront.cuh" // the wavefront integrator shares every helper above
 #include "rt_debug.cuh"     // per-function parity hooks: the same device functions on explicit inputs
+#include "rt_denoise.cuh"   // first-hit feature buffers and the a-trous denoiser

@@ -591,7 +591,7 @@ rt_status compile_scene(const rt_scene_desc* sd, const rt_render_opts* o, HostSc
   // ---- materials (createMaterial, scenes.ts:144-199) ----
   const uint32_t nm = sd->n_materials;
   if (nm && (!sd->mat_type || !sd->mat_color || !sd->mat_param)) { err = "material arrays missing"; return RT_ERR_INVALID_ARGUMENT; }
-  S.matA.resize(nm); S.matB.resize(nm); S.matE.resize(nm);
+  S.matA.resize(nm); S.matB.resize(nm); S.matE.resize(nm); S.matF.resize(nm);
   for (uint32_t i = 0; i < nm; ++i) {
     int ty = sd->mat_type[i];
     const double* c = sd->mat_color + 3 * (size_t)i;
@@ -599,6 +599,10 @@ rt_status compile_scene(const rt_scene_desc* sd, const rt_render_opts* o, HostSc
     int c0 = sd->mat_child ? sd->mat_child[2 * i] : -1, c1 = sd->mat_child ? sd->mat_child[2 * i + 1] : -1;
     H3 col = from_d(c);
     H3 emit = map3([](int) { return 0.0; });
+    // feature albedo (the denoiser's demodulation): the colour of Lambert / Metal, 1 for Glass and Light (emission passes
+    // through unchanged), folded through Mixed / Layered exactly like the emission
+    H3 alb = ty == MAT_LAMBERT || ty == MAT_METAL ? col : map3([](int) { return 1.0; });
+    auto f3 = [&](int k) { return H3{{S.matF[k].x, S.matF[k].y, S.matF[k].z}}; };
     auto child_ok = [&](int ci) { return ci >= 0 && (uint32_t)ci < i; }; // children precede parents => acyclic
     switch (ty) {
       case MAT_LAMBERT: break;
@@ -610,6 +614,7 @@ rt_status compile_scene(const rt_scene_desc* sd, const rt_render_opts* o, HostSc
         prm = std::max(0.0, std::min(1.0, prm)); // mixedMaterial.ts:29
         H3 e1{{S.matE[c0].x, S.matE[c0].y, S.matE[c0].z}}, e2{{S.matE[c1].x, S.matE[c1].y, S.matE[c1].z}};
         emit = vsum(vtimes(e1, prm), vtimes(e2, 1.0 - prm)); // mixedMaterial.ts:52-57
+        alb = vsum(vtimes(f3(c0), prm), vtimes(f3(c1), 1.0 - prm));
         break;
       }
       case MAT_LAYERED: {
@@ -618,6 +623,7 @@ rt_status compile_scene(const rt_scene_desc* sd, const rt_render_opts* o, HostSc
         if (!child_ok(c0)) { err = "Material not found: " + std::to_string(c0); return RT_ERR_MATERIAL_NOT_FOUND; }
         prm = sd->mat_param[c1];                                        // outer ior
         emit = H3{{S.matE[c0].x, S.matE[c0].y, S.matE[c0].z}};          // layeredMaterial.ts:61-63
+        alb = f3(c0);
         break;
       }
       default: err = "Unknown material type: " + std::to_string(ty); return RT_ERR_UNKNOWN_MATERIAL_TYPE;
@@ -626,6 +632,7 @@ rt_status compile_scene(const rt_scene_desc* sd, const rt_render_opts* o, HostSc
     S.matA[i] = F4{col[0], col[1], col[2], (float)prm};
     S.matB[i] = I4{ty, c0, c1, has_e ? 1 : 0};
     S.matE[i] = F4{emit[0], emit[1], emit[2], has_e ? 1.f : 0.f};
+    S.matF[i] = F4{alb[0], alb[1], alb[2], 0.f};
   }
   lap("materials");
   // ---- objects (createSceneObject, scenes.ts:109-139) ----

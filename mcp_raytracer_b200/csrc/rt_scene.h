@@ -24,7 +24,7 @@ struct HostScene {
   std::vector<F4> p0, p1, p2, p3;
   std::vector<I2> slot_info;
   std::vector<ExactPrim> exact;
-  std::vector<F4> matA, matE;
+  std::vector<F4> matA, matE, matF;
   std::vector<I4> matB;
   std::vector<DevLight> lights;
 };

@@ -16,6 +16,7 @@
 //   matA    [n_mats]   float4              (r,g,b,param)
 //   matB    [n_mats]   int4                (type, child0, child1, has_emission)
 //   matE    [n_mats]   float4              precomputed emitted() of the subtree rooted here
+//   matF    [n_mats]   float4              feature albedo of the subtree rooted here (the denoiser demodulates by it)
 //   lights  [n_lights] DevLight
 // Slots are primitives in BVH-leaf order, so a leaf is a contiguous slot range.
 #pragma once
@@ -110,6 +111,7 @@ struct DevScene {
   const I4* matB;
   const F4* matE;
   const DevLight* lights;
+  const F4* matF;
   int n_nodes, n_slots, n_unbounded, n_mats, n_lights;
   int bvh_kind;
   int planar_any; // scene has planes/quads
@@ -193,6 +195,24 @@ struct alignas(8) PixState {
 };
 static_assert(sizeof(PixState) == 40 && offsetof(PixState, samples) == 12 && offsetof(PixState, sum_ill) == 16 && offsetof(PixState, bounces) == 32,
               "adstate_load / adstate_store (rt_megakernel.cu) move a PixState as five 64-bit words");
+// ---- denoiser (rt_denoise.cuh): one filter launch sequence over the pixels of a region ----
+// Every buffer is indexed by whole-image pixel (y * width + x); only pixels inside [x0, x1) x [y0, y1) are read or written.
+struct DenoiseParams {
+  int width;
+  int x0, y0, x1, y1;
+  const float* color;   // [H][W][3] linear colour (the pixel mean)
+  const float* albedo;  // [H][W][3] feature albedo
+  const float* normal;  // [H][W][3] feature normal (zero on a miss)
+  const float* depth;   // [H][W] feature depth (-1 on a miss)
+  const float* moments; // [H][W][8] as rt_camera_render_moments writes them
+  F4* buf[2];           // (demodulated colour, luminance variance); x = NaN marks a pixel the filter passes through
+  F4* feat;             // (normal, depth)
+  float* grad;          // [H][W][2] depth gradient
+  int iterations;
+  float sigma_l, sigma_n, sigma_z;
+  float* out;           // [H][W][3] linear result; may be `color` (both are read and written pixel by pixel)
+  uint8_t* rgb8;        // [H][W][3] or null
+};
 // ---- wavefront integrator (rt_wavefront.cuh): path pool + queues in HBM ----
 struct U2 { uint32_t x, y; };
 enum : int { WF_TAGS = 3 };

@@ -3,6 +3,7 @@ by native dispatch (the seam SURVEY.md §8b names).
 
 * `generateImageBuffer(sceneConfig, options)`  <- src/raytracer.ts:39-113
     options.parallel=False : `camera.render(pixelData)`            (raytracer.ts:56-59)
+    options.denoise=True or {iterations, sigma*}: `camera.renderDenoised(pixelData)` on one GPU (not in the reference)
     options.parallel=True  : the image is split over GPUs instead of worker threads
                              (raytracer.ts:60-90): `MultiCamera` (rt_multi_* of the C ABI) compiles
                              the scene once, every visible device renders its interleaved set of 8x4
@@ -69,7 +70,16 @@ def renderScene(sceneConfig: Dict[str, Any], options: Optional[Dict[str, Any]] =
     render = sceneConfig.get("render")
     ndev = _native.lib().rt_device_count()
     threads = options.get("threads") or ndev  # "threads" = number of GPUs here
-    if not parallel or threads <= 1:
+    dn = options.get("denoise")
+    if dn:
+        # the filter reads every pixel's neighbours, so a denoised image is rendered on ONE GPU even when `parallel` is set
+        if verbose:
+            print("Denoising: rendering on one GPU" + (" (parallel ignored)" if parallel else ""), file=sys.stderr)
+        with createCameraFromSceneData(sceneData, render) as camera:
+            W, H = camera.imageWidth, camera.imageHeight
+            pixelData = np.zeros(W * H * 3, np.uint8)
+            stats = camera.renderDenoised(pixelData, options=None if dn is True else dn)
+    elif not parallel or threads <= 1:
         with createCameraFromSceneData(sceneData, render) as camera:
             pixelData = np.zeros(camera.imageWidth * camera.imageHeight * camera.channels, np.uint8)
             stats = camera.render(pixelData)

@@ -111,6 +111,23 @@ class rt_stats(C.Structure):
     ]
 
 
+class rt_denoise_opts(C.Structure):
+    _fields_ = [("iterations", C.c_int32), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float), ("sigma_depth", C.c_float)]
+
+
+DENOISE_OPTION_KEYS = ("iterations", "sigmaLuminance", "sigmaNormal", "sigmaDepth")
+
+
+def denoise_opts_struct(options: Optional[Dict[str, Any]]) -> rt_denoise_opts:
+    """Denoiser options {iterations (default 5), sigmaLuminance, sigmaNormal, sigmaDepth (0 or absent = default)} -> struct."""
+    o = dict(options or {})
+    unknown = set(o) - set(DENOISE_OPTION_KEYS)
+    if unknown:
+        raise RaytracerError(f"unknown denoise options: {sorted(unknown)}")
+    return rt_denoise_opts(iterations=int(o.get("iterations", 5)), sigma_luminance=float(o.get("sigmaLuminance", 0.0)),
+                           sigma_normal=float(o.get("sigmaNormal", 0.0)), sigma_depth=float(o.get("sigmaDepth", 0.0)))
+
+
 class rt_camera_info(C.Structure):
     _fields_ = [
         ("image_width", C.c_int32), ("image_height", C.c_int32), ("channels", C.c_int32),

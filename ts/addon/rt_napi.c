@@ -13,6 +13,8 @@
  *   renderRegion(handle, region, pixelData) -> stats            rt_camera_render_region / rt_multi_render_region, synchronous
  *   renderRegionAsync(handle, region, pixelData) -> Promise     same on a libuv worker (napi_async_work): keeps the event loop
  *                                                               free, like the reference's worker threads (src/raytracer.ts:60-90)
+ *   renderDenoised(handle, region, pixelData, options?) -> stats rt_camera_render_denoised (one-GPU cameras), synchronous;
+ *                                                               options {iterations, sigmaLuminance, sigmaNormal, sigmaDepth}
  *   cameraInfo(handle) -> { imageWidth, imageHeight, ... }      rt_camera_get_info / rt_multi_get_info
  *   destroyCamera(handle)                                       rt_camera_destroy / rt_multi_destroy — releases the GPU memory NOW
  *   deviceCount(), trimDeviceCache()
@@ -193,6 +195,32 @@ static napi_value RenderRegion(napi_env env, napi_callback_info info) {
   return stats_object(env, &st);
 }
 
+/* render + denoise on the device (not in the reference) */
+static napi_value RenderDenoised(napi_env env, napi_callback_info info) {
+  size_t argc = 4; napi_value argv[4];
+  napi_typedarray_type ty; size_t len; void* data; napi_value ab; size_t off;
+  napi_valuetype vt = napi_undefined;
+  rt_region reg; rt_stats st; cam_box* b;
+  rt_denoise_opts o = {5, 0.f, 0.f, 0.f};
+  CHECK(env, napi_get_cb_info(env, info, &argc, argv, NULL, NULL));
+  if (argc < 3) return throw_msg(env, "renderDenoised(handle, region, pixelData, options?)");
+  if (!(b = get_box(env, argv[0]))) return NULL;
+  if (!b->cam) return throw_msg(env, "renderDenoised renders on one GPU: create the camera with createCamera");
+  if (b->busy) return throw_msg(env, "an asynchronous render is in flight on this camera");
+  if (!read_region(env, argv[1], &reg)) return throw_msg(env, "region must be {x, y, width, height}");
+  CHECK(env, napi_get_typedarray_info(env, argv[2], &ty, &len, &data, &ab, &off));
+  if (ty != napi_uint8_clamped_array && ty != napi_uint8_array) return throw_msg(env, "pixelData must be a Uint8ClampedArray");
+  if (argc > 3) CHECK(env, napi_typeof(env, argv[3], &vt));
+  if (vt == napi_object) {
+    o.iterations = (int32_t)num_field(env, argv[3], "iterations", 5);
+    o.sigma_luminance = (float)num_field(env, argv[3], "sigmaLuminance", 0);
+    o.sigma_normal = (float)num_field(env, argv[3], "sigmaNormal", 0);
+    o.sigma_depth = (float)num_field(env, argv[3], "sigmaDepth", 0);
+  }
+  if (rt_camera_render_denoised(b->cam, &reg, (uint8_t*)data, len, NULL, &o, &st) != RT_OK) return throw_rt(env);
+  return stats_object(env, &st);
+}
+
 /* ---- the same call on a libuv worker thread ---- */
 typedef struct render_job {
   cam_box* box; rt_region reg; uint8_t* data; size_t len; rt_stats st; rt_status rc; char err[512];
@@ -274,6 +302,7 @@ static napi_value Init(napi_env env, napi_value exports) {
   napi_property_descriptor d[] = {
     {"createCamera", 0, CreateCamera, 0, 0, 0, napi_default, 0}, {"createMulti", 0, CreateMulti, 0, 0, 0, napi_default, 0},
     {"renderRegion", 0, RenderRegion, 0, 0, 0, napi_default, 0}, {"renderRegionAsync", 0, RenderRegionAsync, 0, 0, 0, napi_default, 0},
+    {"renderDenoised", 0, RenderDenoised, 0, 0, 0, napi_default, 0},
     {"cameraInfo", 0, CameraInfo, 0, 0, 0, napi_default, 0}, {"destroyCamera", 0, DestroyCamera, 0, 0, 0, napi_default, 0},
     {"deviceCount", 0, DeviceCount, 0, 0, 0, napi_default, 0}, {"trimDeviceCache", 0, TrimDeviceCache, 0, 0, 0, napi_default, 0},
   };

@@ -94,6 +94,8 @@ export function applySceneCameraOptions(sceneData: SceneData, cam?: Record<strin
 
 type NativeOpts = { seed?: number, device?: number, partIndex?: number, partCount?: number, nDevices?: number,
                     lightSampling?: 'mixture' | 'shadowRays' };   // RT_LIGHTS_*: shadowRays = next-event estimation (not the reference's estimator)
+/** rt_denoise_opts: iterations 0..8 (default 5); a sigma of 0 or absent selects its default. */
+export type DenoiseOptions = { iterations?: number, sigmaLuminance?: number, sigmaNormal?: number, sigmaDepth?: number };
 
 /** One GPU (`multi` false) or every visible GPU inside one call (`multi` true: rt_multi_*, the native stand-in for the
  *  worker pool of src/raytracer.ts:60-90).  Same `render` / `renderRegion` signatures as src/camera.ts:388,439. */
@@ -127,6 +129,11 @@ export class NativeCamera {
   /** The render on a libuv worker (napi_async_work): generateImageBuffer stays `async` without blocking the event loop. */
   async renderAsync(pixelData: Uint8ClampedArray): Promise<RenderStats> {
     return NativeCamera.stats(await addon.renderRegionAsync(this.handle, { x: 0, y: 0, width: this.imageWidth, height: this.imageHeight }, pixelData));
+  }
+  /** Render, then denoise on the device (rt_camera_render_denoised; one-GPU cameras only).  Not in the reference. */
+  renderDenoised(pixelData: Uint8ClampedArray, region?: RenderRegion, options: DenoiseOptions = {}): RenderStats {
+    return NativeCamera.stats(addon.renderDenoised(this.handle, region ?? { x: 0, y: 0, width: this.imageWidth, height: this.imageHeight },
+                                                   pixelData, options));
   }
   /** Release the GPU memory now (the reference builds a camera per request: do not wait for the GC). */
   destroy(): void { addon.destroyCamera(this.handle); }
