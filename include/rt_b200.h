@@ -274,8 +274,8 @@ rt_status rt_camera_render_features(rt_camera* cam, const rt_region* region, int
                                     float* albedo, float* normal, float* depth);
 /* The filter on explicit HOST inputs [H][W][...] of one whole image (width x height): colour [3], albedo [3], normal [3],
  * depth [1] as rt_camera_render_features writes them, moments [8] as rt_camera_render_moments writes them; out [H][W][3]
- * must not alias an input.  A pixel whose inputs are not finite is passed through unchanged and is no neighbour's tap.
- * device -1 = current.  Synchronous. */
+ * must not alias an input.  A pixel whose inputs are not finite, or whose colour over max(albedo, 1e-3) overflows FP32, is
+ * passed through unchanged and is no neighbour's tap.  Any width and height > 0.  device -1 = current.  Synchronous. */
 rt_status rt_denoise(int32_t device, int32_t width, int32_t height, const float* color, const float* albedo, const float* normal,
                      const float* depth, const float* moments, const rt_denoise_opts* opts, float* out);
 /* Render with moments, features of the first min(samples, 8) samples, and the filter, all on the device; one copy back.

@@ -59,11 +59,13 @@ __global__ void __launch_bounds__(256) k_render_features(const DevScene S, const
 constexpr float kDnAlbedoMin = 1e-3f; // demodulation floor
 RT_DEV float dn_lum(float r, float g, float b) { return 0.299f * r + 0.587f * g + 0.114f * b; } // the project's illuminance weights
 RT_DEV bool dn_finite3(const float* p) { return isfinite(p[0]) && isfinite(p[1]) && isfinite(p[2]); }
-RT_DEV bool dn_pixel(const DenoiseParams& D, int& x, int& y) {
-  x = D.x0 + (int)(blockIdx.x * blockDim.x + threadIdx.x);
-  y = D.y0 + (int)(blockIdx.y * blockDim.y + threadIdx.y);
-  return x < D.x1 && y < D.y1;
-}
+// the filter kernels run 16x16 blocks and each thread strides over rows by the grid's height: CUDA caps gridDim.y at
+// 65535, so on an image taller than 65535 * 16 rows a thread filters more than one pixel of its column
+constexpr int kDnBlock = 16;
+constexpr unsigned kDnMaxGridY = 65535;
+RT_DEV int dn_x(const DenoiseParams& D) { return D.x0 + (int)(blockIdx.x * blockDim.x + threadIdx.x); }
+RT_DEV int dn_y0(const DenoiseParams& D) { return D.y0 + (int)(blockIdx.y * blockDim.y + threadIdx.y); }
+RT_DEV int dn_ystride() { return (int)(gridDim.y * blockDim.y); }
 RT_DEV bool dn_inside(const DenoiseParams& D, int x, int y) { return x >= D.x0 && x < D.x1 && y >= D.y0 && y < D.y1; }
 
 // depth usable for a gradient: inside the region and a hit
@@ -82,9 +84,7 @@ RT_DEV float dn_gradient(const DenoiseParams& D, int x, int y, int ax, int ay, f
   return 0.f;
 }
 
-__global__ void __launch_bounds__(256) k_denoise_prepare(const DenoiseParams D) {
-  int x, y;
-  if (!dn_pixel(D, x, y)) return;
+RT_DEV void dn_prepare_pixel(const DenoiseParams& D, int x, int y) {
   const size_t p = (size_t)y * D.width + x;
   const float* c = D.color + p * 3;
   const float* a = D.albedo + p * 3;
@@ -111,11 +111,14 @@ __global__ void __launch_bounds__(256) k_denoise_prepare(const DenoiseParams D) 
   D.grad[p * 2] = hit ? dn_gradient(D, x, y, 1, 0, z) : 0.f;
   D.grad[p * 2 + 1] = hit ? dn_gradient(D, x, y, 0, 1, z) : 0.f;
 }
+__global__ void __launch_bounds__(256) k_denoise_prepare(const DenoiseParams D) {
+  const int x = dn_x(D);
+  if (x >= D.x1) return;
+  for (int y = dn_y0(D); y < D.y1; y += dn_ystride()) dn_prepare_pixel(D, x, y);
+}
 
 // one a-trous pass with step 2^k: 5x5 B3-spline taps weighted by normal, depth and luminance edge stops
-__global__ void __launch_bounds__(256) k_denoise_pass(const DenoiseParams D, const F4* __restrict__ in, F4* __restrict__ out, int step) {
-  int x, y;
-  if (!dn_pixel(D, x, y)) return;
+RT_DEV void dn_pass_pixel(const DenoiseParams& D, const F4* __restrict__ in, F4* __restrict__ out, int step, int x, int y) {
   const size_t p = (size_t)y * D.width + x;
   const F4 c = in[p];
   if (isnan(c.x)) { out[p] = c; return; }
@@ -170,10 +173,13 @@ __global__ void __launch_bounds__(256) k_denoise_pass(const DenoiseParams D, con
     }
   out[p] = F4{sr / sw, sg / sw, sb / sw, sv / (sw * sw)};
 }
+__global__ void __launch_bounds__(256) k_denoise_pass(const DenoiseParams D, const F4* __restrict__ in, F4* __restrict__ out, int step) {
+  const int x = dn_x(D);
+  if (x >= D.x1) return;
+  for (int y = dn_y0(D); y < D.y1; y += dn_ystride()) dn_pass_pixel(D, in, out, step, x, y);
+}
 
-__global__ void __launch_bounds__(256) k_denoise_finish(const DenoiseParams D, const F4* __restrict__ in) {
-  int x, y;
-  if (!dn_pixel(D, x, y)) return;
+RT_DEV void dn_finish_pixel(const DenoiseParams& D, const F4* __restrict__ in, int x, int y) {
   const size_t p = (size_t)y * D.width + x;
   const F4 c = in[p];
   float o[3];
@@ -185,6 +191,11 @@ __global__ void __launch_bounds__(256) k_denoise_finish(const DenoiseParams D, c
   }
   D.out[p * 3] = o[0]; D.out[p * 3 + 1] = o[1]; D.out[p * 3 + 2] = o[2];
   if (D.rgb8) { D.rgb8[p * 3] = gamma_rgb8(o[0]); D.rgb8[p * 3 + 1] = gamma_rgb8(o[1]); D.rgb8[p * 3 + 2] = gamma_rgb8(o[2]); }
+}
+__global__ void __launch_bounds__(256) k_denoise_finish(const DenoiseParams D, const F4* __restrict__ in) {
+  const int x = dn_x(D);
+  if (x >= D.x1) return;
+  for (int y = dn_y0(D); y < D.y1; y += dn_ystride()) dn_finish_pixel(D, in, x, y);
 }
 
 // launchers (called from rt_api.cu)
@@ -206,8 +217,9 @@ cudaError_t launch_render_features(const DevScene& S, const RenderParams& R, int
 cudaError_t launch_denoise(const DenoiseParams& D, cudaStream_t st, int* launches) {
   *launches = 0;
   if (D.x1 <= D.x0 || D.y1 <= D.y0) return cudaSuccess;
-  const dim3 block(16, 16, 1);
-  const dim3 grid((unsigned)((D.x1 - D.x0 + 15) / 16), (unsigned)((D.y1 - D.y0 + 15) / 16), 1);
+  const dim3 block(kDnBlock, kDnBlock, 1);
+  const unsigned rows = (unsigned)((D.y1 - D.y0 + kDnBlock - 1) / kDnBlock);
+  const dim3 grid((unsigned)((D.x1 - D.x0 + kDnBlock - 1) / kDnBlock), rows < kDnMaxGridY ? rows : kDnMaxGridY, 1);
   k_denoise_prepare<<<grid, block, 0, st>>>(D);
   int cur = 0;
   for (int k = 0; k < D.iterations; ++k, cur ^= 1) k_denoise_pass<<<grid, block, 0, st>>>(D, D.buf[cur], D.buf[cur ^ 1], 1 << k);

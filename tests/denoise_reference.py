@@ -6,7 +6,9 @@ The spatial filter of SVGF (Schied et al., HPG 2017) without its temporal part, 
 * prepare: demodulate i = c / max(a, 1e-3); luminance variance of the pixel mean (sum_c w_c sd_c)^2 / n over
   max(lum(a), 1e-3)^2 with sd_c = sqrt(M2_c / (n - 1)), +inf (unknown: luminance weights 1) when n < 2; depth gradient by
   central differences, one-sided at the image border and next to misses.  A pixel whose colour, albedo, normal, depth or
-  demodulated colour is not finite is passed through unchanged and is no neighbour's tap.
+  demodulated colour is not finite is passed through unchanged and is no neighbour's tap.  The demodulated colour is
+  the FP32 quotient the filter stores: a finite colour over a small albedo (3e38 / 1e-3) overflows there, although it
+  is finite in float64.
 * K a-trous passes, step 2^k, taps h = (1,4,6,4,1)/16 x itself, weight h * w_n * w_z * w_l:
     w_n = max(0, n_p.n_q)^sigma_n for two hits, 1 for two misses, 0 for a hit and a miss;
     w_z = exp(-|z_p - z_q| / (sigma_z |grad z_p . (q - p)| + 1e-3 z_p + 1e-10)) for two hits, else 1;
@@ -61,8 +63,9 @@ def prepare(color, albedo, normal, depth, moments):
         sd = (np.sqrt(m2 / (ns - 1)[..., None]) * LUM).sum(-1)
         la = np.maximum(a @ LUM, ALBEDO_MIN)
         var = np.where(ns >= 2, sd * sd / ns / (la * la), np.inf)
+        i32 = np.asarray(color, np.float32) / np.maximum(np.asarray(albedo, np.float32), np.float32(ALBEDO_MIN))
     fin = lambda x: np.isfinite(x).all(-1)  # noqa: E731
-    valid = fin(c) & fin(a) & fin(n) & np.isfinite(z) & fin(i)
+    valid = fin(c) & fin(a) & fin(n) & np.isfinite(z) & fin(i32)
     hit = valid & (z >= 0)
     usable = np.isfinite(z) & (z >= 0)
     H, W = z.shape

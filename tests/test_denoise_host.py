@@ -7,6 +7,7 @@ import subprocess
 import numpy as np
 import pytest
 
+import denoise_cases as dc
 import denoise_reference as dref
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -152,3 +153,96 @@ def test_reference_unknown_variance_lets_the_features_decide():
     moments[..., 6] = 1  # one sample: no variance estimate, luminance weights are 1
     out = dref.denoise(color, albedo, normal, depth, moments)
     assert np.isfinite(out).all() and out.std() < 0.5 * color.std()
+
+
+# ---- the edge-case generator of the GPU parity test (tests/denoise_cases.py) and the spec properties it relies on ----
+def _recount(args):
+    """The claims of a case, counted from its arrays alone."""
+    c, a, n, z, m = args
+    with np.errstate(all="ignore"):
+        demod = c / np.maximum(a, np.float32(dref.ALBEDO_MIN))  # FP32, as the filter stores it
+    fin = lambda x: np.isfinite(x).all(-1)  # noqa: E731
+    valid = fin(c) & fin(a) & fin(n) & np.isfinite(z) & fin(demod)
+    miss = valid & (z == -1) & (n == 0).all(-1) & (a == 1).all(-1)
+    return {"misses": int(miss.sum()), "invalid": int((~valid).sum()), "few_samples": int((m[..., 6] < 2).sum()),
+            "negative_m2": int((m[..., 3:6] < 0).any(-1).sum()), "zero_albedo": int((a == 0).any(-1).sum())}, valid, miss
+
+
+@pytest.mark.parametrize("kind", dc.KINDS)
+def test_case_generator_produces_what_each_case_claims(kind):
+    for H, W in dc.SHAPES:
+        args, claims = dc.make_case(kind, H, W)
+        assert all(x.dtype == np.float32 for x in args)
+        assert [x.shape for x in args] == [(H, W, 3), (H, W, 3), (H, W, 3), (H, W), (H, W, 8)]
+        counts, valid, miss = _recount(args)
+        assert counts == claims, (H, W)
+        assert np.array_equal(dref.prepare(*args)["valid"], valid), (H, W)  # the spec sees the same invalid pixels
+        if kind in dc.DEFINES:
+            assert claims[dc.DEFINES[kind]] > 0, (H, W)
+        if kind.startswith("miss_") and H * W > 1:
+            assert (valid & ~miss).any(), (H, W)  # misses next to hits
+        c, a, n, z, m = args
+        hit = valid & (z >= 0)
+        assert np.all(np.abs(np.linalg.norm(n[hit], axis=-1) - 1) <= 1e-6)  # unit normals, as the features write them
+        assert np.all(hit | miss | ~valid)
+        if kind in ("n0", "n1", "n2", "n64"):
+            assert np.all(m[..., 6] == float(kind[1:]))
+        if kind == "m2_zero":
+            assert np.all(m[..., 3:6] == 0)
+
+
+def test_parity_sets_cover_every_case_shape_iteration_count_and_option():
+    sets = dc.parity_sets()
+    assert len({s[0] for s in sets}) == len(sets)
+    assert {s[1] for s in sets} == set(dc.KINDS)
+    assert {s[2] for s in sets} == set(dc.SHAPES)
+    assert {s[3]["iterations"] for s in sets} == set(range(9))
+    for _, opts in dc.OPTIONS:
+        assert any({k: v for k, v in s[3].items() if k != "iterations"} == opts for s in sets)
+
+
+@pytest.mark.parametrize("kind", [k for k in dc.KINDS if k.startswith("nonfinite_")] + ["demod_overflow"])
+def test_reference_passes_invalid_pixels_through_bit_for_bit(kind):
+    for H, W in dc.SHAPES:
+        args, claims = dc.make_case(kind, H, W)
+        _, valid, _ = _recount(args)
+        out = dref.denoise(*args)
+        assert np.array_equal(out[~valid], args[0][~valid].astype(np.float64), equal_nan=True)
+        assert np.isfinite(out[valid]).all()
+
+
+@pytest.mark.parametrize("kind", ["miss_single", "n0", "n1", "n64", "m2_zero", "albedo_edges", "depth_tiny", "depth_huge"])
+def test_reference_leaves_a_1x1_image_unchanged(kind):
+    args, _ = dc.make_case(kind, 1, 1)
+    for it in range(9):
+        out = dref.denoise(*args, {"iterations": it})
+        np.testing.assert_allclose(out, args[0], rtol=1e-15, atol=0)  # demodulate, divide by the one weight, remodulate
+
+
+@pytest.mark.parametrize("shape", [(16, 16), (17, 33), (33, 17), (7, 300)])
+def test_reference_miss_block_ignores_the_colours_of_hits(shape):
+    args, _ = dc.make_case("miss_block", *shape)
+    _, _, miss = _recount(args)
+    other = list(args)
+    other[0] = args[0].copy()
+    other[0][~miss] = np.random.default_rng(1).uniform(0, 5, (int((~miss).sum()), 3)).astype(np.float32)
+    # a hit is no miss' tap.  Only the hits' variance reaches a miss, through the 3x3 blur; it is the render's until the
+    # first pass, after which it depends on the hits' colours (their luminance weights), so the property is one pass's.
+    a = dref.denoise(*args, {"iterations": 1})
+    b = dref.denoise(*other, {"iterations": 1})
+    assert np.array_equal(a[miss], b[miss])
+    assert not np.array_equal(a[~miss], b[~miss])
+
+
+@pytest.mark.parametrize("kind", ["miss_block", "n_mixed", "depth_ramps", "facets", "albedo_edges"])
+def test_reference_step_beyond_the_image_is_the_centre_tap(kind):
+    for H, W in dc.SHAPES:
+        args, _ = dc.make_case(kind, H, W)
+        P = dref.prepare(*args)
+        o = dref.options()
+        for step in (max(H, W), 2 * max(H, W) + 1, 128):
+            if step < max(H, W):
+                continue
+            i, v = dref.atrous_pass(P, P["i"], P["var"], step, o)
+            np.testing.assert_allclose(i, P["i"], rtol=1e-15, atol=0)
+            np.testing.assert_allclose(v, P["var"], rtol=1e-15, atol=0)

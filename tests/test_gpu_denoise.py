@@ -1,12 +1,18 @@
-"""GPU checks of the opt-in denoiser: feature buffers against the primary-visibility hook, the FP32 filter against its numpy
-specification (tests/denoise_reference.py), region / determinism / option plumbing, and image quality against a
-high-sample render with another seed.  Run on a B200 with `-m gpu`."""
+"""GPU checks of the opt-in denoiser: feature buffers against the primary-visibility hook and against the oracle's own
+camera rays, the FP32 filter against its numpy specification (tests/denoise_reference.py) on renders and on the edge
+inputs of tests/denoise_cases.py, the render's per-pixel moments against the oracle's on the same random streams,
+region / determinism / option plumbing, and image quality against a high-sample render with another seed.  Run on a
+B200 with `-m gpu`."""
+import functools
+
 import numpy as np
 import pytest
 
+import denoise_cases as dc
 import denoise_reference as dref
+import oracle_binding as ob
 from mcp_raytracer_b200 import (
-    Camera, RaytracerError, createCameraFromSceneData, denoise, generateCornellSceneData,
+    Camera, RaytracerError, createCameraFromSceneData, denoise, generateCornellSceneData, generateDefaultSceneData,
     generateImageBuffer, generateLayeredMixedSceneData, generateRainSceneData, generateSceneData, generateSpheresSceneData,
     generateWeekendFinalSceneData,
 )
@@ -21,6 +27,7 @@ SCENES = {
     "C3-weekend": generateWeekendFinalSceneData,
     "C4-rain": lambda: generateRainSceneData({"count": 20000, "seed": 1, "sphereRadius": 0.01}),
     "C5-layered": generateLayeredMixedSceneData,
+    "default": generateDefaultSceneData,
 }
 MAT_LAMBERT, MAT_METAL, MAT_GLASS, MAT_LIGHT, MAT_MIXED, MAT_LAYERED = range(6)
 
@@ -63,7 +70,7 @@ def camera_dir_norm(cam):
     return np.sqrt((d * d).sum(-1))
 
 
-@pytest.mark.parametrize("name", list(SCENES))
+@pytest.mark.parametrize("name", [k for k in SCENES if k != "default"])
 @pytest.mark.parametrize("bvh", ["reference", "sah", "list"])
 def test_features_at_one_sample_equal_the_primary_hits(gpu, name, bvh):
     sd = SCENES[name]()
@@ -82,35 +89,93 @@ def test_features_at_one_sample_equal_the_primary_hits(gpu, name, bvh):
     assert np.array_equal(f["albedo"], object_albedo(sd, ids))
 
 
-def _uniform_3x3(ids):
-    H, W = ids.shape
-    same = np.zeros((H, W), bool)
-    same[1:-1, 1:-1] = True
-    for dy in (-1, 0, 1):
-        for dx in (-1, 0, 1):
-            same[1:-1, 1:-1] &= ids[1 + dy:H - 1 + dy, 1 + dx:W - 1 + dx] == ids[1:-1, 1:-1]
-    return same & (ids >= 0)
+FEATURE_OPTS = {"width": 160, "samples": 16, "seed": 4}  # samples > 1: every sample's camera ray is jittered
 
 
-@pytest.mark.parametrize("name", ["C2-cornell", "C5-layered"])
-def test_features_over_jittered_samples(gpu, name):
+@functools.lru_cache(maxsize=None)
+def oracle_camera_rays(name, n_samples=8):
+    """The camera rays of samples 0..n_samples-1 of every pixel (OracleCamera.get_ray: the device's Philox streams and
+    getRay, bit for bit) traced to their first hit by the oracle: origins, directions [S,H,W,3], ids [S,H,W], t, normals."""
     sd = SCENES[name]()
-    with createCameraFromSceneData(sd, {"width": 128, "samples": 8, "seed": 2}) as cam:
-        ids, _, nrm, _ = cam.tracePrimary()
-        f1 = cam.renderFeatures(8)
-        f2 = cam.renderFeatures(8)
-    for k in f1:
-        assert np.array_equal(f1[k], f2[k]), k
-    flat = FlatScene(sd)
-    planar = np.asarray(flat.obj_type) != 0
-    sel = _uniform_3x3(ids)
-    sel[sel] &= planar[ids[sel]]
-    assert sel.sum() > 1000
-    assert np.abs(f1["normal"][sel] - nrm[sel]).max() <= 2e-6
-    assert np.abs(f1["albedo"][sel] - object_albedo(sd, ids)[sel]).max() <= 2e-6
-    assert np.all(f1["depth"][sel] > 0)
+    oc = ob.OracleCamera(sd, FEATURE_OPTS)
+    W, H = oc.imageWidth, oc.imageHeight
+    o = np.zeros((n_samples, H, W, 3), np.float32)
+    d = np.zeros((n_samples, H, W, 3), np.float32)
+    for s in range(n_samples):
+        for j in range(H):
+            for i in range(W):
+                o[s, j, i], d[s, j, i] = oc.get_ray(i, j, s, FEATURE_OPTS["seed"])
+    ids, t, nrm, _ = oc.trace_rays(o.reshape(-1, 3), d.reshape(-1, 3))
+    shape = (n_samples, H, W)
+    return oc, o, d, ids.reshape(shape), t.reshape(shape), nrm.reshape(shape + (3,))
 
 
+def oracle_features(name, F):
+    """The features restated in float64 over the oracle's rays of samples 0..F-1: albedo = mean feature albedo (1 on a
+    miss); normal = sum of the face-forwarded normals, renormalised when more than one ray hit, 0 when none did;
+    depth = mean t |d| over the rays that hit, -1 when none did."""
+    _, _, d, ids, t, nrm = oracle_camera_rays(name)
+    ids, t, nrm, d = ids[:F], t[:F], nrm[:F].astype(np.float64), d[:F].astype(np.float64)
+    hit = ids >= 0
+    albedo = object_albedo(SCENES[name](), ids).astype(np.float64).mean(0)
+    hits = hit.sum(0)
+    nsum = np.where(hit[..., None], nrm, 0.0).sum(0)
+    norm = np.sqrt((nsum * nsum).sum(-1, keepdims=True))
+    normal = np.where((hits > 1)[..., None], nsum / np.where(norm > 0, norm, 1.0), nsum)
+    z = np.where(hit, t * np.sqrt((d * d).sum(-1)), 0.0).sum(0)
+    depth = np.where(hits > 0, z / np.maximum(hits, 1), -1.0)
+    return {"albedo": albedo, "normal": normal, "depth": depth}, hits
+
+
+def _feature_failures(name, F, got, ref, hits):
+    """Pixels outside the bars, with the oracle's rays there, their ids and t with the tree and by brute force."""
+    bad = ~(np.abs(got["albedo"] - ref["albedo"]) <= 1e-6 * np.abs(ref["albedo"])).all(-1)
+    bad |= ~(np.abs(got["normal"] - ref["normal"]) <= 2e-4).all(-1)
+    bad |= ~(np.abs(got["depth"] - ref["depth"]) <= 1e-4 * np.abs(ref["depth"]))
+    bad |= (hits == 0) != (got["depth"] == -1)
+    if not bad.any():
+        return None
+    oc, o, d, ids, t, _ = oracle_camera_rays(name)
+    lines = [f"{int(bad.sum())} pixels outside the bars at F={F}"]
+    for j, i in list(zip(*np.nonzero(bad)))[:4]:
+        bf_ids, bf_t, _, _ = oc.trace_rays(o[:F, j, i], d[:F, j, i], use_bvh=False)
+        lines.append(f"pixel ({i},{j}): gpu albedo {got['albedo'][j, i]} normal {got['normal'][j, i]} depth {got['depth'][j, i]}; "
+                     f"oracle {ref['albedo'][j, i]} {ref['normal'][j, i]} {ref['depth'][j, i]}")
+        for s in range(F):
+            lines.append(f"  sample {s}: o {o[s, j, i].tolist()} d {d[s, j, i].tolist()} oracle id {ids[s, j, i]} t {t[s, j, i]!r}, "
+                         f"brute force id {bf_ids[s]} t {bf_t[s]!r}")
+    return "\n".join(lines)
+
+
+@pytest.mark.parametrize("name", ["C1-spheres", "C2-cornell", "C5-layered", "default", "C3-weekend"])
+@pytest.mark.parametrize("bvh", ["reference", "sah", "list"])
+def test_features_match_the_oracle_rays(gpu, name, bvh):
+    """Jittered rays (samples 16, so even F = 1 jitters), silhouettes, averaged sphere normals, pixels where only some
+    rays hit, and defocus (default: aperture 0.05, C3: 0.1), on every pixel; then a region with x0, y0 off the 16-pixel
+    tile grid touching the right edge equals the whole image bit for bit and leaves the rest 0."""
+    sd = SCENES[name]()
+    if bvh == "list" and len(sd["objects"]) > 128:
+        pytest.skip("LIST trees hold at most 128 objects")
+    with Camera(sd, None, {**FEATURE_OPTS, "bvh": bvh}) as cam:
+        W, H = cam.imageWidth, cam.imageHeight
+        whole = {F: cam.renderFeatures(F) for F in (1, 3, 8)}
+        again = cam.renderFeatures(8)
+        region = {"x": 37, "y": 21, "width": W - 37, "height": min(30, H - 21)}
+        part = cam.renderFeatures(8, region)
+    for k in again:
+        assert np.array_equal(again[k], whole[8][k]), k  # deterministic
+    for F, got in whole.items():
+        ref, hits = oracle_features(name, F)
+        msg = _feature_failures(name, F, got, ref, hits)
+        assert msg is None, msg
+    inside = np.zeros((H, W), bool)
+    inside[region["y"]:region["y"] + region["height"], region["x"]:] = True
+    for k in part:
+        assert np.array_equal(part[k][inside], whole[8][k][inside]), k
+        assert np.all(part[k][~inside] == 0), k
+
+
+@functools.lru_cache(maxsize=None)
 def _crop_inputs(seed=5):
     sd = generateCornellSceneData()
     with createCameraFromSceneData(sd, {"width": 128, "samples": 8, "aTolerance": 0, "seed": seed}) as cam:
@@ -123,22 +188,78 @@ def _crop_inputs(seed=5):
     return lin[ys, xs], f["albedo"][ys, xs], f["normal"][ys, xs], f["depth"][ys, xs], mom[ys, xs]
 
 
-@pytest.mark.parametrize("iterations", [0, 1, 5])
-def test_filter_matches_the_numpy_specification(gpu, iterations):
-    args = _crop_inputs()
-    got = denoise(*args, options={"iterations": iterations})
-    ref = dref.denoise(*args, {"iterations": iterations})
-    err = np.abs(got - ref)
-    assert np.all(err <= 1e-4 * np.abs(ref) + 1e-7), float((err / (np.abs(ref) + 1e-7)).max())
-    if iterations:
+def check_against_spec(got, args, opts=None):
+    """The bars of the filter against its specification, on every pixel: 1e-4 relative (+1e-7) wherever the spec's
+    output is finite, non-finite outputs exactly where the spec's are, and pass-through pixels bit-equal to the input
+    colour."""
+    ref = dref.denoise(*args, opts)
+    fin = np.isfinite(ref)
+    assert np.array_equal(np.isfinite(got), fin), np.argwhere(np.isfinite(got) != fin)[:8]
+    with np.errstate(invalid="ignore"):
+        err = np.abs(got.astype(np.float64) - ref)
+    ok = err <= 1e-4 * np.abs(ref) + 1e-7
+    assert np.all(ok[fin]), (np.argwhere(~ok & fin)[:8], float((err[fin] / (np.abs(ref[fin]) + 1e-7)).max()))
+    passed = ~dref.prepare(*args)["valid"]
+    color = np.asarray(args[0], np.float32)
+    assert np.array_equal(got[passed].view(np.uint32), color[passed].view(np.uint32))
+    return ref
+
+
+PARITY_SETS = [pytest.param("crop", None, {"iterations": k}, id=str(k)) for k in (0, 1, 5)] + [
+    pytest.param(kind, shape, opts, id=i) for i, kind, shape, opts in dc.parity_sets()]
+
+
+@pytest.mark.parametrize("kind,shape,opts", PARITY_SETS)
+def test_filter_matches_the_numpy_specification(gpu, kind, shape, opts):
+    """A crop of a Cornell render, and the edge inputs of tests/denoise_cases.py: misses, non-finite inputs and FP32
+    overflow of the demodulated colour, sample counts 0..64, clamped moments, albedo floors, depth ramps and scales,
+    facets of nearly parallel normals; shapes from 1x1 to 7x300 that are not multiples of the 16x16 block, iterations
+    0..8 (steps up to 128, where most taps fall outside the image) and non-default sigmas."""
+    args = _crop_inputs() if kind == "crop" else dc.make_case(kind, *shape)[0]
+    got = denoise(*args, options=opts)
+    check_against_spec(got, args, opts)
+    if kind == "crop" and opts["iterations"]:
         assert np.abs(got - args[0]).max() > 1e-3  # it filtered
 
 
-def test_region_writes_only_region_pixels_and_equals_denoise_of_the_crop(gpu):
-    sd = generateCornellSceneData()
-    region = {"x": 20, "y": 12, "width": 70, "height": 50}
+def test_denoise_covers_images_taller_than_the_launch_grid(gpu):
+    """2 x 1 048 600: more rows than 65535 blocks of 16 cover.  The input repeats a 256-row case, so the spec of the
+    whole image is known from that of its first and last 1024 rows: the filter's reach over 5 passes is
+    sum_k (2 * 2^k + 1) + 1 = 68 rows (taps, 3x3 variance blur, depth gradient), and every row further than that from
+    both ends sees the rows the same row of the period sees in the first crop."""
+    H, W, P, C = 1_048_600, 2, 256, 1024
+    tile, _ = dc.make_case("miss_border", P, W)
+    args = [np.tile(a, (H // P + 1,) + (1,) * (a.ndim - 1))[:H] for a in tile]
+    got = denoise(*args)
+    top = dref.denoise(*(a[:C] for a in args))
+    bottom = dref.denoise(*(a[H - C:] for a in args))
+    y = np.arange(H)
+    src = np.where(y < C - 128, y, P + (y % P))  # rows of `top`
+    ref = top[np.minimum(src, C - 1)]
+    ref[H - (C - 128):] = bottom[128:]
+    err = np.abs(got.astype(np.float64) - ref)
+    bad = ~(err <= 1e-4 * np.abs(ref) + 1e-7)
+    assert not bad.any(), (int(bad.any(-1).sum()), np.argwhere(bad.any(-1))[:8].ravel())
+    assert np.abs(got[-40:] - args[0][-40:]).max() > 1e-3  # the rows past 65535 blocks were filtered
+
+
+REGIONS = {  # as functions of the image size
+    "interior": lambda W, H: {"x": 20, "y": 12, "width": 70, "height": 50},        # x0, y0 off the 16-pixel grid
+    "right-bottom": lambda W, H: {"x": W - 45, "y": H - 29, "width": 45, "height": 29},
+    "column": lambda W, H: {"x": 57, "y": 5, "width": 1, "height": H - 10},
+    "clipped": lambda W, H: {"x": W - 23, "y": H - 17, "width": 40, "height": 40},  # runs past the image
+}
+
+
+def check_denoised_region(name, region_name):
+    """renderDenoised on a region against the spec of the crop of the same camera's renderRegion(linear, moments) and
+    renderFeatures(min(samples, 8), region): renders are bit-deterministic and take their moments from the same kernel.
+    Pixels outside the region stay as they were, the region's RGB8 is gamma_rgb8 of its linear output, and rt_denoise
+    on the crop gives the same image."""
+    sd = SCENES[name]()
     with createCameraFromSceneData(sd, {"width": 128, "samples": 16, "aTolerance": 0, "seed": 8}) as cam:
         W, H = cam.imageWidth, cam.imageHeight
+        region = REGIONS[region_name](W, H)
         rgb = np.full(W * H * 3, 7, np.uint8)
         lin = np.full((H, W, 3), -5.0, np.float32)
         st = cam.renderDenoised(rgb, lin, region)
@@ -146,14 +267,31 @@ def test_region_writes_only_region_pixels_and_equals_denoise_of_the_crop(gpu):
         mom = np.zeros((H, W, 8), np.float32)
         cam.renderRegion(None, region, lin0, mom)
         f = cam.renderFeatures(8, region)
-    ys, xs = slice(12, 62), slice(20, 90)
+    x0, y0 = region["x"], region["y"]
+    x1, y1 = min(W, x0 + region["width"]), min(H, y0 + region["height"])
+    ys, xs = slice(y0, y1), slice(x0, x1)
     inside = np.zeros((H, W), bool)
     inside[ys, xs] = True
     rgb = rgb.reshape(H, W, 3)
     assert np.all(rgb[~inside] == 7) and np.all(lin[~inside] == -5.0)
-    assert st.pixels == 70 * 50 and st.kernelLaunches >= 1 + 1 + 5 + 2
-    crop = denoise(lin0[ys, xs], f["albedo"][ys, xs], f["normal"][ys, xs], f["depth"][ys, xs], mom[ys, xs])
-    np.testing.assert_allclose(lin[ys, xs], crop, rtol=1e-6, atol=1e-7)
+    assert st.pixels == (x1 - x0) * (y1 - y0) and st.kernelLaunches >= 1 + 1 + 5 + 2
+    args = (lin0[ys, xs], f["albedo"][ys, xs], f["normal"][ys, xs], f["depth"][ys, xs], mom[ys, xs])
+    check_against_spec(lin[ys, xs], args)
+    assert np.array_equal(rgb[ys, xs], dref.gamma_rgb8(lin[ys, xs]))
+    np.testing.assert_allclose(lin[ys, xs], denoise(*args), rtol=1e-6, atol=1e-7)
+    print(f"{name} {region_name}: {int((args[3] == -1).sum())} miss pixels of {args[3].size}")
+
+
+def test_region_writes_only_region_pixels_and_equals_denoise_of_the_crop(gpu):
+    check_denoised_region("C2-cornell", "interior")
+
+
+@pytest.mark.parametrize("name,region_name", [(n, r) for n in ("C2-cornell", "default") for r in REGIONS
+                                              if (n, r) != ("C2-cornell", "interior")])
+def test_denoised_regions_match_the_specification(gpu, name, region_name):
+    """Regions touching the right and bottom edges, one pixel wide, and clipped at the image; the default scene brings
+    misses (sky) and defocus."""
+    check_denoised_region(name, region_name)
 
 
 def test_denoised_render_is_deterministic_and_rgb8_follows_the_gamma_rule(gpu):
@@ -167,6 +305,76 @@ def test_denoised_render_is_deterministic_and_rgb8_follows_the_gamma_rule(gpu):
         out.append((rgb, lin))
     assert np.array_equal(out[0][0], out[1][0]) and np.array_equal(out[0][1], out[1][1])
     assert np.array_equal(out[0][0].reshape(lin.shape), dref.gamma_rgb8(out[0][1]))
+
+
+MOMENT_CASES = {  # scene, render options; the pixel-stream kernel that writes the moments
+    "C2-cornell-16spp": ("C2-cornell", {"width": 96, "samples": 16, "aTolerance": 0}),         # k_render_stream
+    "C5-layered-16spp": ("C5-layered", {"width": 96, "samples": 16, "aTolerance": 0}),
+    "default-16spp": ("default", {"width": 128, "samples": 16, "aTolerance": 0}),
+    "C2-cornell-adaptive": ("C2-cornell", {"width": 64}),                                      # the reference's defaults
+    "C4-rain100k-depth2": ("C4-rain100k", {"width": 160, "samples": 12, "aTolerance": 0, "depth": 2}),  # k_render_stream_trav
+}
+# per-sample agreement delta of same-path samples: 1e-6, except where reflections off 1 cm drops magnify FP32 direction
+# differences a hundredfold (test_gpu_full_parity.run_c4_same_seed); there the selection's 1e-5 on sum c is the bound.
+# Measured on a B200 with 1e-6 for C4: one pixel at 1.01 x the bar ((31, 2) red, n 12, M2 off by 1.3e-3 relative).
+SAMPLE_DELTA = {"C4-rain100k-depth2": 1e-5}
+# same-path fractions measured on a B200: 0.9990, 0.9820, 0.9990, 0.9985, 0.9747 (deterministic: same seed, bit-deterministic renders)
+SAME_PATH_FLOOR = {"C2-cornell-16spp": 0.99, "C5-layered-16spp": 0.97, "default-16spp": 0.99, "C2-cornell-adaptive": 0.99,
+                   "C4-rain100k-depth2": 0.96}
+
+
+@pytest.mark.parametrize("case", list(MOMENT_CASES))
+def test_moments_match_the_oracle_on_the_same_random_streams(gpu, case):
+    """The render's Welford moments (sum c, M2 = sum of squared deviations from the mean, n, bounces) against the
+    oracle's float64 sums on the same seed: M2_o = sum c^2 - (sum c)^2 / n.  Compared on same-path pixels only: equal
+    bounce totals and sum c within 1e-5 relative per channel.
+
+    The bar |M2_g - M2_o| <= a M2_o + b sqrt(M2_o sum c^2_o) + (b / 2)^2 sum c^2_o.  If each deviation from the mean
+    d_k carries an error |f_k| <= (b / 2) |c_k|, Cauchy-Schwarz on M2_g = sum (d_k + f_k)^2 gives
+    |dM2| <= 2 sqrt(M2 sum f^2) + sum f^2 <= b sqrt(M2 sum c^2) + (b / 2)^2 sum c^2.  Two sources of f_k:
+    * per-sample agreement.  A same-path sample is the same product of FP32 factors on both sides, equal to a relative
+      delta (SAMPLE_DELTA, 1e-6), which shifts the sample and the mean by delta |c| at most.
+    * FP32 Welford.  The running sum after k samples is off by at most k eps sum|c| (eps = 2^-24) and 1 / (n - 1) is
+      rounded, so the running mean, and with it each deviation, is off by about n eps |c|.  Each non-negative term
+      (x - mean_old)(x - mean_new) and the FMA that adds it round to eps, so the sum is off by (n + 2) eps M2 relative.
+    So b = 2 (delta + n 2^-24), about 4e-6 at 16 spp; the last term is what is left when every sample is equal
+    (M2_o = 0: a sky channel of 1.0, the light); a = (n + 2) 2^-24 <= 1e-4 for n <= 1600, kept at 1e-3.
+    Pixels with one sample have M2 = 0 exactly (moments_add starts at the second)."""
+    name, opts = MOMENT_CASES[case]
+    sd = rain100k() if name == "C4-rain100k" else SCENES[name]()
+    opts = {**opts, "seed": 11}
+    with createCameraFromSceneData(sd, opts) as cam:
+        W, H = cam.imageWidth, cam.imageHeight
+        if name == "C4-rain100k":
+            assert cam.info.n_bvh_nodes >= 16384 and cam.info.bvh_kind == 2  # deep tree: k_render_stream_trav
+        lin = np.zeros((H, W, 3), np.float32)
+        mom = np.zeros((H, W, 8), np.float32)
+        cam.renderRegion(None, None, lin, mom)
+    o = ob.OracleCamera(sd, opts).render(seed=11, threads=8, want_moments=True)["moments"]
+    g = mom.astype(np.float64)
+    n_o = o[..., 6]
+    m2_o = np.maximum(o[..., 3:6] - o[..., 0:3] ** 2 / np.maximum(n_o, 1)[..., None], 0.0)  # >= 0 up to float64 rounding
+    same = (g[..., 7] == o[..., 7]) & (np.abs(g[..., 0:3] - o[..., 0:3]) <= 1e-5 * np.abs(o[..., 0:3])).all(-1)
+    frac = float(same.mean())
+    n_g = g[..., 6]
+    a, b = 1e-3, 2 * (SAMPLE_DELTA.get(case, 1e-6) + n_o * 2.0 ** -24)
+    bound = a * m2_o + b[..., None] * np.sqrt(m2_o * o[..., 3:6]) + (b[..., None] / 2) ** 2 * o[..., 3:6]
+    err = np.abs(g[..., 3:6] - m2_o)
+    ratio = np.where(bound > 0, err / np.where(bound > 0, bound, 1), np.where(err > 0, np.inf, 0))
+    print(f"{case}: {W}x{H}, same-path pixels {frac:.4f}, n {int(n_o.min())}..{int(n_o.max())}, "
+          f"worst |dM2| / bar {float(ratio[same].max()):.3g}, worst |dM2| / M2 {float((err / np.maximum(m2_o, 1e-30))[same].max()):.3g}")
+    assert frac >= SAME_PATH_FLOOR[case]
+    assert np.array_equal(n_g[same], n_o[same])
+    bad = np.argwhere(same[..., None] & ~(err <= bound))[:4]
+    assert len(bad) == 0, [(tuple(k), n_o[k[0], k[1]], g[k[0], k[1], 3 + k[2]], m2_o[tuple(k)], o[k[0], k[1], 3 + k[2]]) for k in bad]
+    one = same & (n_o == 1)
+    assert np.all(g[one][:, 3:6] == 0)
+    if "adaptive" in case:
+        assert n_o[same].min() < n_o[same].max()  # the sample count differs per pixel
+
+
+def rain100k():
+    return generateRainSceneData({"count": 100000, "seed": 1, "sphereRadius": 0.01})
 
 
 def rel_mse(x, r, mask=None):
