@@ -303,6 +303,19 @@ rt_status rt_multi_get_info(const rt_multi* multi, rt_camera_info* info, int32_t
  * RenderStats.merge (src/render-utils/renderStats.ts:42-64), device_ms = the slowest device.  Synchronous. */
 rt_status rt_multi_render_region(rt_multi* multi, const rt_region* region, uint8_t* rgb8, size_t rgb8_len,
                                  float* linear_rgb, rt_stats* stats);
+/* rt_camera_render_denoised on every device of the rt_multi: rgb8 / linear_rgb are bit-identical to that call's on one
+ * camera with the same scene, options and region, for every n_devices and on both paths.  Device k renders its blocks'
+ * colour and moments into device[0]'s memory; after every device's render, each device filters a contiguous band of the
+ * region's rows, recomputing the rows its passes read beyond the band (up to 2^(iterations+1) - 1 rows each side, clipped
+ * to the region) and reading the colour over the peer mapping; the bands land in device[0]'s framebuffer.  Without peer
+ * access the colour and moments are merged on the host and device[0] filters the whole region.  Each device holds
+ * whole-image feature and filter buffers (84 bytes per pixel); device[0] also holds the colour and moments (44 bytes per
+ * pixel).  Errors as rt_camera_render_denoised (RT_ERR_UNSUPPORTED for render modes other than RT_MODE_DEFAULT).
+ * stats: merged as rt_multi_render_region merges them; device_ms = device[0]'s span from the start of its render to the
+ * end of the call's last kernel (waiting for the other devices included); kernel_launches = the sum over the devices.
+ * Synchronous. */
+rt_status rt_multi_render_denoised(rt_multi* multi, const rt_region* region, uint8_t* rgb8, size_t rgb8_len,
+                                   float* linear_rgb, const rt_denoise_opts* opts, rt_stats* stats);
 
 /* ---- one process PER GPU (torch.distributed ranks of one node): a device buffer every rank can write ----
  * Rank 0 creates the framebuffer and hands the 64-byte CUDA IPC handle to the other ranks (any transport);

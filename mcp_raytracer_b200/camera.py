@@ -383,6 +383,25 @@ class MultiCamera:
     def render(self, pixelData: np.ndarray, linear: Optional[np.ndarray] = None) -> RenderStats:
         return self.renderRegion(pixelData, None, linear)
 
+    def renderDenoised(self, pixelData: Optional[np.ndarray], linear: Optional[np.ndarray] = None, region: Optional[Dict[str, int]] = None,
+                       options: Optional[Dict[str, Any]] = None) -> RenderStats:
+        """`Camera.renderDenoised` on every device (rt_multi_render_denoised): the same bytes as one Camera's.  Each device
+        filters a band of the region's rows after every device has rendered."""
+        W, H = self.imageWidth, self.imageHeight
+        if pixelData is not None and (pixelData.dtype != np.uint8 or not pixelData.flags["C_CONTIGUOUS"]):
+            raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
+        if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3 or not linear.flags["C_CONTIGUOUS"]):
+            raise RaytracerError("linear buffer must be float32 [H][W][3]")
+        reg = _region_struct(region, W, H)
+        opts = denoise_opts_struct(options)
+        st = rt_stats()
+        rc = _native.lib().rt_multi_render_denoised(
+            self._h, C.byref(reg), pixelData.ctypes.data if pixelData is not None else None, pixelData.nbytes if pixelData is not None else 0,
+            linear.ctypes.data if linear is not None else None, C.byref(opts), C.byref(st))
+        if rc != 0:
+            raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(rc, rc)}]")
+        return RenderStats.from_struct(st)
+
 
 def createCameraFromSceneData(sceneData: Dict[str, Any], renderOptions: Optional[Dict[str, Any]] = None) -> Camera:
     """src/scenes/scenes.ts:60-104"""

@@ -31,7 +31,7 @@ cudaError_t launch_trace_primary(const DevScene& S, const RenderParams& R, int* 
 cudaError_t launch_fp32_peak(float* out, int blocks, int iters, cudaStream_t st);
 cudaError_t launch_render_features(const DevScene& S, const RenderParams& R, int n_samples, float* albedo, float* normal, float* depth,
                                    cudaStream_t st);
-cudaError_t launch_denoise(const DenoiseParams& D, cudaStream_t st, int* launches);
+cudaError_t launch_denoise(const DenoiseParams& D, int b0, int b1, cudaStream_t st, int* launches);
 cudaError_t launch_render_wavefront(const DevScene& S, const RenderParams& R, WfHost& H, int sms, cudaStream_t st, int* launches);
 cudaError_t launch_finalize_stats(const unsigned long long* raw, rt_stats* out, int launches, cudaStream_t st);
 // per-function parity hooks (rt_debug.cuh)
@@ -957,6 +957,45 @@ static rt_status features_prepare(rt_camera* c, size_t npx) {
   return RT_OK;
 }
 
+// Features and filter of the rows [b0, b1) of the region of P, on camera c's device and stream.  `color` / `moments` are
+// [H][W] buffers this device can read, written by a render of the region; `out` / `rgb8` receive the band's rows.  The
+// camera's whole-image feature and scratch buffers hold what the band's stages compute: the band plus the rows its passes
+// read (dn_halo), clipped to the region.  `out` may alias `color` only when one band covers the region.  `poison` first
+// fills those buffers with NaN, so that a read outside the computed rows changes the image.
+static rt_status denoise_band(rt_camera* c, const RenderParams& P, int b0, int b1, const DenoiseParams& opts, const float* color,
+                              const float* moments, float* out, uint8_t* rgb8, bool poison, int* launches) {
+  *launches = 0;
+  if (P.x1 <= P.x0 || b1 <= b0) return RT_OK;
+  const int W = c->hs->image_width;
+  const size_t npx = (size_t)W * c->hs->image_height;
+  rt_status st = features_prepare(c, npx);
+  if (st != RT_OK) return st;
+  if (!c->d_dn) CU(dev_alloc(&c->d_dn, npx * kDnFloatsPerPixel * sizeof(float)));
+  if (poison) {
+    CU(cudaMemsetAsync(c->d_falb, 0xff, npx * 12, c->stream));
+    CU(cudaMemsetAsync(c->d_fnrm, 0xff, npx * 12, c->stream));
+    CU(cudaMemsetAsync(c->d_fdepth, 0xff, npx * 4, c->stream));
+    CU(cudaMemsetAsync(c->d_dn, 0xff, npx * kDnFloatsPerPixel * sizeof(float), c->stream));
+  }
+  RenderParams F = P; // the feature rows: one beyond what prepare computes
+  const int hf = dn_halo(opts.iterations, -1) + 1;
+  F.y0 = std::max(P.y0, b0 - hf);
+  F.y1 = std::min(P.y1, b1 + hf);
+  const int n_feat = std::max(1, std::min(c->hs->cam.samples, 8));
+  CU(launch_render_features(c->ds, F, n_feat, c->d_falb, c->d_fnrm, c->d_fdepth, c->stream));
+  DenoiseParams D = opts;
+  D.width = W;
+  D.x0 = P.x0; D.y0 = P.y0; D.x1 = P.x1; D.y1 = P.y1;
+  D.color = color; D.albedo = c->d_falb; D.normal = c->d_fnrm; D.depth = c->d_fdepth; D.moments = moments;
+  dn_scratch(D, c->d_dn, npx);
+  D.out = out;
+  D.rgb8 = rgb8;
+  int dn_launches = 0;
+  CU(launch_denoise(D, b0, b1, c->stream, &dn_launches));
+  *launches = 1 + dn_launches;
+  return RT_OK;
+}
+
 rt_status rt_camera_render_features(rt_camera* c, const rt_region* region, int32_t n_samples, float* albedo, float* normal, float* depth) {
   RT_GUARD_BEGIN
   if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
@@ -1020,7 +1059,7 @@ rt_status rt_denoise(int32_t device, int32_t width, int32_t height, const float*
   D.out = d_col;
   D.rgb8 = nullptr;
   int launches = 0;
-  CU(launch_denoise(D, 0, &launches));
+  CU(launch_denoise(D, 0, height, 0, &launches));
   CU(cudaMemcpyAsync(out, d_col, npx * 12, cudaMemcpyDeviceToHost, 0));
   CU(cudaStreamSynchronize(0));
   return RT_OK;
@@ -1047,8 +1086,6 @@ rt_status rt_camera_render_denoised(rt_camera* c, const rt_region* region, uint8
   if (rgb8 && !c->d_rgb8) CU(dev_alloc(&c->d_rgb8, npx * 3));
   if (!c->d_linear) CU(dev_alloc(&c->d_linear, npx * 3 * sizeof(float)));
   if (!c->d_moments) CU(dev_alloc(&c->d_moments, npx * 8 * sizeof(float)));
-  if ((st = features_prepare(c, npx)) != RT_OK) return st;
-  if (!c->d_dn) CU(dev_alloc(&c->d_dn, npx * kDnFloatsPerPixel * sizeof(float)));
   P.rgb8 = nullptr; // RGB8 is written from the filtered image
   P.linear = c->d_linear;
   P.moments = c->d_moments;
@@ -1057,18 +1094,11 @@ rt_status rt_camera_render_denoised(rt_camera* c, const rt_region* region, uint8
   st = enqueue_render(c, P, nullptr, &launches);
   if (st != RT_OK) return st;
   const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
-  if (rw > 0 && rh > 0) {
-    const int n_feat = std::max(1, std::min(c->hs->cam.samples, 8));
-    CU(launch_render_features(c->ds, P, n_feat, c->d_falb, c->d_fnrm, c->d_fdepth, c->stream));
-    D.width = W;
-    D.x0 = P.x0; D.y0 = P.y0; D.x1 = P.x1; D.y1 = P.y1;
-    D.color = c->d_linear; D.albedo = c->d_falb; D.normal = c->d_fnrm; D.depth = c->d_fdepth; D.moments = c->d_moments;
-    dn_scratch(D, c->d_dn, npx);
-    D.out = c->d_linear;
-    D.rgb8 = rgb8 ? c->d_rgb8 : nullptr;
+  if (rw > 0 && rh > 0) { // one band: the whole region, filtered in place
     int dn_launches = 0;
-    CU(launch_denoise(D, c->stream, &dn_launches));
-    launches += 1 + dn_launches;
+    st = denoise_band(c, P, P.y0, P.y1, D, c->d_linear, c->d_moments, c->d_linear, rgb8 ? c->d_rgb8 : nullptr, false, &dn_launches);
+    if (st != RT_OK) return st;
+    launches += dn_launches;
   }
   CU(cudaEventRecord(c->ev1, c->stream));
   unsigned long long raw[kStatCount];
@@ -1145,9 +1175,39 @@ struct rt_multi {
   bool p2p = false;
   uint8_t* d_rgb8 = nullptr;    // on devices[0]
   float* d_linear = nullptr;
+  float* d_color = nullptr;     // on devices[0], rt_multi_render_denoised: the render's colour [H][W][3] and moments [H][W][8]
+  float* d_moments = nullptr;
   std::vector<cudaEvent_t> done;
+  std::vector<cudaEvent_t> rendered; // rt_multi_render_denoised: device k's render has landed in device 0's memory
   unsigned long long* h_stats = nullptr; // pinned [n][kStatCount]
 };
+
+// RenderStats.merge of one rt_multi call: work adds up, extremes combine; device_ms = the slowest device (host-merge path)
+static void merge_stats(const std::vector<rt_stats>& ps, rt_stats* out) {
+  std::memset(out, 0, sizeof(*out));
+  out->samples_min = out->bounces_min = 0x7fffffff;
+  for (const rt_stats& s : ps) {
+    out->pixels += s.pixels; out->samples_total += s.samples_total; out->bounces_total += s.bounces_total; out->rays += s.rays;
+    out->node_visits += s.node_visits; out->prim_tests += s.prim_tests;
+    out->samples_min = std::min(out->samples_min, s.samples_min); out->samples_max = std::max(out->samples_max, s.samples_max);
+    out->bounces_min = std::min(out->bounces_min, s.bounces_min); out->bounces_max = std::max(out->bounces_max, s.bounces_max);
+    out->device_ms = std::max(out->device_ms, s.device_ms); out->kernel_launches += s.kernel_launches;
+  }
+}
+// the same over the raw counters the peer-write path copies to m->h_stats (device_ms and kernel_launches are the caller's)
+static void merge_raw_stats(const rt_multi* m, rt_stats* out) {
+  unsigned long long raw[kStatCount];
+  std::memcpy(raw, kStatsInit, sizeof(raw));
+  for (size_t k = 0; k < m->cams.size(); ++k) {
+    const unsigned long long* r = m->h_stats + k * kStatCount;
+    raw[kStatPixels] += r[kStatPixels]; raw[kStatSamples] += r[kStatSamples]; raw[kStatBounces] += r[kStatBounces]; raw[kStatRays] += r[kStatRays];
+    raw[kStatNodeVisits] += r[kStatNodeVisits]; raw[kStatPrimTests] += r[kStatPrimTests];
+    raw[kStatSamplesMin] = std::min(raw[kStatSamplesMin], r[kStatSamplesMin]); raw[kStatSamplesMax] = std::max(raw[kStatSamplesMax], r[kStatSamplesMax]);
+    raw[kStatBouncesMin] = std::min(raw[kStatBouncesMin], r[kStatBouncesMin]); raw[kStatBouncesMax] = std::max(raw[kStatBouncesMax], r[kStatBouncesMax]);
+  }
+  std::memset(out, 0, sizeof(*out));
+  unpack_stats(raw, out);
+}
 
 static void free_multi(rt_multi* m) {
   if (!m) return;
@@ -1156,9 +1216,13 @@ static void free_multi(rt_multi* m) {
     DeviceGuard g(m->devices[0]);
     dev_free(m->d_rgb8);
     dev_free(m->d_linear);
+    dev_free(m->d_color);
+    dev_free(m->d_moments);
   }
   for (size_t k = 0; k < m->done.size(); ++k)
     if (m->done[k]) { DeviceGuard g(m->devices[k]); cudaEventDestroy(m->done[k]); }
+  for (size_t k = 0; k < m->rendered.size(); ++k)
+    if (m->rendered[k]) { DeviceGuard g(m->devices[k]); cudaEventDestroy(m->rendered[k]); }
   if (m->h_stats) cudaFreeHost(m->h_stats);
   delete m;
 }
@@ -1206,15 +1270,18 @@ rt_status rt_multi_create(const rt_scene_desc* scene, const rt_render_opts* opts
       if (st != RT_OK) { free_multi(m); return st; }
       m->cams.push_back(c);
       DeviceGuard g(m->devices[k]);
-      cudaEvent_t ev = nullptr;
+      cudaEvent_t ev = nullptr, ev_r = nullptr;
       // each device renders on its own non-blocking stream: the legacy default stream would serialise them
-      if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+      if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess ||
+          cudaEventCreateWithFlags(&ev_r, cudaEventDisableTiming) != cudaSuccess) {
+        if (ev) cudaEventDestroy(ev);
         const std::string msg = cudaGetErrorString(cudaGetLastError());
         free_multi(m);
         return fail(RT_ERR_CUDA, "rt_multi_create: stream/event: " + msg);
       }
       c->owns_stream = true;
       m->done.push_back(ev);
+      m->rendered.push_back(ev_r);
     }
     if (cudaMallocHost(&m->h_stats, sizeof(unsigned long long) * kStatCount * (size_t)n_devices) != cudaSuccess) {
       cudaGetLastError();
@@ -1264,16 +1331,7 @@ rt_status rt_multi_render_region(rt_multi* m, const rt_region* region, uint8_t* 
     for (auto& t : th) t.join();
     for (int k = 0; k < n; ++k)
       if (st[k] != RT_OK) return fail(st[k], msg[k]);
-    if (stats) {
-      stats->samples_min = stats->bounces_min = 0x7fffffff;
-      for (const rt_stats& s : ps) {
-        stats->pixels += s.pixels; stats->samples_total += s.samples_total; stats->bounces_total += s.bounces_total; stats->rays += s.rays;
-        stats->node_visits += s.node_visits; stats->prim_tests += s.prim_tests;
-        stats->samples_min = std::min(stats->samples_min, s.samples_min); stats->samples_max = std::max(stats->samples_max, s.samples_max);
-        stats->bounces_min = std::min(stats->bounces_min, s.bounces_min); stats->bounces_max = std::max(stats->bounces_max, s.bounces_max);
-        stats->device_ms = std::max(stats->device_ms, s.device_ms); stats->kernel_launches += s.kernel_launches;
-      }
-    }
+    if (stats) merge_stats(ps, stats);
     return RT_OK;
   }
   // ---- peer-write path ----
@@ -1314,24 +1372,159 @@ rt_status rt_multi_render_region(rt_multi* m, const rt_region* region, uint8_t* 
     CU(cudaStreamSynchronize(c0->stream));
   }
   if (stats) {
-    unsigned long long raw[kStatCount];
-    std::memcpy(raw, kStatsInit, sizeof(raw));
     double ms_max = 0;
     for (int k = 0; k < n; ++k) {
-      const unsigned long long* r = m->h_stats + (size_t)k * kStatCount;
-      raw[kStatPixels] += r[kStatPixels]; raw[kStatSamples] += r[kStatSamples]; raw[kStatBounces] += r[kStatBounces]; raw[kStatRays] += r[kStatRays];
-      raw[kStatNodeVisits] += r[kStatNodeVisits]; raw[kStatPrimTests] += r[kStatPrimTests];
-      raw[kStatSamplesMin] = std::min(raw[kStatSamplesMin], r[kStatSamplesMin]); raw[kStatSamplesMax] = std::max(raw[kStatSamplesMax], r[kStatSamplesMax]);
-      raw[kStatBouncesMin] = std::min(raw[kStatBouncesMin], r[kStatBouncesMin]); raw[kStatBouncesMax] = std::max(raw[kStatBouncesMax], r[kStatBouncesMax]);
       DeviceGuard g(m->cams[k]->device);
       float ms = 0;
       CU(cudaEventElapsedTime(&ms, m->cams[k]->ev0, m->cams[k]->ev1));
       ms_max = std::max(ms_max, (double)ms);
     }
-    unpack_stats(raw, stats);
+    merge_raw_stats(m, stats);
     stats->device_ms = ms_max; // the slowest device (they run concurrently)
     stats->kernel_launches = launches_total;
   }
+  return RT_OK;
+  RT_GUARD_END
+}
+
+// Denoised render on every device (include/rt_b200.h).  Peer-write path: every device renders its blocks' colour and
+// moments straight into device 0's d_color / d_moments, then, after every device's render, filters its band of the
+// region's rows (dn_halo's ghost zones, recomputed instead of exchanged) with prepare reading the colour and moments over
+// the peer mapping, and writes the band's rows of d_linear / d_rgb8 on device 0.  The output never aliases d_color: other
+// bands still read it.  Host-merge path: the colour and moments are merged on the host, and device 0 filters the region.
+// RT_B200_DENOISE_BANDS=n (development switch): n bands dealt to the devices in turn, each band's buffers filled with
+// NaN first, so that the band and halo logic runs, and a read outside a band's computed rows shows, on one GPU.
+rt_status rt_multi_render_denoised(rt_multi* m, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
+                                   const rt_denoise_opts* opts, rt_stats* stats) {
+  RT_GUARD_BEGIN
+  if (!m || m->cams.empty()) return fail(RT_ERR_INVALID_ARGUMENT, "null argument");
+  DenoiseParams D{};
+  rt_status st = dn_options(opts, D);
+  if (st != RT_OK) return st;
+  const int n = (int)m->cams.size();
+  rt_camera* c0 = m->cams[0];
+  const int W = c0->hs->image_width, H = c0->hs->image_height;
+  const size_t npx = (size_t)W * H;
+  if (rgb8 && rgb8_len < npx * 3) return fail(RT_ERR_BUFFER_TOO_SMALL, "rgb8 buffer smaller than width*height*3");
+  if (c0->hs->cam.mode != RT_MODE_DEFAULT) return fail(RT_ERR_UNSUPPORTED, "denoised renders need the default render mode");
+  RenderParams P0;
+  st = clip_region(c0, region, P0);
+  if (st != RT_OK) return st;
+  const int rw = P0.x1 - P0.x0, rh = P0.y1 - P0.y0;
+  int n_bands = n;
+  const char* bands_env = getenv("RT_B200_DENOISE_BANDS");
+  const bool poison = bands_env && atoi(bands_env) >= 1;
+  if (poison) n_bands = atoi(bands_env);
+  auto band = [&](int b, int& b0, int& b1) { // contiguous rows; some bands are empty when the region has fewer rows
+    b0 = P0.y0 + (int)((long long)b * rh / n_bands);
+    b1 = P0.y0 + (int)((long long)(b + 1) * rh / n_bands);
+  };
+  {
+    DeviceGuard g0(m->devices[0]);
+    if (!m->d_color) CU(dev_alloc(&m->d_color, npx * 3 * sizeof(float)));
+    if (!m->d_moments) CU(dev_alloc(&m->d_moments, npx * 8 * sizeof(float)));
+    if (!m->d_linear) CU(dev_alloc(&m->d_linear, npx * 3 * sizeof(float)));
+    if (rgb8 && !m->d_rgb8) CU(dev_alloc(&m->d_rgb8, npx * 3));
+  }
+  uint8_t* out8 = rgb8 ? m->d_rgb8 : nullptr;
+  int launches_total = 0;
+  if (!m->p2p && n > 1) {
+    // host merge: one thread per device renders its blocks' colour and moments into host arrays, device 0 filters
+    std::vector<float> hc(npx * 3), hm(npx * 8);
+    std::vector<rt_status> rs((size_t)n, RT_OK);
+    std::vector<std::string> msg((size_t)n);
+    std::vector<rt_stats> ps((size_t)n);
+    std::vector<std::thread> th;
+    for (int k = 0; k < n; ++k)
+      th.emplace_back([&, k]() {
+        rs[k] = render_host(m->cams[k], region, nullptr, 0, hc.data(), hm.data(), &ps[k]);
+        if (rs[k] != RT_OK) msg[k] = g_err;
+      });
+    for (auto& t : th) t.join();
+    for (int k = 0; k < n; ++k)
+      if (rs[k] != RT_OK) return fail(rs[k], msg[k]);
+    DeviceGuard g0(m->devices[0]);
+    CU(cudaEventRecord(c0->ev0, c0->stream));
+    if (rw > 0 && rh > 0) {
+      const size_t off = (size_t)P0.y0 * W + P0.x0;
+      CU(cudaMemcpy2DAsync(m->d_color + off * 3, (size_t)W * 12, hc.data() + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyHostToDevice, c0->stream));
+      CU(cudaMemcpy2DAsync(m->d_moments + off * 8, (size_t)W * 32, hm.data() + off * 8, (size_t)W * 32, (size_t)rw * 32, rh, cudaMemcpyHostToDevice, c0->stream));
+      for (int b = 0; b < n_bands; ++b) {
+        int b0, b1, l = 0;
+        band(b, b0, b1);
+        st = denoise_band(c0, P0, b0, b1, D, m->d_color, m->d_moments, m->d_linear, out8, poison, &l);
+        if (st != RT_OK) return st;
+        launches_total += l;
+      }
+    }
+    CU(cudaEventRecord(c0->ev1, c0->stream));
+    if (stats) {
+      merge_stats(ps, stats);
+      float ms = 0;
+      CU(cudaEventSynchronize(c0->ev1));
+      CU(cudaEventElapsedTime(&ms, c0->ev0, c0->ev1));
+      stats->device_ms += ms; // the slowest render, then the upload and the filter
+      stats->kernel_launches += launches_total;
+    }
+  } else {
+    // ---- peer-write path ----
+    std::vector<RenderParams> Ps((size_t)n);
+    for (int k = 0; k < n; ++k) {
+      rt_camera* c = m->cams[k];
+      DeviceGuard g(c->device);
+      RenderParams& P = Ps[k];
+      st = clip_region(c, region, P);
+      if (st != RT_OK) return st;
+      P.rgb8 = nullptr; // RGB8 is written from the filtered image
+      P.linear = m->d_color; // device 0's buffers, peer-mapped on device k
+      P.moments = m->d_moments;
+      int launches = 0;
+      CU(cudaEventRecord(c->ev0, c->stream));
+      st = enqueue_render(c, P, nullptr, &launches);
+      if (st != RT_OK) return st;
+      CU(cudaMemcpyAsync(m->h_stats + (size_t)k * kStatCount, c->d_stats, sizeof(unsigned long long) * kStatCount, cudaMemcpyDeviceToHost, c->stream));
+      CU(cudaEventRecord(m->rendered[k], c->stream));
+      launches_total += launches;
+    }
+    if (rw > 0 && rh > 0) {
+      for (int k = 0; k < n; ++k) { // a band's passes read rows other devices rendered
+        DeviceGuard g(m->cams[k]->device);
+        for (int j = 0; j < n; ++j)
+          if (j != k) CU(cudaStreamWaitEvent(m->cams[k]->stream, m->rendered[j], 0));
+      }
+      for (int b = 0; b < n_bands; ++b) {
+        rt_camera* c = m->cams[b % n];
+        DeviceGuard g(c->device);
+        int b0, b1, l = 0;
+        band(b, b0, b1);
+        st = denoise_band(c, Ps[b % n], b0, b1, D, m->d_color, m->d_moments, m->d_linear, out8, poison, &l);
+        if (st != RT_OK) return st;
+        launches_total += l;
+      }
+    }
+    for (int k = 1; k < n; ++k) {
+      DeviceGuard g(m->cams[k]->device);
+      CU(cudaEventRecord(m->done[k], m->cams[k]->stream));
+    }
+    DeviceGuard g0(m->devices[0]);
+    for (int k = 1; k < n; ++k) CU(cudaStreamWaitEvent(c0->stream, m->done[k], 0)); // every band has landed in device 0's memory
+    CU(cudaEventRecord(c0->ev1, c0->stream));
+    if (stats) {
+      CU(cudaEventSynchronize(c0->ev1));
+      float ms = 0;
+      CU(cudaEventElapsedTime(&ms, c0->ev0, c0->ev1));
+      merge_raw_stats(m, stats);
+      stats->device_ms = ms; // device 0, from its render to the last band's last kernel
+      stats->kernel_launches = launches_total;
+    }
+  }
+  DeviceGuard g0(m->devices[0]);
+  if (rw > 0 && rh > 0) {
+    const size_t off = (size_t)P0.y0 * W + P0.x0;
+    if (rgb8) CU(cudaMemcpy2DAsync(rgb8 + off * 3, (size_t)W * 3, m->d_rgb8 + off * 3, (size_t)W * 3, (size_t)rw * 3, rh, cudaMemcpyDeviceToHost, c0->stream));
+    if (linear) CU(cudaMemcpy2DAsync(linear + off * 3, (size_t)W * 12, m->d_linear + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c0->stream));
+  }
+  CU(cudaStreamSynchronize(c0->stream));
   return RT_OK;
   RT_GUARD_END
 }

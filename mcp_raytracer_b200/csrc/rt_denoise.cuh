@@ -59,12 +59,13 @@ __global__ void __launch_bounds__(256) k_render_features(const DevScene S, const
 constexpr float kDnAlbedoMin = 1e-3f; // demodulation floor
 RT_DEV float dn_lum(float r, float g, float b) { return 0.299f * r + 0.587f * g + 0.114f * b; } // the project's illuminance weights
 RT_DEV bool dn_finite3(const float* p) { return isfinite(p[0]) && isfinite(p[1]) && isfinite(p[2]); }
-// the filter kernels run 16x16 blocks and each thread strides over rows by the grid's height: CUDA caps gridDim.y at
-// 65535, so on an image taller than 65535 * 16 rows a thread filters more than one pixel of its column
+// the filter kernels run 16x16 blocks over the launch's window of rows and each thread strides over rows by the grid's
+// height: CUDA caps gridDim.y at 65535, so on a window taller than 65535 * 16 rows a thread filters more than one pixel of
+// its column
 constexpr int kDnBlock = 16;
 constexpr unsigned kDnMaxGridY = 65535;
 RT_DEV int dn_x(const DenoiseParams& D) { return D.x0 + (int)(blockIdx.x * blockDim.x + threadIdx.x); }
-RT_DEV int dn_y0(const DenoiseParams& D) { return D.y0 + (int)(blockIdx.y * blockDim.y + threadIdx.y); }
+RT_DEV int dn_y0(const DenoiseParams& D) { return D.wy0 + (int)(blockIdx.y * blockDim.y + threadIdx.y); }
 RT_DEV int dn_ystride() { return (int)(gridDim.y * blockDim.y); }
 RT_DEV bool dn_inside(const DenoiseParams& D, int x, int y) { return x >= D.x0 && x < D.x1 && y >= D.y0 && y < D.y1; }
 
@@ -114,7 +115,7 @@ RT_DEV void dn_prepare_pixel(const DenoiseParams& D, int x, int y) {
 __global__ void __launch_bounds__(256) k_denoise_prepare(const DenoiseParams D) {
   const int x = dn_x(D);
   if (x >= D.x1) return;
-  for (int y = dn_y0(D); y < D.y1; y += dn_ystride()) dn_prepare_pixel(D, x, y);
+  for (int y = dn_y0(D); y < D.wy1; y += dn_ystride()) dn_prepare_pixel(D, x, y);
 }
 
 // one a-trous pass with step 2^k: 5x5 B3-spline taps weighted by normal, depth and luminance edge stops
@@ -176,7 +177,7 @@ RT_DEV void dn_pass_pixel(const DenoiseParams& D, const F4* __restrict__ in, F4*
 __global__ void __launch_bounds__(256) k_denoise_pass(const DenoiseParams D, const F4* __restrict__ in, F4* __restrict__ out, int step) {
   const int x = dn_x(D);
   if (x >= D.x1) return;
-  for (int y = dn_y0(D); y < D.y1; y += dn_ystride()) dn_pass_pixel(D, in, out, step, x, y);
+  for (int y = dn_y0(D); y < D.wy1; y += dn_ystride()) dn_pass_pixel(D, in, out, step, x, y);
 }
 
 RT_DEV void dn_finish_pixel(const DenoiseParams& D, const F4* __restrict__ in, int x, int y) {
@@ -195,7 +196,7 @@ RT_DEV void dn_finish_pixel(const DenoiseParams& D, const F4* __restrict__ in, i
 __global__ void __launch_bounds__(256) k_denoise_finish(const DenoiseParams D, const F4* __restrict__ in) {
   const int x = dn_x(D);
   if (x >= D.x1) return;
-  for (int y = dn_y0(D); y < D.y1; y += dn_ystride()) dn_finish_pixel(D, in, x, y);
+  for (int y = dn_y0(D); y < D.wy1; y += dn_ystride()) dn_finish_pixel(D, in, x, y);
 }
 
 // launchers (called from rt_api.cu)
@@ -213,16 +214,28 @@ cudaError_t launch_render_features(const DevScene& S, const RenderParams& R, int
   return cudaGetLastError();
 }
 
-// prepare + `iterations` passes + finish; *launches = kernels enqueued
-cudaError_t launch_denoise(const DenoiseParams& D, cudaStream_t st, int* launches) {
+// prepare + `iterations` passes + finish of the rows [b0, b1) of the region: each stage computes the rows the next one
+// reads (dn_halo, rt_types.h); b0 = y0, b1 = y1 filters the whole region.  *launches = kernels enqueued
+cudaError_t launch_denoise(const DenoiseParams& D0, int b0, int b1, cudaStream_t st, int* launches) {
   *launches = 0;
-  if (D.x1 <= D.x0 || D.y1 <= D.y0) return cudaSuccess;
+  if (D0.x1 <= D0.x0 || b1 <= b0) return cudaSuccess;
+  DenoiseParams D = D0;
   const dim3 block(kDnBlock, kDnBlock, 1);
-  const unsigned rows = (unsigned)((D.y1 - D.y0 + kDnBlock - 1) / kDnBlock);
-  const dim3 grid((unsigned)((D.x1 - D.x0 + kDnBlock - 1) / kDnBlock), rows < kDnMaxGridY ? rows : kDnMaxGridY, 1);
+  const unsigned cols = (unsigned)((D.x1 - D.x0 + kDnBlock - 1) / kDnBlock);
+  auto window = [&](int h) { // rows [b0 - h, b1 + h) clipped to the region -> D.wy0 / D.wy1 and the launch grid
+    D.wy0 = std::max(D.y0, b0 - h);
+    D.wy1 = std::min(D.y1, b1 + h);
+    const unsigned rows = (unsigned)((D.wy1 - D.wy0 + kDnBlock - 1) / kDnBlock);
+    return dim3(cols, rows < kDnMaxGridY ? rows : kDnMaxGridY, 1);
+  };
+  dim3 grid = window(dn_halo(D.iterations, -1));
   k_denoise_prepare<<<grid, block, 0, st>>>(D);
   int cur = 0;
-  for (int k = 0; k < D.iterations; ++k, cur ^= 1) k_denoise_pass<<<grid, block, 0, st>>>(D, D.buf[cur], D.buf[cur ^ 1], 1 << k);
+  for (int k = 0; k < D.iterations; ++k, cur ^= 1) {
+    grid = window(dn_halo(D.iterations, k));
+    k_denoise_pass<<<grid, block, 0, st>>>(D, D.buf[cur], D.buf[cur ^ 1], 1 << k);
+  }
+  grid = window(0);
   k_denoise_finish<<<grid, block, 0, st>>>(D, D.buf[cur]);
   *launches = D.iterations + 2;
   return cudaGetLastError();

@@ -197,9 +197,11 @@ static_assert(sizeof(PixState) == 40 && offsetof(PixState, samples) == 12 && off
               "adstate_load / adstate_store (rt_megakernel.cu) move a PixState as five 64-bit words");
 // ---- denoiser (rt_denoise.cuh): one filter launch sequence over the pixels of a region ----
 // Every buffer is indexed by whole-image pixel (y * width + x); only pixels inside [x0, x1) x [y0, y1) are read or written.
+// A launch computes the rows [wy0, wy1) of the region (its window); taps and gradients test the region, not the window.
 struct DenoiseParams {
   int width;
   int x0, y0, x1, y1;
+  int wy0, wy1;
   const float* color;   // [H][W][3] linear colour (the pixel mean)
   const float* albedo;  // [H][W][3] feature albedo
   const float* normal;  // [H][W][3] feature normal (zero on a miss)
@@ -210,9 +212,14 @@ struct DenoiseParams {
   float* grad;          // [H][W][2] depth gradient
   int iterations;
   float sigma_l, sigma_n, sigma_z;
-  float* out;           // [H][W][3] linear result; may be `color` (both are read and written pixel by pixel)
+  float* out;           // [H][W][3] linear result; may be `color` when one band covers the region (read and written pixel by pixel)
   uint8_t* rgb8;        // [H][W][3] or null
 };
+// Filtering a band of rows [b0, b1) on its own (ghost zones, no exchange between passes): pass k (step 2^k) reads up to
+// 2^(k+1) rows away (taps at +-2 * 2^k, the variance blur at +-1), so of K passes, pass k computes h = 2^(K+1) - 2^(k+2)
+// rows beyond each side of the band and the last pass exactly the band.  stage -1 = prepare: 2^(K+1) - 2 rows; the
+// features are needed one row further (the depth gradient reads +-1).  Every window is clipped to the region.
+inline int dn_halo(int iterations, int stage) { return (1 << (iterations + 1)) - (1 << (stage + 2)); }
 // ---- wavefront integrator (rt_wavefront.cuh): path pool + queues in HBM ----
 struct U2 { uint32_t x, y; };
 enum : int { WF_TAGS = 3 };

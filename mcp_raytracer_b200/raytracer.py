@@ -3,7 +3,9 @@ by native dispatch (the seam SURVEY.md §8b names).
 
 * `generateImageBuffer(sceneConfig, options)`  <- src/raytracer.ts:39-113
     options.parallel=False : `camera.render(pixelData)`            (raytracer.ts:56-59)
-    options.denoise=True or {iterations, sigma*}: `camera.renderDenoised(pixelData)` on one GPU (not in the reference)
+    options.denoise=True or {iterations, sigma*}: `camera.renderDenoised(pixelData)` (not in the reference); with
+                             parallel=True on more than one GPU `MultiCamera.renderDenoised`: every device renders its
+                             blocks and filters a band of rows, the same bytes as on one GPU
     options.parallel=True  : the image is split over GPUs instead of worker threads
                              (raytracer.ts:60-90): `MultiCamera` (rt_multi_* of the C ABI) compiles
                              the scene once, every visible device renders its interleaved set of 8x4
@@ -71,10 +73,18 @@ def renderScene(sceneConfig: Dict[str, Any], options: Optional[Dict[str, Any]] =
     ndev = _native.lib().rt_device_count()
     threads = options.get("threads") or ndev  # "threads" = number of GPUs here
     dn = options.get("denoise")
-    if dn:
-        # the filter reads every pixel's neighbours, so a denoised image is rendered on ONE GPU even when `parallel` is set
+    if dn and parallel and min(threads, ndev) > 1:
+        threads = min(threads, ndev)
         if verbose:
-            print("Denoising: rendering on one GPU" + (" (parallel ignored)" if parallel else ""), file=sys.stderr)
+            print(f"Denoising: rendering and filtering on {threads} GPUs", file=sys.stderr)
+        # every device renders its blocks, then filters a band of rows: the bytes of the one-GPU denoiser
+        with MultiCamera(sceneData, render, nDevices=threads) as camera:
+            W, H = camera.imageWidth, camera.imageHeight
+            pixelData = np.zeros(W * H * 3, np.uint8)
+            stats = camera.renderDenoised(pixelData, options=None if dn is True else dn)
+    elif dn:
+        if verbose:
+            print("Denoising: rendering on one GPU", file=sys.stderr)
         with createCameraFromSceneData(sceneData, render) as camera:
             W, H = camera.imageWidth, camera.imageHeight
             pixelData = np.zeros(W * H * 3, np.uint8)

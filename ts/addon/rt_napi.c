@@ -13,7 +13,7 @@
  *   renderRegion(handle, region, pixelData) -> stats            rt_camera_render_region / rt_multi_render_region, synchronous
  *   renderRegionAsync(handle, region, pixelData) -> Promise     same on a libuv worker (napi_async_work): keeps the event loop
  *                                                               free, like the reference's worker threads (src/raytracer.ts:60-90)
- *   renderDenoised(handle, region, pixelData, options?) -> stats rt_camera_render_denoised (one-GPU cameras), synchronous;
+ *   renderDenoised(handle, region, pixelData, options?) -> stats rt_camera_render_denoised / rt_multi_render_denoised, synchronous;
  *                                                               options {iterations, sigmaLuminance, sigmaNormal, sigmaDepth}
  *   cameraInfo(handle) -> { imageWidth, imageHeight, ... }      rt_camera_get_info / rt_multi_get_info
  *   destroyCamera(handle)                                       rt_camera_destroy / rt_multi_destroy — releases the GPU memory NOW
@@ -205,7 +205,6 @@ static napi_value RenderDenoised(napi_env env, napi_callback_info info) {
   CHECK(env, napi_get_cb_info(env, info, &argc, argv, NULL, NULL));
   if (argc < 3) return throw_msg(env, "renderDenoised(handle, region, pixelData, options?)");
   if (!(b = get_box(env, argv[0]))) return NULL;
-  if (!b->cam) return throw_msg(env, "renderDenoised renders on one GPU: create the camera with createCamera");
   if (b->busy) return throw_msg(env, "an asynchronous render is in flight on this camera");
   if (!read_region(env, argv[1], &reg)) return throw_msg(env, "region must be {x, y, width, height}");
   CHECK(env, napi_get_typedarray_info(env, argv[2], &ty, &len, &data, &ab, &off));
@@ -217,7 +216,9 @@ static napi_value RenderDenoised(napi_env env, napi_callback_info info) {
     o.sigma_normal = (float)num_field(env, argv[3], "sigmaNormal", 0);
     o.sigma_depth = (float)num_field(env, argv[3], "sigmaDepth", 0);
   }
-  if (rt_camera_render_denoised(b->cam, &reg, (uint8_t*)data, len, NULL, &o, &st) != RT_OK) return throw_rt(env);
+  if ((b->cam ? rt_camera_render_denoised(b->cam, &reg, (uint8_t*)data, len, NULL, &o, &st)
+              : rt_multi_render_denoised(b->multi, &reg, (uint8_t*)data, len, NULL, &o, &st)) != RT_OK)
+    return throw_rt(env);
   return stats_object(env, &st);
 }
 

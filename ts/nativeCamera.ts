@@ -130,7 +130,8 @@ export class NativeCamera {
   async renderAsync(pixelData: Uint8ClampedArray): Promise<RenderStats> {
     return NativeCamera.stats(await addon.renderRegionAsync(this.handle, { x: 0, y: 0, width: this.imageWidth, height: this.imageHeight }, pixelData));
   }
-  /** Render, then denoise on the device (rt_camera_render_denoised; one-GPU cameras only).  Not in the reference. */
+  /** Render, then denoise on the device (rt_camera_render_denoised; `multi`: rt_multi_render_denoised, every GPU renders its
+   *  blocks and filters a band of rows, the same bytes as on one GPU).  Not in the reference. */
   renderDenoised(pixelData: Uint8ClampedArray, region?: RenderRegion, options: DenoiseOptions = {}): RenderStats {
     return NativeCamera.stats(addon.renderDenoised(this.handle, region ?? { x: 0, y: 0, width: this.imageWidth, height: this.imageHeight },
                                                    pixelData, options));
