@@ -92,6 +92,23 @@ class RenderStats:
         return m
 
 
+def _check(st: int) -> None:
+    """Raise RaytracerError for a failed library call (a non-zero rt_status), with the library's message."""
+    if st != 0:
+        raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
+
+
+def _image_outputs(rgb8: Optional[np.ndarray], linear: Optional[np.ndarray], W: int, H: int):
+    """Check the RGB8 and linear output arrays of a render of a W x H image (None = not wanted): the library writes them
+    through their base pointers as C-contiguous [H][W][3] arrays.  Returns (rgb8 pointer, rgb8 bytes, linear pointer)."""
+    if rgb8 is not None and (rgb8.dtype != np.uint8 or not rgb8.flags["C_CONTIGUOUS"]):
+        raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
+    if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3 or not linear.flags["C_CONTIGUOUS"]):
+        raise RaytracerError("linear buffer must be float32 [H][W][3]")
+    return (rgb8.ctypes.data if rgb8 is not None else None, rgb8.nbytes if rgb8 is not None else 0,
+            linear.ctypes.data if linear is not None else None)
+
+
 def _region_struct(region: Optional[Dict[str, int]], W: int, H: int) -> rt_region:
     if region is None:
         return rt_region(0, 0, W, H)
@@ -114,9 +131,7 @@ class Camera:
         self._opts = render_opts_struct(self.options)
         L = _native.lib()
         h = C.c_void_p()
-        st = L.rt_camera_create(C.byref(self._flat.desc), C.byref(self._opts), C.byref(h))
-        if st != 0:
-            raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
+        _check(L.rt_camera_create(C.byref(self._flat.desc), C.byref(self._opts), C.byref(h)))
         self._h = h
         info = rt_camera_info()
         L.rt_camera_get_info(self._h, C.byref(info))
@@ -153,34 +168,23 @@ class Camera:
     def __exit__(self, *a):
         self.close()
 
-    def _check(self, st: int) -> None:
-        if st != 0:
-            raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
-
     def setStream(self, cuda_stream: int) -> None:
-        self._check(_native.lib().rt_camera_set_stream(self._h, C.c_void_p(cuda_stream)))
+        _check(_native.lib().rt_camera_set_stream(self._h, C.c_void_p(cuda_stream)))
 
     # -- the hot path --
     def renderRegion(self, buffer: np.ndarray, region: Optional[Dict[str, int]], linear: Optional[np.ndarray] = None,
                      moments: Optional[np.ndarray] = None) -> RenderStats:
         W, H = self.imageWidth, self.imageHeight
-        if buffer is not None:
-            if buffer.dtype != np.uint8 or not buffer.flags["C_CONTIGUOUS"]:
-                raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
+        bp, bl, lp = _image_outputs(buffer, linear, W, H)
         reg = _region_struct(region, W, H)
         st = rt_stats()
-        bp = buffer.ctypes.data if buffer is not None else None
-        bl = buffer.nbytes if buffer is not None else 0
-        lp = linear.ctypes.data if linear is not None else None
-        if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3):
-            raise RaytracerError("linear buffer must be float32 [H][W][3]")
         L = _native.lib()
         if moments is not None:
             if moments.dtype != np.float32 or moments.size < W * H * 8:
                 raise RaytracerError("moments buffer must be float32 [H][W][8]")
-            self._check(L.rt_camera_render_moments(self._h, C.byref(reg), bp, bl, lp, moments.ctypes.data, C.byref(st)))
+            _check(L.rt_camera_render_moments(self._h, C.byref(reg), bp, bl, lp, moments.ctypes.data, C.byref(st)))
         else:
-            self._check(L.rt_camera_render_region(self._h, C.byref(reg), bp, bl, lp, C.byref(st)))
+            _check(L.rt_camera_render_region(self._h, C.byref(reg), bp, bl, lp, C.byref(st)))
         return RenderStats.from_struct(st)
 
     def render(self, pixelData: np.ndarray, linear: Optional[np.ndarray] = None) -> RenderStats:
@@ -192,10 +196,7 @@ class Camera:
         onPass(pass, passes, samplesCap, RenderStats) is called after each pass with `pixelData` refreshed; return True to
         stop early.  The reference has no preview surface (SURVEY.md section 8f row 2)."""
         W, H = self.imageWidth, self.imageHeight
-        if pixelData is not None and (pixelData.dtype != np.uint8 or not pixelData.flags["C_CONTIGUOUS"]):
-            raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
-        if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3):
-            raise RaytracerError("linear buffer must be float32 [H][W][3]")
+        bp, bl, lp = _image_outputs(pixelData, linear, W, H)
         reg = _region_struct(region, W, H)
         st = rt_stats()
         errors: List[BaseException] = []
@@ -210,9 +211,8 @@ class Camera:
                 errors.append(e)
                 return 1
 
-        self._check(_native.lib().rt_camera_render_progressive(
-            self._h, C.byref(reg), pixelData.ctypes.data if pixelData is not None else None, pixelData.nbytes if pixelData is not None else 0,
-            linear.ctypes.data if linear is not None else None, int(passes), C.cast(cb, C.c_void_p), None, C.byref(st)))
+        _check(_native.lib().rt_camera_render_progressive(self._h, C.byref(reg), bp, bl, lp, int(passes), C.cast(cb, C.c_void_p), None,
+                                                          C.byref(st)))
         if errors:
             raise errors[0]
         return RenderStats.from_struct(st)
@@ -221,7 +221,7 @@ class Camera:
         """Enqueue on the camera's stream; device pointers; no synchronisation."""
         reg = _region_struct(region, self.imageWidth, self.imageHeight)
         vp = lambda p: C.c_void_p(p) if p else None  # noqa: E731
-        self._check(_native.lib().rt_camera_render_region_device(self._h, C.byref(reg), vp(rgb8_ptr), vp(linear_ptr),
+        _check(_native.lib().rt_camera_render_region_device(self._h, C.byref(reg), vp(rgb8_ptr), vp(linear_ptr),
                                                                  vp(moments_ptr), vp(stats_ptr)))
 
     # -- parity hook --
@@ -232,7 +232,7 @@ class Camera:
         t = np.zeros((H, W), np.float32)
         nrm = np.zeros((H, W, 3), np.float32)
         ff = np.zeros((H, W), np.uint8)
-        self._check(_native.lib().rt_camera_trace_primary(self._h, C.byref(reg), ids.ctypes.data, t.ctypes.data,
+        _check(_native.lib().rt_camera_trace_primary(self._h, C.byref(reg), ids.ctypes.data, t.ctypes.data,
                                                           nrm.ctypes.data, ff.ctypes.data))
         return ids, t, nrm, ff
 
@@ -245,7 +245,7 @@ class Camera:
         alb = np.zeros((H, W, 3), np.float32)
         nrm = np.zeros((H, W, 3), np.float32)
         dep = np.zeros((H, W), np.float32)
-        self._check(_native.lib().rt_camera_render_features(self._h, C.byref(reg), int(nSamples), alb.ctypes.data, nrm.ctypes.data,
+        _check(_native.lib().rt_camera_render_features(self._h, C.byref(reg), int(nSamples), alb.ctypes.data, nrm.ctypes.data,
                                                             dep.ctypes.data))
         return {"albedo": alb, "normal": nrm, "depth": dep}
 
@@ -254,16 +254,11 @@ class Camera:
         """Render, then denoise on the device (rt_camera_render_denoised): `pixelData` / `linear` receive the filtered image.
         options: {iterations, sigmaLuminance, sigmaNormal, sigmaDepth}; absent = defaults."""
         W, H = self.imageWidth, self.imageHeight
-        if pixelData is not None and (pixelData.dtype != np.uint8 or not pixelData.flags["C_CONTIGUOUS"]):
-            raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
-        if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3 or not linear.flags["C_CONTIGUOUS"]):
-            raise RaytracerError("linear buffer must be float32 [H][W][3]")
+        bp, bl, lp = _image_outputs(pixelData, linear, W, H)
         reg = _region_struct(region, W, H)
         opts = denoise_opts_struct(options)
         st = rt_stats()
-        self._check(_native.lib().rt_camera_render_denoised(
-            self._h, C.byref(reg), pixelData.ctypes.data if pixelData is not None else None, pixelData.nbytes if pixelData is not None else 0,
-            linear.ctypes.data if linear is not None else None, C.byref(opts), C.byref(st)))
+        _check(_native.lib().rt_camera_render_denoised(self._h, C.byref(reg), bp, bl, lp, C.byref(opts), C.byref(st)))
         return RenderStats.from_struct(st)
 
     # -- per-function parity hooks (rt_debug_*): one device function of the render path on explicit inputs --
@@ -287,7 +282,7 @@ class Camera:
         hits[:, 12] = ff.view(np.float64).reshape(n)
         u = self._uniforms(uniforms, n)
         out = np.zeros((n, 11), np.float32)  # rt_debug_scatter_out: 2 int32 + 9 float
-        self._check(_native.lib().rt_debug_scatter(self._h, int(objectIndex), n, hits.ctypes.data, u.ctypes.data, out.ctypes.data))
+        _check(_native.lib().rt_debug_scatter(self._h, int(objectIndex), n, hits.ctypes.data, u.ctypes.data, out.ctypes.data))
         ints = out[:, 0:2].copy().view(np.int32)
         return {"kind": ints[:, 0], "used": ints[:, 1], "attenuation": out[:, 2:5], "dir": out[:, 5:8], "emitted": out[:, 8:11]}
 
@@ -298,20 +293,20 @@ class Camera:
         u = self._uniforms(uniforms, n)
         out = np.zeros((n, 6), np.float32)
         used = np.zeros(n, np.int32)
-        self._check(_native.lib().rt_debug_get_ray(self._h, n, a.ctypes.data, u.ctypes.data, out.ctypes.data, used.ctypes.data))
+        _check(_native.lib().rt_debug_get_ray(self._h, n, a.ctypes.data, u.ctypes.data, out.ctypes.data, used.ctypes.data))
         return out[:, 0:3], out[:, 3:6], used
 
     def debugLightPdf(self, lightIndex: int, origin, direction) -> np.ndarray:
         o, d = (np.ascontiguousarray(np.atleast_2d(x), np.float64) for x in (origin, direction))
         out = np.zeros(o.shape[0], np.float32)
-        self._check(_native.lib().rt_debug_light_pdf(self._h, int(lightIndex), o.shape[0], o.ctypes.data, d.ctypes.data, out.ctypes.data))
+        _check(_native.lib().rt_debug_light_pdf(self._h, int(lightIndex), o.shape[0], o.ctypes.data, d.ctypes.data, out.ctypes.data))
         return out
 
     def debugLightRandomVec(self, lightIndex: int, origin, uniforms) -> np.ndarray:
         o = np.ascontiguousarray(np.atleast_2d(origin), np.float64)
         u = self._uniforms(uniforms, o.shape[0])
         out = np.zeros((o.shape[0], 3), np.float32)
-        self._check(_native.lib().rt_debug_light_random_vec(self._h, int(lightIndex), o.shape[0], o.ctypes.data, u.ctypes.data, out.ctypes.data))
+        _check(_native.lib().rt_debug_light_random_vec(self._h, int(lightIndex), o.shape[0], o.ctypes.data, u.ctypes.data, out.ctypes.data))
         return out
 
     def debugDiffuseBounce(self, p, normal, uniforms) -> np.ndarray:
@@ -319,7 +314,7 @@ class Camera:
         pp, nn = (np.ascontiguousarray(np.atleast_2d(x), np.float64) for x in (p, normal))
         u = self._uniforms(uniforms, pp.shape[0])
         out = np.zeros((pp.shape[0], 6), np.float32)
-        self._check(_native.lib().rt_debug_diffuse_bounce(self._h, pp.shape[0], pp.ctypes.data, nn.ctypes.data, u.ctypes.data, out.ctypes.data))
+        _check(_native.lib().rt_debug_diffuse_bounce(self._h, pp.shape[0], pp.ctypes.data, nn.ctypes.data, u.ctypes.data, out.ctypes.data))
         return out
 
 
@@ -338,9 +333,7 @@ class MultiCamera:
         L = _native.lib()
         h = C.c_void_p()
         dev = (C.c_int32 * len(devices))(*devices) if devices else None
-        st = L.rt_multi_create(C.byref(self._flat.desc), C.byref(self._opts), len(devices) if devices else int(nDevices), dev, C.byref(h))
-        if st != 0:
-            raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
+        _check(L.rt_multi_create(C.byref(self._flat.desc), C.byref(self._opts), len(devices) if devices else int(nDevices), dev, C.byref(h)))
         self._h = h
         info, n, p2p = rt_camera_info(), C.c_int32(), C.c_int32()
         L.rt_multi_get_info(self._h, C.byref(info), C.byref(n), C.byref(p2p))
@@ -367,17 +360,10 @@ class MultiCamera:
 
     def renderRegion(self, buffer: np.ndarray, region: Optional[Dict[str, int]], linear: Optional[np.ndarray] = None) -> RenderStats:
         W, H = self.imageWidth, self.imageHeight
-        if buffer is not None and (buffer.dtype != np.uint8 or not buffer.flags["C_CONTIGUOUS"]):
-            raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
-        if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3):
-            raise RaytracerError("linear buffer must be float32 [H][W][3]")
+        bp, bl, lp = _image_outputs(buffer, linear, W, H)
         reg = _region_struct(region, W, H)
         st = rt_stats()
-        rc = _native.lib().rt_multi_render_region(self._h, C.byref(reg), buffer.ctypes.data if buffer is not None else None,
-                                                  buffer.nbytes if buffer is not None else 0,
-                                                  linear.ctypes.data if linear is not None else None, C.byref(st))
-        if rc != 0:
-            raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(rc, rc)}]")
+        _check(_native.lib().rt_multi_render_region(self._h, C.byref(reg), bp, bl, lp, C.byref(st)))
         return RenderStats.from_struct(st)
 
     def render(self, pixelData: np.ndarray, linear: Optional[np.ndarray] = None) -> RenderStats:
@@ -388,18 +374,11 @@ class MultiCamera:
         """`Camera.renderDenoised` on every device (rt_multi_render_denoised): the same bytes as one Camera's.  Each device
         filters a band of the region's rows after every device has rendered."""
         W, H = self.imageWidth, self.imageHeight
-        if pixelData is not None and (pixelData.dtype != np.uint8 or not pixelData.flags["C_CONTIGUOUS"]):
-            raise RaytracerError("pixel buffer must be a C-contiguous uint8 array")
-        if linear is not None and (linear.dtype != np.float32 or linear.size < W * H * 3 or not linear.flags["C_CONTIGUOUS"]):
-            raise RaytracerError("linear buffer must be float32 [H][W][3]")
+        bp, bl, lp = _image_outputs(pixelData, linear, W, H)
         reg = _region_struct(region, W, H)
         opts = denoise_opts_struct(options)
         st = rt_stats()
-        rc = _native.lib().rt_multi_render_denoised(
-            self._h, C.byref(reg), pixelData.ctypes.data if pixelData is not None else None, pixelData.nbytes if pixelData is not None else 0,
-            linear.ctypes.data if linear is not None else None, C.byref(opts), C.byref(st))
-        if rc != 0:
-            raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(rc, rc)}]")
+        _check(_native.lib().rt_multi_render_denoised(self._h, C.byref(reg), bp, bl, lp, C.byref(opts), C.byref(st)))
         return RenderStats.from_struct(st)
 
 
@@ -428,18 +407,14 @@ def denoise(color, albedo, normal, depth, moments, options: Optional[Dict[str, A
             raise RaytracerError(f"{name} must have shape {shapes[name]}, not {arrs[name].shape}")
     opts = denoise_opts_struct(options)
     out = np.zeros((H, W, 3), np.float32)
-    st = _native.lib().rt_denoise(int(device), W, H, c.ctypes.data, arrs["albedo"].ctypes.data, arrs["normal"].ctypes.data,
-                                  arrs["depth"].ctypes.data, arrs["moments"].ctypes.data, C.byref(opts), out.ctypes.data)
-    if st != 0:
-        raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
+    _check(_native.lib().rt_denoise(int(device), W, H, c.ctypes.data, arrs["albedo"].ctypes.data, arrs["normal"].ctypes.data,
+                                    arrs["depth"].ctypes.data, arrs["moments"].ctypes.data, C.byref(opts), out.ctypes.data))
     return out
 
 
 def measureFp32Peak(device: int = -1):
     t, mhz = C.c_double(), C.c_double()
-    st = _native.lib().rt_measure_fp32_peak(device, C.byref(t), C.byref(mhz))
-    if st != 0:
-        raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
+    _check(_native.lib().rt_measure_fp32_peak(device, C.byref(t), C.byref(mhz)))
     return t.value, mhz.value
 
 
@@ -454,9 +429,7 @@ def validateScene(sceneData: Dict[str, Any], renderOptions: Optional[Dict[str, A
     flat = FlatScene(sceneData)
     opts = render_opts_struct(merge_render_options(flat.render, renderOptions))
     rep = _SceneReport()
-    st = _native.lib().rt_scene_validate(C.byref(flat.desc), C.byref(opts), C.byref(rep))
-    if st != 0:
-        raise RaytracerError(f"{_native.last_error()} [{_native.STATUS_NAMES.get(st, st)}]")
+    _check(_native.lib().rt_scene_validate(C.byref(flat.desc), C.byref(opts), C.byref(rep)))
     return {n: int(getattr(rep, n)) for n, _ in _SceneReport._fields_ if n != "reserved"}
 
 

@@ -9,6 +9,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <memory>
 #include <thread>
@@ -253,17 +254,51 @@ static rt_status clip_region(const rt_camera* c, const rt_region* r, RenderParam
 
 static const unsigned long long kStatsInit[kStatCount] = {0, 0, 0, 0, 0x7fffffffull, 0, 0x7fffffffull, 0, 0, 0};
 
-static void unpack_stats(const unsigned long long* raw, rt_stats* s) {
-  s->pixels = raw[kStatPixels];
-  s->samples_total = raw[kStatSamples];
-  s->bounces_total = raw[kStatBounces];
-  s->rays = raw[kStatRays];
-  s->samples_min = (int32_t)raw[kStatSamplesMin];
-  s->samples_max = (int32_t)raw[kStatSamplesMax];
-  s->bounces_min = (int32_t)raw[kStatBouncesMin];
-  s->bounces_max = (int32_t)raw[kStatBouncesMax];
-  s->node_visits = raw[kStatNodeVisits];
-  s->prim_tests = raw[kStatPrimTests];
+// Raw counters -> rt_stats without timing or launches.  unpack_stats(kStatsInit) is the identity of merge_stats.
+static rt_stats unpack_stats(const unsigned long long* raw) {
+  rt_stats s;
+  std::memset(&s, 0, sizeof(s));
+  s.pixels = raw[kStatPixels];
+  s.samples_total = raw[kStatSamples];
+  s.bounces_total = raw[kStatBounces];
+  s.rays = raw[kStatRays];
+  s.samples_min = (int32_t)raw[kStatSamplesMin];
+  s.samples_max = (int32_t)raw[kStatSamplesMax];
+  s.bounces_min = (int32_t)raw[kStatBouncesMin];
+  s.bounces_max = (int32_t)raw[kStatBouncesMax];
+  s.node_visits = raw[kStatNodeVisits];
+  s.prim_tests = raw[kStatPrimTests];
+  return s;
+}
+
+// RenderStats.merge: work and kernel launches add up, extremes combine.  device_ms is each caller's own rule.
+static void merge_stats(rt_stats* total, const rt_stats& s) {
+  total->pixels += s.pixels; total->samples_total += s.samples_total; total->bounces_total += s.bounces_total; total->rays += s.rays;
+  total->node_visits += s.node_visits; total->prim_tests += s.prim_tests;
+  total->samples_min = std::min(total->samples_min, s.samples_min); total->samples_max = std::max(total->samples_max, s.samples_max);
+  total->bounces_min = std::min(total->bounces_min, s.bounces_min); total->bounces_max = std::max(total->bounces_max, s.bounces_max);
+  total->kernel_launches += s.kernel_launches;
+}
+
+// Copy the region of P out of (or into) an [H][W] image of `k` bytes per pixel: `dst` and `src` have that same layout.
+static cudaError_t copy_region(void* dst, const void* src, size_t k, const RenderParams& P, int W, cudaMemcpyKind kind, cudaStream_t st) {
+  if (P.x1 <= P.x0 || P.y1 <= P.y0) return cudaSuccess;
+  const size_t off = ((size_t)P.y0 * W + P.x0) * k, pitch = (size_t)W * k;
+  return cudaMemcpy2DAsync((char*)dst + off, pitch, (const char*)src + off, pitch, (size_t)(P.x1 - P.x0) * k, P.y1 - P.y0, kind, st);
+}
+
+// Grow-only device buffer of the camera: at least `need` elements.  Work in flight may still use the old block, so the
+// camera's stream is drained before it goes back to the cache.
+template <class T, class N>
+static rt_status grow(rt_camera* c, T*& buf, N& capacity, size_t need) {
+  if (need <= (size_t)capacity) return RT_OK;
+  CU(cudaStreamSynchronize(c->stream));
+  dev_free(buf);
+  buf = nullptr;
+  capacity = 0;
+  CU(dev_alloc(&buf, need * sizeof(T)));
+  capacity = (N)need;
+  return RT_OK;
 }
 
 extern "C" {
@@ -588,13 +623,8 @@ static rt_status wf_prepare(rt_camera* c, const RenderParams& P) {
     }
     c->wf_ready = true;
   }
-  if ((int)owned.size() > H.owned_capacity) {
-    CU(cudaStreamSynchronize(c->stream));
-    dev_free(H.owned_blocks);
-    H.owned_blocks = nullptr;
-    CU(dev_alloc(&H.owned_blocks, std::max<size_t>(owned.size(), 1) * sizeof(int)));
-    H.owned_capacity = (int)owned.size();
-  }
+  rt_status st = grow(c, H.owned_blocks, H.owned_capacity, owned.size());
+  if (st != RT_OK) return st;
   if (!owned.empty()) { // on the camera's stream (a user stream may be non-blocking: the legacy default stream does not order with it)
     CU(cudaMemcpyAsync(H.owned_blocks, owned.data(), owned.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     CU(cudaStreamSynchronize(c->stream)); // `owned` is a pageable local
@@ -657,38 +687,20 @@ static rt_status enqueue_render(rt_camera* c, RenderParams& P, rt_stats* stats_d
       const int gb = pass ? 0 : render_adaptive_blocks(c->ds, P, c->sms, &warps);
       if (gb > 0) {
         if (!c->d_pixstate) CU(dev_alloc(&c->d_pixstate, (size_t)c->hs->image_width * c->hs->image_height * sizeof(PixState)));
-        const size_t need_r = (size_t)warps * gb * 32 * (size_t)c->hs->cam.a_batch;
-        if (need_r > c->adrec_elems) {
-          CU(cudaStreamSynchronize(c->stream));
-          dev_free(c->d_adrec);
-          c->d_adrec = nullptr;
-          c->adrec_elems = 0;
-          CU(dev_alloc(&c->d_adrec, need_r * sizeof(AdRecord)));
-          c->adrec_elems = need_r;
-        }
+        rt_status st = grow(c, c->d_adrec, c->adrec_elems, (size_t)warps * gb * 32 * (size_t)c->hs->cam.a_batch);
+        if (st != RT_OK) return st;
         P.adstate = c->d_pixstate;
         P.adrec = c->d_adrec;
         P.ad_blocks = gb;
       }
     }
     const size_t need_q = 1 + std::max((size_t)P.tiles_x * P.tiles_y * 8, (size_t)P.n_runs); // queue head + one completion counter per 8x4 block / run
-    if (need_q > c->queue_ints) {
-      CU(cudaStreamSynchronize(c->stream));
-      dev_free(c->d_queue);
-      c->d_queue = nullptr;
-      CU(dev_alloc(&c->d_queue, need_q * sizeof(int)));
-      c->queue_ints = need_q;
-    }
+    rt_status st = grow(c, c->d_queue, c->queue_ints, need_q);
+    if (st != RT_OK) return st;
     // fixed-point radiance sums [H][W][4] u64, only when a pixel's samples are split over CTAs
     const bool wavefront = c->integrator == RT_INTEGRATOR_WAVEFRONT && !render_needs_full(c->ds, P) && !pass; // passes: megakernel layouts only
     const size_t need_s = (P.chunks > 1 || wavefront || P.keep_accum) ? (size_t)4 * c->hs->image_width * c->hs->image_height : 0;
-    if (need_s > c->scratch_elems) {
-      CU(cudaStreamSynchronize(c->stream));
-      dev_free(c->d_scratch);
-      c->d_scratch = nullptr;
-      CU(dev_alloc(&c->d_scratch, need_s * sizeof(unsigned long long)));
-      c->scratch_elems = need_s;
-    }
+    if ((st = grow(c, c->d_scratch, c->scratch_elems, need_s)) != RT_OK) return st;
     CU(cudaMemsetAsync(c->d_queue, 0, need_q * sizeof(int), c->stream));
     if (need_s && !(pass && !pass->first)) {
       // only the rows of the region are touched
@@ -739,8 +751,30 @@ rt_status rt_camera_render_region_device(rt_camera* c, const rt_region* region, 
   RT_GUARD_END
 }
 
+// ev0, enqueue_render, the optional step `post` (more work on the camera's stream, its launches counted), `end`, then the
+// raw counters to `raw` (kStatCount values of host memory).  No synchronisation.
+static rt_status timed_render(rt_camera* c, RenderParams& P, cudaEvent_t end, unsigned long long* raw, int* launches,
+                              const ProgPass* pass = nullptr, const std::function<rt_status(int*)>& post = {}) {
+  CU(cudaEventRecord(c->ev0, c->stream));
+  rt_status st = enqueue_render(c, P, nullptr, launches, pass);
+  if (st != RT_OK) return st;
+  if (post) {
+    int l = 0;
+    if ((st = post(&l)) != RT_OK) return st;
+    *launches += l;
+  }
+  CU(cudaEventRecord(end, c->stream));
+  CU(cudaMemcpyAsync(raw, c->d_stats, sizeof(unsigned long long) * kStatCount, cudaMemcpyDeviceToHost, c->stream));
+  return RT_OK;
+}
+
+static rt_status denoise_band(rt_camera* c, const RenderParams& P, int b0, int b1, const DenoiseParams& opts, const float* color,
+                              const float* moments, float* out, uint8_t* rgb8, bool poison, int* launches);
+
+// Render the region and copy it to the caller's [H][W] arrays.  With `dn`, the colour and moments stay on the device and
+// are filtered in place before ev1 (one band covering the region); RGB8 is written from the filtered image.
 static rt_status render_host(rt_camera* c, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
-                             float* moments, rt_stats* stats) {
+                             float* moments, rt_stats* stats, const DenoiseParams* dn = nullptr) {
   RT_GUARD_BEGIN
   if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
   const int W = c->hs->image_width, H = c->hs->image_height;
@@ -751,27 +785,25 @@ static rt_status render_host(rt_camera* c, const rt_region* region, uint8_t* rgb
   rt_status st = clip_region(c, region, P);
   if (st != RT_OK) return st;
   if (rgb8 && !c->d_rgb8) CU(dev_alloc(&c->d_rgb8, npx * 3));
-  if (linear && !c->d_linear) CU(dev_alloc(&c->d_linear, npx * 3 * sizeof(float)));
-  if (moments && !c->d_moments) CU(dev_alloc(&c->d_moments, npx * 8 * sizeof(float)));
-  P.rgb8 = rgb8 ? c->d_rgb8 : nullptr;
-  P.linear = linear ? c->d_linear : nullptr;
-  P.moments = moments ? c->d_moments : nullptr;
+  if ((linear || dn) && !c->d_linear) CU(dev_alloc(&c->d_linear, npx * 3 * sizeof(float)));
+  if ((moments || dn) && !c->d_moments) CU(dev_alloc(&c->d_moments, npx * 8 * sizeof(float)));
+  P.rgb8 = rgb8 && !dn ? c->d_rgb8 : nullptr;
+  P.linear = linear || dn ? c->d_linear : nullptr;
+  P.moments = moments || dn ? c->d_moments : nullptr;
+  std::function<rt_status(int*)> denoise;
+  if (dn)
+    denoise = [&](int* l) { return denoise_band(c, P, P.y0, P.y1, *dn, P.linear, P.moments, P.linear, rgb8 ? c->d_rgb8 : nullptr, false, l); };
   int launches = 0;
-  CU(cudaEventRecord(c->ev0, c->stream));
-  st = enqueue_render(c, P, nullptr, &launches);
-  if (st != RT_OK) return st;
-  CU(cudaEventRecord(c->ev1, c->stream));
   unsigned long long raw[kStatCount];
-  CU(cudaMemcpyAsync(raw, c->d_stats, sizeof(raw), cudaMemcpyDeviceToHost, c->stream));
+  if ((st = timed_render(c, P, c->ev1, raw, &launches, nullptr, denoise)) != RT_OK) return st;
   const bool whole_tiles = c->opts.part_count <= 1;
   const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
   if (rw > 0 && rh > 0) {
     if (whole_tiles) {
       // only the region's pixels are written (camera.ts:400-401): pitched copies of the sub-rectangle
-      const size_t off = (size_t)P.y0 * W + P.x0;
-      if (rgb8) CU(cudaMemcpy2DAsync(rgb8 + off * 3, (size_t)W * 3, c->d_rgb8 + off * 3, (size_t)W * 3, (size_t)rw * 3, rh, cudaMemcpyDeviceToHost, c->stream));
-      if (linear) CU(cudaMemcpy2DAsync(linear + off * 3, (size_t)W * 12, c->d_linear + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
-      if (moments) CU(cudaMemcpy2DAsync(moments + off * 8, (size_t)W * 32, c->d_moments + off * 8, (size_t)W * 32, (size_t)rw * 32, rh, cudaMemcpyDeviceToHost, c->stream));
+      if (rgb8) CU(copy_region(rgb8, c->d_rgb8, 3, P, W, cudaMemcpyDeviceToHost, c->stream));
+      if (linear) CU(copy_region(linear, c->d_linear, 12, P, W, cudaMemcpyDeviceToHost, c->stream));
+      if (moments) CU(copy_region(moments, c->d_moments, 32, P, W, cudaMemcpyDeviceToHost, c->stream));
       CU(cudaStreamSynchronize(c->stream));
     } else {
       // partitioned render: stage the rows, then copy only the tiles this part owns
@@ -802,8 +834,7 @@ static rt_status render_host(rt_camera* c, const rt_region* region, uint8_t* rgb
     CU(cudaStreamSynchronize(c->stream));
   }
   if (stats) {
-    std::memset(stats, 0, sizeof(*stats));
-    unpack_stats(raw, stats);
+    *stats = unpack_stats(raw);
     float ms = 0;
     CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
     stats->device_ms = ms;
@@ -844,10 +875,7 @@ rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, ui
   const int S = c->hs->cam.samples;
   const bool stream = c->hs->cam.adaptive || c->hs->cam.mode != 0;
   const int batch = c->hs->cam.adaptive ? std::max(1, c->hs->cam.a_batch) : 1;
-  rt_stats total;
-  std::memset(&total, 0, sizeof(total));
-  total.samples_min = total.bounces_min = 0x7fffffff;
-  const int rw = P0.x1 - P0.x0, rh = P0.y1 - P0.y0;
+  rt_stats total = unpack_stats(kStatsInit);
   int prev = 0, passes_run = 0;
   for (int k = 1; k <= n_passes; ++k) {
     // prefix of the samples after pass k; the pixel stream stops on batch boundaries only (the convergence check of
@@ -861,35 +889,24 @@ rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, ui
     P.linear = linear ? c->d_linear : nullptr;
     const ProgPass pass{prev, (int)cap, passes_run == 0};
     int launches = 0;
-    CU(cudaEventRecord(c->ev0, c->stream));
-    st = enqueue_render(c, P, nullptr, &launches, (S > 0 && n_passes > 1) ? &pass : nullptr);
-    if (st != RT_OK) return st;
-    CU(cudaEventRecord(c->ev1, c->stream));
     unsigned long long raw[kStatCount];
-    CU(cudaMemcpyAsync(raw, c->d_stats, sizeof(raw), cudaMemcpyDeviceToHost, c->stream));
-    if (rw > 0 && rh > 0) {
-      const size_t off = (size_t)P0.y0 * W + P0.x0;
-      if (rgb8) CU(cudaMemcpy2DAsync(rgb8 + off * 3, (size_t)W * 3, c->d_rgb8 + off * 3, (size_t)W * 3, (size_t)rw * 3, rh, cudaMemcpyDeviceToHost, c->stream));
-      if (linear) CU(cudaMemcpy2DAsync(linear + off * 3, (size_t)W * 12, c->d_linear + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
-    }
+    st = timed_render(c, P, c->ev1, raw, &launches, (S > 0 && n_passes > 1) ? &pass : nullptr);
+    if (st != RT_OK) return st;
+    if (rgb8) CU(copy_region(rgb8, c->d_rgb8, 3, P0, W, cudaMemcpyDeviceToHost, c->stream));
+    if (linear) CU(copy_region(linear, c->d_linear, 12, P0, W, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
-    rt_stats ps;
-    std::memset(&ps, 0, sizeof(ps));
-    unpack_stats(raw, &ps);
+    rt_stats ps = unpack_stats(raw);
+    ps.kernel_launches = launches;
     float ms = 0;
     CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-    // RenderStats.merge over the passes: work adds up; a pixel is counted by the pass that completes it
-    total.samples_total += ps.samples_total; total.bounces_total += ps.bounces_total; total.rays += ps.rays;
-    total.node_visits += ps.node_visits; total.prim_tests += ps.prim_tests;
-    total.device_ms += ms; total.kernel_launches += launches;
-    total.bounces_min = std::min(total.bounces_min, ps.bounces_min); total.bounces_max = std::max(total.bounces_max, ps.bounces_max);
-    if (stream) {
-      total.pixels += ps.pixels;
-      total.samples_min = std::min(total.samples_min, ps.samples_min); total.samples_max = std::max(total.samples_max, ps.samples_max);
-    } else { // fixed spp: every pass touches every pixel; all of them have `cap` samples now
+    // over the passes: device_ms adds up; a pixel is counted by the pass that completes it
+    const int32_t samples_min = total.samples_min;
+    merge_stats(&total, ps);
+    total.device_ms += ms;
+    if (!stream) { // fixed spp: every pass touches every pixel; all of them have `cap` samples now
       total.pixels = ps.pixels;
-      total.samples_min = total.samples_max = ps.pixels ? (int32_t)cap : total.samples_min;
-      if (!ps.pixels) total.samples_max = 0;
+      total.samples_min = ps.pixels ? (int32_t)cap : samples_min;
+      total.samples_max = ps.pixels ? (int32_t)cap : 0;
     }
     prev = (int)cap;
     ++passes_run;
@@ -902,6 +919,7 @@ rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, ui
 
 rt_status rt_camera_trace_primary(rt_camera* c, const rt_region* region, int32_t* obj_id, float* t, float* normal,
                                   uint8_t* front_face) {
+  RT_GUARD_BEGIN
   if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
   DeviceGuard g(c->device);
   const int W = c->hs->image_width, H = c->hs->image_height;
@@ -914,16 +932,13 @@ rt_status rt_camera_trace_primary(rt_camera* c, const rt_region* region, int32_t
   if (!c->d_normal) CU(dev_alloc(&c->d_normal, npx * 12));
   if (!c->d_front) CU(dev_alloc(&c->d_front, npx));
   CU(launch_trace_primary(c->ds, P, c->d_ids, c->d_t, c->d_normal, c->d_front, c->stream));
-  const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
-  if (rw > 0 && rh > 0) {
-    const size_t off = (size_t)P.y0 * W + P.x0;
-    if (obj_id) CU(cudaMemcpy2DAsync(obj_id + off, (size_t)W * 4, c->d_ids + off, (size_t)W * 4, (size_t)rw * 4, rh, cudaMemcpyDeviceToHost, c->stream));
-    if (t) CU(cudaMemcpy2DAsync(t + off, (size_t)W * 4, c->d_t + off, (size_t)W * 4, (size_t)rw * 4, rh, cudaMemcpyDeviceToHost, c->stream));
-    if (normal) CU(cudaMemcpy2DAsync(normal + off * 3, (size_t)W * 12, c->d_normal + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
-    if (front_face) CU(cudaMemcpy2DAsync(front_face + off, (size_t)W, c->d_front + off, (size_t)W, (size_t)rw, rh, cudaMemcpyDeviceToHost, c->stream));
-  }
+  if (obj_id) CU(copy_region(obj_id, c->d_ids, 4, P, W, cudaMemcpyDeviceToHost, c->stream));
+  if (t) CU(copy_region(t, c->d_t, 4, P, W, cudaMemcpyDeviceToHost, c->stream));
+  if (normal) CU(copy_region(normal, c->d_normal, 12, P, W, cudaMemcpyDeviceToHost, c->stream));
+  if (front_face) CU(copy_region(front_face, c->d_front, 1, P, W, cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   return RT_OK;
+  RT_GUARD_END
 }
 
 // ---- denoiser (rt_denoise.cuh) ----
@@ -1008,13 +1023,9 @@ rt_status rt_camera_render_features(rt_camera* c, const rt_region* region, int32
   if (st != RT_OK) return st;
   if ((st = features_prepare(c, npx)) != RT_OK) return st;
   CU(launch_render_features(c->ds, P, n_samples, c->d_falb, c->d_fnrm, c->d_fdepth, c->stream));
-  const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
-  if (rw > 0 && rh > 0) {
-    const size_t off = (size_t)P.y0 * W + P.x0;
-    if (albedo) CU(cudaMemcpy2DAsync(albedo + off * 3, (size_t)W * 12, c->d_falb + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
-    if (normal) CU(cudaMemcpy2DAsync(normal + off * 3, (size_t)W * 12, c->d_fnrm + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
-    if (depth) CU(cudaMemcpy2DAsync(depth + off, (size_t)W * 4, c->d_fdepth + off, (size_t)W * 4, (size_t)rw * 4, rh, cudaMemcpyDeviceToHost, c->stream));
-  }
+  if (albedo) CU(copy_region(albedo, c->d_falb, 12, P, W, cudaMemcpyDeviceToHost, c->stream));
+  if (normal) CU(copy_region(normal, c->d_fnrm, 12, P, W, cudaMemcpyDeviceToHost, c->stream));
+  if (depth) CU(copy_region(depth, c->d_fdepth, 4, P, W, cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   return RT_OK;
   RT_GUARD_END
@@ -1073,51 +1084,12 @@ rt_status rt_camera_render_denoised(rt_camera* c, const rt_region* region, uint8
   DenoiseParams D{};
   rt_status st = dn_options(opts, D);
   if (st != RT_OK) return st;
-  const int W = c->hs->image_width, H = c->hs->image_height;
-  const size_t npx = (size_t)W * H;
-  if (rgb8 && rgb8_len < npx * 3) return fail(RT_ERR_BUFFER_TOO_SMALL, "rgb8 buffer smaller than width*height*3");
+  if (rgb8 && rgb8_len < (size_t)c->hs->image_width * c->hs->image_height * 3)
+    return fail(RT_ERR_BUFFER_TOO_SMALL, "rgb8 buffer smaller than width*height*3");
   // the filter reads the neighbours of a pixel, which other parts render; modes other than default are not radiance
   if (c->opts.part_count > 1) return fail(RT_ERR_UNSUPPORTED, "denoised renders are not partitioned");
   if (c->hs->cam.mode != RT_MODE_DEFAULT) return fail(RT_ERR_UNSUPPORTED, "denoised renders need the default render mode");
-  DeviceGuard g(c->device);
-  RenderParams P;
-  st = clip_region(c, region, P);
-  if (st != RT_OK) return st;
-  if (rgb8 && !c->d_rgb8) CU(dev_alloc(&c->d_rgb8, npx * 3));
-  if (!c->d_linear) CU(dev_alloc(&c->d_linear, npx * 3 * sizeof(float)));
-  if (!c->d_moments) CU(dev_alloc(&c->d_moments, npx * 8 * sizeof(float)));
-  P.rgb8 = nullptr; // RGB8 is written from the filtered image
-  P.linear = c->d_linear;
-  P.moments = c->d_moments;
-  int launches = 0;
-  CU(cudaEventRecord(c->ev0, c->stream));
-  st = enqueue_render(c, P, nullptr, &launches);
-  if (st != RT_OK) return st;
-  const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
-  if (rw > 0 && rh > 0) { // one band: the whole region, filtered in place
-    int dn_launches = 0;
-    st = denoise_band(c, P, P.y0, P.y1, D, c->d_linear, c->d_moments, c->d_linear, rgb8 ? c->d_rgb8 : nullptr, false, &dn_launches);
-    if (st != RT_OK) return st;
-    launches += dn_launches;
-  }
-  CU(cudaEventRecord(c->ev1, c->stream));
-  unsigned long long raw[kStatCount];
-  CU(cudaMemcpyAsync(raw, c->d_stats, sizeof(raw), cudaMemcpyDeviceToHost, c->stream));
-  if (rw > 0 && rh > 0) {
-    const size_t off = (size_t)P.y0 * W + P.x0;
-    if (rgb8) CU(cudaMemcpy2DAsync(rgb8 + off * 3, (size_t)W * 3, c->d_rgb8 + off * 3, (size_t)W * 3, (size_t)rw * 3, rh, cudaMemcpyDeviceToHost, c->stream));
-    if (linear) CU(cudaMemcpy2DAsync(linear + off * 3, (size_t)W * 12, c->d_linear + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c->stream));
-  }
-  CU(cudaStreamSynchronize(c->stream));
-  if (stats) {
-    std::memset(stats, 0, sizeof(*stats));
-    unpack_stats(raw, stats);
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-    stats->device_ms = ms;
-    stats->kernel_launches = launches;
-  }
-  return RT_OK;
+  return render_host(c, region, rgb8, rgb8_len, linear, nullptr, stats, &D);
   RT_GUARD_END
 }
 
@@ -1182,31 +1154,36 @@ struct rt_multi {
   unsigned long long* h_stats = nullptr; // pinned [n][kStatCount]
 };
 
-// RenderStats.merge of one rt_multi call: work adds up, extremes combine; device_ms = the slowest device (host-merge path)
-static void merge_stats(const std::vector<rt_stats>& ps, rt_stats* out) {
-  std::memset(out, 0, sizeof(*out));
-  out->samples_min = out->bounces_min = 0x7fffffff;
-  for (const rt_stats& s : ps) {
-    out->pixels += s.pixels; out->samples_total += s.samples_total; out->bounces_total += s.bounces_total; out->rays += s.rays;
-    out->node_visits += s.node_visits; out->prim_tests += s.prim_tests;
-    out->samples_min = std::min(out->samples_min, s.samples_min); out->samples_max = std::max(out->samples_max, s.samples_max);
-    out->bounces_min = std::min(out->bounces_min, s.bounces_min); out->bounces_max = std::max(out->bounces_max, s.bounces_max);
-    out->device_ms = std::max(out->device_ms, s.device_ms); out->kernel_launches += s.kernel_launches;
-  }
+// One host thread per device runs job(k); returns the first failing device's status, with its message.
+static rt_status on_every_device(int n, const std::function<rt_status(int)>& job) {
+  std::vector<rt_status> st((size_t)n, RT_OK);
+  std::vector<std::string> msg((size_t)n);
+  std::vector<std::thread> th;
+  for (int k = 0; k < n; ++k)
+    th.emplace_back([&, k]() {
+      st[k] = job(k);
+      if (st[k] != RT_OK) msg[k] = g_err;
+    });
+  for (auto& t : th) t.join();
+  for (int k = 0; k < n; ++k)
+    if (st[k] != RT_OK) return fail(st[k], msg[k]);
+  return RT_OK;
 }
-// the same over the raw counters the peer-write path copies to m->h_stats (device_ms and kernel_launches are the caller's)
-static void merge_raw_stats(const rt_multi* m, rt_stats* out) {
-  unsigned long long raw[kStatCount];
-  std::memcpy(raw, kStatsInit, sizeof(raw));
-  for (size_t k = 0; k < m->cams.size(); ++k) {
-    const unsigned long long* r = m->h_stats + k * kStatCount;
-    raw[kStatPixels] += r[kStatPixels]; raw[kStatSamples] += r[kStatSamples]; raw[kStatBounces] += r[kStatBounces]; raw[kStatRays] += r[kStatRays];
-    raw[kStatNodeVisits] += r[kStatNodeVisits]; raw[kStatPrimTests] += r[kStatPrimTests];
-    raw[kStatSamplesMin] = std::min(raw[kStatSamplesMin], r[kStatSamplesMin]); raw[kStatSamplesMax] = std::max(raw[kStatSamplesMax], r[kStatSamplesMax]);
-    raw[kStatBouncesMin] = std::min(raw[kStatBouncesMin], r[kStatBouncesMin]); raw[kStatBouncesMax] = std::max(raw[kStatBouncesMax], r[kStatBouncesMax]);
+
+// The host-merge path's stats: device_ms is the slowest device's (they run concurrently).
+static rt_stats merge_host_stats(const std::vector<rt_stats>& ps) {
+  rt_stats out = unpack_stats(kStatsInit);
+  for (const rt_stats& s : ps) {
+    merge_stats(&out, s);
+    out.device_ms = std::max(out.device_ms, s.device_ms);
   }
-  std::memset(out, 0, sizeof(*out));
-  unpack_stats(raw, out);
+  return out;
+}
+// The merged counters the peer-write path copied to m->h_stats (device_ms and kernel_launches are the caller's).
+static rt_stats merge_raw_stats(const rt_multi* m) {
+  rt_stats out = unpack_stats(kStatsInit);
+  for (size_t k = 0; k < m->cams.size(); ++k) merge_stats(&out, unpack_stats(m->h_stats + k * kStatCount));
+  return out;
 }
 
 static void free_multi(rt_multi* m) {
@@ -1319,19 +1296,10 @@ rt_status rt_multi_render_region(rt_multi* m, const rt_region* region, uint8_t* 
   if (stats) std::memset(stats, 0, sizeof(*stats));
   if (!m->p2p && n > 1) {
     // host merge: one thread per device, each copies the blocks it owns into the caller's buffer
-    std::vector<rt_status> st((size_t)n, RT_OK);
-    std::vector<std::string> msg((size_t)n);
     std::vector<rt_stats> ps((size_t)n);
-    std::vector<std::thread> th;
-    for (int k = 0; k < n; ++k)
-      th.emplace_back([&, k]() {
-        st[k] = render_host(m->cams[k], region, rgb8, rgb8_len, linear, nullptr, &ps[k]);
-        if (st[k] != RT_OK) msg[k] = g_err;
-      });
-    for (auto& t : th) t.join();
-    for (int k = 0; k < n; ++k)
-      if (st[k] != RT_OK) return fail(st[k], msg[k]);
-    if (stats) merge_stats(ps, stats);
+    rt_status st = on_every_device(n, [&](int k) { return render_host(m->cams[k], region, rgb8, rgb8_len, linear, nullptr, &ps[k]); });
+    if (st != RT_OK) return st;
+    if (stats) *stats = merge_host_stats(ps);
     return RT_OK;
   }
   // ---- peer-write path ----
@@ -1351,11 +1319,7 @@ rt_status rt_multi_render_region(rt_multi* m, const rt_region* region, uint8_t* 
     P.rgb8 = rgb8 ? m->d_rgb8 : nullptr;       // device 0's framebuffer, peer-mapped on device k
     P.linear = linear ? m->d_linear : nullptr;
     int launches = 0;
-    CU(cudaEventRecord(c->ev0, c->stream));
-    st = enqueue_render(c, P, nullptr, &launches);
-    if (st != RT_OK) return st;
-    CU(cudaEventRecord(c->ev1, c->stream));
-    CU(cudaMemcpyAsync(m->h_stats + (size_t)k * kStatCount, c->d_stats, sizeof(unsigned long long) * kStatCount, cudaMemcpyDeviceToHost, c->stream));
+    if ((st = timed_render(c, P, c->ev1, m->h_stats + (size_t)k * kStatCount, &launches)) != RT_OK) return st;
     CU(cudaEventRecord(m->done[k], c->stream));
     launches_total += launches;
     if (k == 0) P0 = P;
@@ -1363,12 +1327,8 @@ rt_status rt_multi_render_region(rt_multi* m, const rt_region* region, uint8_t* 
   {
     DeviceGuard g0(m->devices[0]);
     for (int k = 1; k < n; ++k) CU(cudaStreamWaitEvent(c0->stream, m->done[k], 0)); // peers' pixels have landed in device 0's memory
-    const int rw = P0.x1 - P0.x0, rh = P0.y1 - P0.y0;
-    if (rw > 0 && rh > 0) {
-      const size_t off = (size_t)P0.y0 * W + P0.x0;
-      if (rgb8) CU(cudaMemcpy2DAsync(rgb8 + off * 3, (size_t)W * 3, m->d_rgb8 + off * 3, (size_t)W * 3, (size_t)rw * 3, rh, cudaMemcpyDeviceToHost, c0->stream));
-      if (linear) CU(cudaMemcpy2DAsync(linear + off * 3, (size_t)W * 12, m->d_linear + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c0->stream));
-    }
+    if (rgb8) CU(copy_region(rgb8, m->d_rgb8, 3, P0, W, cudaMemcpyDeviceToHost, c0->stream));
+    if (linear) CU(copy_region(linear, m->d_linear, 12, P0, W, cudaMemcpyDeviceToHost, c0->stream));
     CU(cudaStreamSynchronize(c0->stream));
   }
   if (stats) {
@@ -1379,7 +1339,7 @@ rt_status rt_multi_render_region(rt_multi* m, const rt_region* region, uint8_t* 
       CU(cudaEventElapsedTime(&ms, m->cams[k]->ev0, m->cams[k]->ev1));
       ms_max = std::max(ms_max, (double)ms);
     }
-    merge_raw_stats(m, stats);
+    *stats = merge_raw_stats(m);
     stats->device_ms = ms_max; // the slowest device (they run concurrently)
     stats->kernel_launches = launches_total;
   }
@@ -1431,24 +1391,14 @@ rt_status rt_multi_render_denoised(rt_multi* m, const rt_region* region, uint8_t
   if (!m->p2p && n > 1) {
     // host merge: one thread per device renders its blocks' colour and moments into host arrays, device 0 filters
     std::vector<float> hc(npx * 3), hm(npx * 8);
-    std::vector<rt_status> rs((size_t)n, RT_OK);
-    std::vector<std::string> msg((size_t)n);
     std::vector<rt_stats> ps((size_t)n);
-    std::vector<std::thread> th;
-    for (int k = 0; k < n; ++k)
-      th.emplace_back([&, k]() {
-        rs[k] = render_host(m->cams[k], region, nullptr, 0, hc.data(), hm.data(), &ps[k]);
-        if (rs[k] != RT_OK) msg[k] = g_err;
-      });
-    for (auto& t : th) t.join();
-    for (int k = 0; k < n; ++k)
-      if (rs[k] != RT_OK) return fail(rs[k], msg[k]);
+    st = on_every_device(n, [&](int k) { return render_host(m->cams[k], region, nullptr, 0, hc.data(), hm.data(), &ps[k]); });
+    if (st != RT_OK) return st;
     DeviceGuard g0(m->devices[0]);
     CU(cudaEventRecord(c0->ev0, c0->stream));
     if (rw > 0 && rh > 0) {
-      const size_t off = (size_t)P0.y0 * W + P0.x0;
-      CU(cudaMemcpy2DAsync(m->d_color + off * 3, (size_t)W * 12, hc.data() + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyHostToDevice, c0->stream));
-      CU(cudaMemcpy2DAsync(m->d_moments + off * 8, (size_t)W * 32, hm.data() + off * 8, (size_t)W * 32, (size_t)rw * 32, rh, cudaMemcpyHostToDevice, c0->stream));
+      CU(copy_region(m->d_color, hc.data(), 12, P0, W, cudaMemcpyHostToDevice, c0->stream));
+      CU(copy_region(m->d_moments, hm.data(), 32, P0, W, cudaMemcpyHostToDevice, c0->stream));
       for (int b = 0; b < n_bands; ++b) {
         int b0, b1, l = 0;
         band(b, b0, b1);
@@ -1459,7 +1409,7 @@ rt_status rt_multi_render_denoised(rt_multi* m, const rt_region* region, uint8_t
     }
     CU(cudaEventRecord(c0->ev1, c0->stream));
     if (stats) {
-      merge_stats(ps, stats);
+      *stats = merge_host_stats(ps);
       float ms = 0;
       CU(cudaEventSynchronize(c0->ev1));
       CU(cudaEventElapsedTime(&ms, c0->ev0, c0->ev1));
@@ -1479,11 +1429,7 @@ rt_status rt_multi_render_denoised(rt_multi* m, const rt_region* region, uint8_t
       P.linear = m->d_color; // device 0's buffers, peer-mapped on device k
       P.moments = m->d_moments;
       int launches = 0;
-      CU(cudaEventRecord(c->ev0, c->stream));
-      st = enqueue_render(c, P, nullptr, &launches);
-      if (st != RT_OK) return st;
-      CU(cudaMemcpyAsync(m->h_stats + (size_t)k * kStatCount, c->d_stats, sizeof(unsigned long long) * kStatCount, cudaMemcpyDeviceToHost, c->stream));
-      CU(cudaEventRecord(m->rendered[k], c->stream));
+      if ((st = timed_render(c, P, m->rendered[k], m->h_stats + (size_t)k * kStatCount, &launches)) != RT_OK) return st;
       launches_total += launches;
     }
     if (rw > 0 && rh > 0) {
@@ -1513,17 +1459,14 @@ rt_status rt_multi_render_denoised(rt_multi* m, const rt_region* region, uint8_t
       CU(cudaEventSynchronize(c0->ev1));
       float ms = 0;
       CU(cudaEventElapsedTime(&ms, c0->ev0, c0->ev1));
-      merge_raw_stats(m, stats);
+      *stats = merge_raw_stats(m);
       stats->device_ms = ms; // device 0, from its render to the last band's last kernel
       stats->kernel_launches = launches_total;
     }
   }
   DeviceGuard g0(m->devices[0]);
-  if (rw > 0 && rh > 0) {
-    const size_t off = (size_t)P0.y0 * W + P0.x0;
-    if (rgb8) CU(cudaMemcpy2DAsync(rgb8 + off * 3, (size_t)W * 3, m->d_rgb8 + off * 3, (size_t)W * 3, (size_t)rw * 3, rh, cudaMemcpyDeviceToHost, c0->stream));
-    if (linear) CU(cudaMemcpy2DAsync(linear + off * 3, (size_t)W * 12, m->d_linear + off * 3, (size_t)W * 12, (size_t)rw * 12, rh, cudaMemcpyDeviceToHost, c0->stream));
-  }
+  if (rgb8) CU(copy_region(rgb8, m->d_rgb8, 3, P0, W, cudaMemcpyDeviceToHost, c0->stream));
+  if (linear) CU(copy_region(linear, m->d_linear, 12, P0, W, cudaMemcpyDeviceToHost, c0->stream));
   CU(cudaStreamSynchronize(c0->stream));
   return RT_OK;
   RT_GUARD_END

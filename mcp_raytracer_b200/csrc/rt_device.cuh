@@ -21,10 +21,6 @@ namespace rt {
 
 #define RT_DEV __device__ __forceinline__
 
-#ifndef RT_EXACT_RCP
-#define RT_FAST_RCP 1 // per-ray reciprocals via MUFU (measured +7 % on Cornell); -DRT_EXACT_RCP restores IEEE division
-#endif
-
 static constexpr float kEps32 = 5.9604645e-08f; // 2^-24
 static constexpr float kRayTMin = 0.001f;       // camera.ts:249
 
@@ -62,10 +58,6 @@ RT_DEV float rsqrt_approx(float x) {
 RT_DEV V3 normalize3(V3 a) { // gl-matrix normalize: zero stays zero
   float l = dot3(a, a);
   float s = l > 0.f ? rsqrt_approx(l) : 0.f;
-#ifdef RT_EXACT_NORMALIZE
-  // one Newton step brings rsqrt.approx (2 ulp) to ~0.5 ulp
-  s = s * fmaf(-0.5f * l * s, s, 1.5f);
-#endif
   // rsqrt.approx is good to 2 ulp: unit vectors are unit to 2.4e-7, the level of the FP32 roundings around every use
   // (directions are never required to be unit by the tests that consume them: a = |d|^2 is carried, camera.ts:176-210)
   return a * s;
@@ -181,22 +173,14 @@ struct RayPre {
 RT_DEV RayPre precompute(const Ray& r, bool need_box) {
   RayPre p;
   p.a = dot3(r.d, r.d);
-#ifdef RT_FAST_RCP
-  // MUFU reciprocals (1-2 ulp): the primitive tests' error bounds have that much slack built in
-  // (8 eps on t), and box tests pad tmax by 4 ulp
+  // MUFU reciprocals (1-2 ulp; measured +7 % on Cornell against IEEE division): the primitive tests' error bounds have
+  // that much slack built in (8 eps on t), and box tests pad tmax by 4 ulp
   p.inva = rcp_approx(p.a);
-#else
-  p.inva = 1.0f / p.a;
-#endif
   p.l1d = l1norm(r.d);
   p.omax175 = 1.75f * maxabs(r.o);
   p.dmax = maxabs(r.d);
   if (need_box) {
-#ifdef RT_FAST_RCP
     p.idir = V3{rcp_approx(r.d.x), rcp_approx(r.d.y), rcp_approx(r.d.z)};
-#else
-    p.idir = V3{1.0f / r.d.x, 1.0f / r.d.y, 1.0f / r.d.z};
-#endif
     p.oid = r.o * p.idir;
   } else {
     p.idir = V3{0, 0, 0};
@@ -543,7 +527,6 @@ template <class Scene>
 RT_DEV void trace_list(const Scene& S, const SmemList& L, const Ray& r, const RayPre& pre, float& tbest, int& sbest) {
   int s = 0;
   float t;
-#ifndef RT_AAQUAD_GENERIC_LOOP
   // early exit on a sure miss: with many small spheres the whole warp nearly always takes it (49-sphere box:
   // 109.5 -> 93.9 ms; Cornell with its two big spheres: +1 %)
   // A bound of E that holds for every sphere of the list, from per-ray and per-scene constants only:
@@ -558,21 +541,6 @@ RT_DEV void trace_list(const Scene& S, const SmemList& L, const Ray& r, const Ra
   aaquad_run<0>(S.exact, L, s, s + S.list_n[1], r, pre, tbest, sbest);
   aaquad_run<1>(S.exact, L, s, s + S.list_n[2], r, pre, tbest, sbest);
   aaquad_run<2>(S.exact, L, s, s + S.list_n[3], r, pre, tbest, sbest);
-#else
-#ifdef RT_UNROLL2
-#define RT_LIST_UNROLL _Pragma("unroll 2")
-#else
-#define RT_LIST_UNROLL
-#endif
-  RT_LIST_UNROLL
-  for (const int e = s + S.list_n[0]; s < e; ++s) take_hit(S.exact, sphere_test(L.p0(s), r, pre, tbest, t), t, s, r, tbest, sbest);
-  RT_LIST_UNROLL
-  for (const int e = s + S.list_n[1]; s < e; ++s) take_hit(S.exact, aaquad_test<0>(L.p1(s), L.p2(s), r, pre, tbest, t), t, s, r, tbest, sbest);
-  RT_LIST_UNROLL
-  for (const int e = s + S.list_n[2]; s < e; ++s) take_hit(S.exact, aaquad_test<1>(L.p1(s), L.p2(s), r, pre, tbest, t), t, s, r, tbest, sbest);
-  RT_LIST_UNROLL
-  for (const int e = s + S.list_n[3]; s < e; ++s) take_hit(S.exact, aaquad_test<2>(L.p1(s), L.p2(s), r, pre, tbest, t), t, s, r, tbest, sbest);
-#endif
   for (const int e = s + S.list_n[4]; s < e; ++s)
     take_hit(S.exact, planar_test(L.p0(s), L.p1(s), L.p2(s), L.p3(s), true, r, pre, tbest, t), t, s, r, tbest, sbest);
   for (const int e = s + S.list_n[5]; s < e; ++s)
@@ -614,11 +582,8 @@ struct BoxPre {
 };
 RT_DEV BoxPre box_precompute(const Ray& r) {
   BoxPre b;
-#ifdef RT_FAST_RCP // like precompute(): MUFU reciprocals, the slab tests pad the exit distance by 4 ulp
+  // like precompute(): MUFU reciprocals, the slab tests pad the exit distance by 4 ulp
   b.idir = V3{rcp_approx(r.d.x), rcp_approx(r.d.y), rcp_approx(r.d.z)};
-#else
-  b.idir = V3{1.0f / r.d.x, 1.0f / r.d.y, 1.0f / r.d.z};
-#endif
   b.oid = r.o * b.idir;
   return b;
 }
@@ -862,17 +827,12 @@ RT_DEV Onb make_onb(V3 n) { // onbasis.ts:18-25
 }
 RT_DEV V3 onb_local(const Onb& b, V3 a) { return fma3(a.x, b.u, fma3(a.y, b.v, b.w * a.z)); }
 RT_DEV V3 cosine_direction(float r1, float r2) { // vec3.ts:325-337
-  float sn, cs;
-#ifndef RT_EXACT_SINCOS
   // phi = 2 pi r1 folded to [-pi, pi) so the MUFU sin / cos stay in their accurate range (absolute error ~5e-7, the
   // level of the FP32 roundings around it); sincospif costs ~25 instructions more per diffuse bounce.
   // Measured (1024^2 @256 / 2048^2 @64 / 1920x1080 @64): Cornell 30.23 -> 29.77 ms, layered 88.96 -> 88.40, weekend 37.86 -> 37.09.
   const float rr = r1 - (r1 >= 0.5f ? 1.f : 0.f);
-  sn = __sinf(6.28318530718f * rr);
-  cs = __cosf(6.28318530718f * rr);
-#else
-  sincospif(2.f * r1, &sn, &cs);
-#endif
+  const float sn = __sinf(6.28318530718f * rr);
+  const float cs = __cosf(6.28318530718f * rr);
   const float s = sqrtf(r2);
   return mk3(cs * s, sn * s, sqrtf(1.f - r2));
 }
@@ -884,7 +844,6 @@ RT_DEV V3 random_in_unit_sphere(G& g) {
     if (dot3(p, p) < 1.f) return p;
   }
 }
-#ifndef RT_NO_TRIAL_REFILL
 // The Philox stream: a trial needs three uniforms and a block yields five, so the second trial of the rejection loop (48 % of
 // the fuzzy-metal hits, 23 % need a third ...) ran into Rng::next()'s out-of-line refill in the middle of a trial — one lane at a
 // time (ncu, 100 k metal spheres: that call at 2 of 32 lanes).  Here the block is generated at the TOP of a trial that cannot be
@@ -918,7 +877,6 @@ RT_DEV V3 random_in_unit_sphere(Rng& g) {
     if (dot3(p, p) < 1.f) return p;
   }
 }
-#endif
 RT_DEV float cosine_pdf_value(V3 w_unit, V3 dir) { // pdf.ts:43-46
   float c = dot3(normalize3(dir), w_unit);
   return c <= 0.f ? 0.f : c * 0.31830988618f;

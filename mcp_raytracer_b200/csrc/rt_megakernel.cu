@@ -144,7 +144,6 @@ RT_DEV bool path_pre(const DevCamera& cam, PathState& ps, Rng& g) {
 
 // rayColor, part 2 (camera.ts:249-319) given the closest hit (slot < 0: miss).  True = the path ended
 // (its radiance is complete); otherwise ps.ray / ps.tp / ps.bounces describe the next call.
-#ifndef RT_SINGLE_EXIT
 template <int KIND, bool LV = true> // LV: light records by 128-bit loads (light_ld4, rt_device.cuh)
 RT_DEV bool path_post(const DevScene& S, const ListSmem* sm, const MixW& mw, PathState& ps, Rng& g, float t, int slot) {
   const DevCamera& cam = S.cam;
@@ -187,52 +186,6 @@ RT_DEV bool path_post(const DevScene& S, const ListSmem* sm, const MixW& mw, Pat
   ps.ray = Ray{sf.p, dir};
   return false;
 }
-#else
-// Single-exit form: every branch rejoins before the next one starts, so the diffuse and the specular update are
-// laid out once each and the warp reconverges between the stages (miss | emission + dispatch | scatter | update).
-template <int KIND, bool LV = true> // LV: light records by 128-bit loads (light_ld4, rt_device.cuh)
-RT_DEV bool path_post(const DevScene& S, const ListSmem* sm, const MixW& mw, PathState& ps, Rng& g, float t, int slot) {
-  const DevCamera& cam = S.cam;
-  int kind = SCATTER_NONE;
-  V3 att = mk3(0, 0, 0), sdir = mk3(0, 0, 0);
-  Surf sf{mk3(0, 0, 0), mk3(0, 0, 1), true};
-  if (slot < 0) { // camera.ts:252-258
-    V3 ud = normalize3(ps.ray.d);
-    float a = 0.5f * (ud.y + 1.0f);
-    V3 bg = ld3(cam.bg_top) * (1.0f - a) + ld3(cam.bg_bottom) * a;
-    ps.radiance = ps.radiance + bg * ps.tp;
-  } else {
-    int type, root;
-    F4 p0;
-    if (KIND == BVH_LIST) { type = sm->type(slot); root = sm->mat(slot); p0 = sm->p0(slot); }
-    else { I2 info = ldgi2(S.slot_info + slot); type = (info.y >> 30) & 3; root = info.x; p0 = ldg4(S.p0 + slot); }
-    sf = surface_at(type, p0, ps.ray, t);
-    const I4 mb = ldgi4(S.matB + root);
-    const F4 ma = ldg4(S.matA + root);
-    if (mb.w) { // emitted * throughput (camera.ts:261)
-      F4 e = ldg4(S.matE + root);
-      ps.radiance = ps.radiance + xyz(e) * ps.tp;
-    }
-    if (mb.x == MAT_LAMBERT) { kind = SCATTER_DIFFUSE; att = xyz(ma); }
-    else if (mb.x != MAT_LIGHT) { // a light: scatter == null, emitted only, bounce not counted (camera.ts:267-269)
-      const Scatter sc = scatter_material(S, root, mb, ma, ps.ray.d, sf, g);
-      kind = sc.kind; att = sc.attenuation; sdir = sc.dir;
-    }
-  }
-  if (kind != SCATTER_NONE) ++ps.bounces; // camera.ts:271
-  if (kind == SCATTER_DIFFUSE) { // camera.ts:285-315 with the mixture pdf of pdf.ts:57-99
-    const float u_sel = g.next(), r1 = g.next(), r2 = g.next();
-    float cosv, pdf_value;
-    diffuse_bounce<LV>(S, mw, sf.p, sf.n, u_sel, r1, r2, sdir, cosv, pdf_value);
-    att = att * (cosv * rcp_approx(pdf_value));
-    if (!(pdf_value > 0.0001f)) kind = SCATTER_NONE; // camera.ts:298-301 (NaN also ends the path)
-  }
-  if (kind == SCATTER_NONE) return true;
-  ps.tp = ps.tp * att; // specular: camera.ts:275-282
-  ps.ray = Ray{sf.p, sdir};
-  return false;
-}
-#endif
 
 // One whole rayColor call on the path's current ray.
 template <int KIND, bool LEAF_LOOP = true, bool LV = true>
@@ -609,11 +562,9 @@ k_render_pool(const DevScene S, const RenderParams R) {
         // 1.9 % (Cornell) and 3 % (weekend-final, which has no light at all: register allocation and code placement of the walk)
         ended = path_step<KIND, true, (KIND == BVH_LIST && POOL) || KIND == BVH_REFERENCE>(S, L, sm, mw, ps, g, wc);
       }
-#ifndef RT_NO_RECONVERGE
       // every way a path can end (miss, light, absorbed, roulette, depth, pdf 0) meets here: ONE copy of the end-of-path code
       // instead of one per exit of path_step (measured on Cornell 1024^2 @256: 31.45 -> 30.19 ms)
       __syncwarp();
-#endif
       if (ended) { // pixel.add(rayColor, bounces) — renderStats.ts:76-88
         if (POOL) acc_add(acc, lp, ps.radiance);
         else { own[0] += to_fixed(ps.radiance.x); own[1] += to_fixed(ps.radiance.y); own[2] += to_fixed(ps.radiance.z); }
@@ -828,194 +779,6 @@ __global__ void __launch_bounds__(256, 3) k_render_sorted(const DevScene S, cons
   }
   flush_stats(R, st_pixels, cam.samples, st_paths, st_bounces, st_rays, st_bmin, st_bmax);
 }
-
-// =========================================================================================
-// k_render_wq — fixed spp, default mode: warp-local wavefront.  A warp keeps NS > 32 paths of its item
-// in shared memory and runs STAGES over up to 32 of them at a time: "trace" (closest hit for paths
-// whose next ray is ready) and "shade" for the paths whose hit has one material class.  Every stage
-// takes the fullest queue, so a stage runs with (nearly) all lanes on one piece of code; nothing is
-// shared between warps, so there is no CTA barrier — only __syncwarp between stages.
-//   queues (stacks of slot numbers, counts in warp-uniform registers):
-//     0 lambert  1 metal  2 glass  3 done (light hit, miss, roulette kill, empty slot)  4 mixed  5 layered  6 trace
-//   shade stage: path_post; finished paths are accumulated (exact fixed point) and their slots take
-//   the next (pixel, sample) pairs of the item; then Philox block + roulette test of the next bounce.
-// Path records (88 B): G0 (o, t) G1 (d, slot) G2 (throughput, bounces) G3 (radiance, pixel | sample << 5)
-// G4 (q0..q3) G5 (q4, avail | block << 3).  Bit-identical to k_render_pool (counter-based RNG, exact sums).
-//
-// MEASURED AND NOT USED (compiled only with -DRT_EXPERIMENTAL_WQ; RT_B200_WQ=1..3 selects NS/CTAs):
-// lanes per instruction rise from 22 to 29.6 of 32, but queue upkeep + record traffic add ~390
-// instructions per ray to k_render_pool's ~980, and at 80 registers the records leave too little L1
-// for the spills.  Cornell 1024^2 @1024 spp: 153.5 ms (NS 96, 2 CTAs/SM) vs 128 ms for k_render_pool.
-// =========================================================================================
-#ifdef RT_EXPERIMENTAL_WQ
-enum : int { Q_DONE = 3, Q_TRACE = 6, Q_COUNT = 7 };
-enum : int { SLOT_DEAD = -2, SLOT_EMPTY = -3 };
-
-template <int NS>
-struct alignas(16) WqWarp {
-  float4 st[5][NS];
-  float2 st5[NS];
-  unsigned char q[Q_COUNT][NS];
-  unsigned int acc[32 * 9];
-};
-
-extern __shared__ __align__(16) unsigned char wq_smem[];
-
-template <int KIND, int NS, int BLOCKS>
-__global__ void __launch_bounds__(256, BLOCKS) k_render_wq(const DevScene S, const RenderParams R) {
-  ListSmemData& sm_data = *reinterpret_cast<ListSmemData*>(wq_smem);
-  const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-  WqWarp<NS>& W = reinterpret_cast<WqWarp<NS>*>(wq_smem + (KIND == BVH_LIST ? sizeof(ListSmemData) : 0))[warp];
-  const ListSmem sm = stage_list<KIND>(S, sm_data);
-  const ListSmem& L = sm;
-  const DevCamera& cam = S.cam;
-  const MixW mw = make_mixw(S);
-  const unsigned lt_mask = (1u << lane) - 1u;
-  const unsigned full = 0xffffffffu;
-
-  unsigned int st_pixels = 0, st_paths = 0, st_bounces = 0, st_rays = 0;
-  int st_bmin = 0x7fffffff, st_bmax = 0;
-
-  WarpItem it;
-  while (next_warp_item(R, cam.samples, (cam.width + 7) >> 3, lane, it)) {
-    const int pool = 32 * (it.s_end - it.s_begin); // (pixel, sample) pairs of this item
-    acc_clear(W.acc, lane);
-    int next = 0; // warp-uniform cursor into the pairs
-    for (int s = (int)lane; s < NS; s += 32) { // every slot starts empty in the "done" queue: the first stages fill them
-      W.q[Q_DONE][s] = (unsigned char)s;
-      W.st[1][s].w = __int_as_float(SLOT_EMPTY);
-    }
-    int n[Q_COUNT];
-#pragma unroll
-    for (int c = 0; c < Q_COUNT; ++c) n[c] = c == Q_DONE ? NS : 0;
-    __syncwarp();
-
-    for (;;) {
-      // ---- the fullest queue is the next stage ----
-      int best = Q_TRACE, cnt = n[Q_TRACE];
-#pragma unroll
-      for (int c = 0; c < Q_TRACE; ++c)
-        if (n[c] > cnt) { cnt = n[c]; best = c; }
-      if (cnt == 0) break;
-      const int k = min(cnt, 32), base = cnt - k;
-#pragma unroll
-      for (int c = 0; c < Q_COUNT; ++c)
-        if (c == best) n[c] = base;
-      const bool active = (int)lane < k;
-      const int idx = active ? (int)W.q[best][base + (int)lane] : 0;
-      int cls = -1; // queue this slot goes to next
-      if (best == Q_TRACE) {
-        if (active) {
-          const float4 a0 = W.st[0][idx], a1 = W.st[1][idx];
-          const Ray r{mk3(a0.x, a0.y, a0.z), mk3(a1.x, a1.y, a1.z)};
-          float t;
-          int slot;
-          ++st_rays;
-          closest_hit<KIND>(S, L, r, t, slot); // world.hit(r, (0.001, inf)) — camera.ts:249
-          W.st[0][idx].w = t;
-          W.st[1][idx].w = __int_as_float(slot);
-          cls = Q_DONE;
-          if (slot >= 0) {
-            const int root = KIND == BVH_LIST ? sm.mat(slot) : ldgi2(S.slot_info + slot).x;
-            const int type = __ldg(&S.matB[root].x);
-            cls = type == MAT_LIGHT ? Q_DONE : type;
-          }
-        }
-#pragma unroll
-        for (int c = 0; c < Q_TRACE; ++c) {
-          const unsigned m = __ballot_sync(full, cls == c);
-          if (cls == c) W.q[c][n[c] + __popc(m & lt_mask)] = (unsigned char)idx;
-          n[c] += __popc(m);
-        }
-      } else {
-        PathState ps{Ray{mk3(0, 0, 0), mk3(0, 0, 1)}, mk3(1, 1, 1), mk3(0, 0, 0), 0};
-        Rng g;
-        g.seed_lo = S.seed_lo; g.seed_hi = S.seed_hi;
-        g.k0 = g.k1 = g.stream = g.block = 0; g.q0 = g.q1 = g.q2 = g.q3 = g.q4 = 0; g.avail = 0;
-        int lp = 0, slot = SLOT_EMPTY;
-        uint32_t sample = 0;
-        bool want = false, start = false, fresh = false;
-        if (active) {
-          const float4 a0 = W.st[0][idx], a1 = W.st[1][idx];
-          slot = __float_as_int(a1.w);
-          want = true;
-          if (slot != SLOT_EMPTY) {
-            const float4 a2 = W.st[2][idx], a3 = W.st[3][idx], a4 = W.st[4][idx];
-            const float2 a5 = W.st5[idx];
-            ps.ray.o = mk3(a0.x, a0.y, a0.z);
-            ps.ray.d = mk3(a1.x, a1.y, a1.z);
-            ps.tp = mk3(a2.x, a2.y, a2.z); ps.bounces = __float_as_int(a2.w);
-            ps.radiance = mk3(a3.x, a3.y, a3.z);
-            const int ls = __float_as_int(a3.w);
-            lp = ls & 31; sample = (uint32_t)ls >> 5;
-            g.q0 = __float_as_uint(a4.x); g.q1 = __float_as_uint(a4.y); g.q2 = __float_as_uint(a4.z); g.q3 = __float_as_uint(a4.w);
-            g.q4 = __float_as_uint(a5.x);
-            const int ab = __float_as_int(a5.y);
-            g.avail = ab & 7; g.block = (uint32_t)ab >> 3;
-            g.k0 = (uint32_t)(it.py0 + (lp >> 3)) * (uint32_t)cam.width + (uint32_t)(it.px0 + (lp & 7));
-            g.k1 = sample; g.stream = (uint32_t)ps.bounces;
-            const bool fin = slot == SLOT_DEAD || path_post<KIND>(S, &sm, mw, ps, g, a0.w, slot);
-            if (fin) { // pixel.add(rayColor, bounces) — renderStats.ts:76-88
-              acc_add(W.acc, lp, ps.radiance);
-              ++st_paths;
-              st_bounces += (unsigned)ps.bounces;
-              st_bmin = min(st_bmin, ps.bounces);
-              st_bmax = max(st_bmax, ps.bounces);
-            } else { want = false; start = true; }
-          }
-        }
-        // ---- finished and empty slots take the next pairs of the item ----
-        const unsigned need = __ballot_sync(full, want);
-        int px = 0, py = 0;
-        if (want) {
-          const int pair = next + __popc(need & lt_mask);
-          if (pair < pool) {
-            lp = pair & 31;
-            px = it.px0 + (lp & 7);
-            py = it.py0 + (lp >> 3);
-            if (px >= R.x0 && px < R.x1 && py >= R.y0 && py < R.y1) {
-              fresh = start = true;
-              sample = (uint32_t)(it.s_begin + (pair >> 5));
-              ps.tp = mk3(1, 1, 1); ps.radiance = mk3(0, 0, 0); ps.bounces = 0;
-            } else { // pairs of pixels outside the region are dropped; the slot asks again
-              cls = Q_DONE;
-              W.st[1][idx].w = __int_as_float(SLOT_EMPTY);
-            }
-          }
-        }
-        next = min(next + __popc(need), pool);
-        if (start) {
-          const uint32_t pixel = (uint32_t)(it.py0 + (lp >> 3)) * (uint32_t)cam.width + (uint32_t)(it.px0 + (lp & 7));
-          g.begin(pixel, sample, (uint32_t)ps.bounces, S.seed_lo, S.seed_hi); // one Philox block per bounce
-          if (fresh) ps.ray = camera_ray(cam, px, py, g, true);
-          const bool dead = path_pre(cam, ps, g);
-          cls = dead ? Q_DONE : Q_TRACE;
-          W.st[0][idx] = make_float4(ps.ray.o.x, ps.ray.o.y, ps.ray.o.z, 0.f);
-          W.st[1][idx] = make_float4(ps.ray.d.x, ps.ray.d.y, ps.ray.d.z, __int_as_float(SLOT_DEAD));
-          W.st[2][idx] = make_float4(ps.tp.x, ps.tp.y, ps.tp.z, __int_as_float(ps.bounces));
-          W.st[3][idx] = make_float4(ps.radiance.x, ps.radiance.y, ps.radiance.z, __int_as_float(lp | (int)(sample << 5)));
-          W.st[4][idx] = make_float4(__uint_as_float(g.q0), __uint_as_float(g.q1), __uint_as_float(g.q2), __uint_as_float(g.q3));
-          W.st5[idx] = make_float2(__uint_as_float(g.q4), __int_as_float(g.avail | (int)(g.block << 3)));
-        }
-        {
-          const unsigned m = __ballot_sync(full, cls == Q_TRACE);
-          if (cls == Q_TRACE) W.q[Q_TRACE][n[Q_TRACE] + __popc(m & lt_mask)] = (unsigned char)idx;
-          n[Q_TRACE] += __popc(m);
-          const unsigned md = __ballot_sync(full, cls == Q_DONE);
-          if (cls == Q_DONE) W.q[Q_DONE][n[Q_DONE] + __popc(md & lt_mask)] = (unsigned char)idx;
-          n[Q_DONE] += __popc(md);
-        }
-      }
-      __syncwarp();
-    }
-    unsigned long long sum[3];
-    acc_read(W.acc, lane, sum);
-    st_pixels += item_epilogue(R, cam, it, lane, sum);
-    __syncwarp(); // acc is cleared at the top of the next item
-  }
-  flush_stats(R, st_pixels, cam.samples, st_paths, st_bounces, st_rays, st_bmin, st_bmax);
-}
-#endif // RT_EXPERIMENTAL_WQ
 
 // =========================================================================================
 // k_render_trav — fixed spp, default mode, SAH trees: traversal interleaved with shading.
@@ -1872,31 +1635,6 @@ static cudaError_t launch_persistent(K kernel, const DevScene& S, const RenderPa
   return cudaGetLastError();
 }
 
-#ifdef RT_EXPERIMENTAL_WQ
-template <int KIND, int NS, int BLOCKS>
-static cudaError_t launch_wq(const DevScene& S, const RenderParams& R, long long ctas_of_work, int sms, cudaStream_t st) {
-  auto kernel = k_render_wq<KIND, NS, BLOCKS>;
-  const int smem = (int)((KIND == BVH_LIST ? sizeof(ListSmemData) : 0) + 8 * sizeof(WqWarp<NS>));
-  static cudaError_t attr = [&]() {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return e;
-    // just enough shared memory for BLOCKS resident CTAs (1 KB per CTA is reserved); the rest stays L1
-    int pct = (int)((BLOCKS * (smem + 1024) * 100LL + 228 * 1024 - 1) / (228 * 1024));
-    return cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct > 100 ? 100 : pct);
-  }();
-  if (attr != cudaSuccess) return attr;
-  int per_sm = 0;
-  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, smem);
-  if (e != cudaSuccess) return e;
-  if (per_sm < 1) per_sm = 1;
-  long long resident = (long long)sms * per_sm;
-  int grid = (int)(ctas_of_work < resident ? ctas_of_work : resident);
-  if (grid < 1) grid = 1;
-  kernel<<<grid, 256, smem, st>>>(S, R);
-  return cudaGetLastError();
-}
-#endif
-
 cudaError_t launch_render_mega(const DevScene& S, const RenderParams& R, int sms, cudaStream_t st) {
   if (R.x1 <= R.x0 || R.y1 <= R.y0) return cudaSuccess;
   const long long tiles = (long long)R.tiles_x * R.tiles_y;
@@ -1942,14 +1680,6 @@ cudaError_t launch_render_mega(const DevScene& S, const RenderParams& R, int sms
       // samples per item: 107.1 vs 107.8 ms; one part of eight, 57 samples per item: 14.35 vs 13.87 ms (ideal 13.39).
       if (pool_list || (R.s_cnt > 0 ? R.s_cnt : S.cam.samples) / (R.chunks > 0 ? R.chunks : 1) < 128)
         return launch_persistent(k_render_pool<BVH_LIST, true>, S, R, work, sms, st, RT_LIST_THREADS);
-#ifdef RT_EXPERIMENTAL_WQ
-      {
-        static const int wq = getenv("RT_B200_WQ") ? atoi(getenv("RT_B200_WQ")) : 0;
-        if (wq == 1) return launch_wq<BVH_LIST, 48, 3>(S, R, work, sms, st);
-        if (wq == 2) return launch_wq<BVH_LIST, 64, 3>(S, R, work, sms, st);
-        if (wq == 3) return launch_wq<BVH_LIST, 96, 2>(S, R, work, sms, st);
-      }
-#endif
       if (sorted_list) {
         // 3 CTAs x 43.4 KB fit the 132 KB split; the rest stays L1.  Function attributes are per device, and one
         // process may drive several GPUs, so this is set at every launch (microseconds, once per render).

@@ -62,6 +62,31 @@ def test_no_cpu_fallback_without_device():
         createCameraFromSceneData(generateCornellSceneData(), {"width": 16})
 
 
+def test_render_output_arrays_are_checked_before_the_library_writes_them():
+    """The library writes RGB8 and linear through their base pointers as C-contiguous [H][W][3]: every render method
+    (Camera.renderRegion / renderProgressive / renderDenoised, MultiCamera.renderRegion / renderDenoised) refuses an
+    array it would write past or around."""
+    from mcp_raytracer_b200 import RaytracerError
+    from mcp_raytracer_b200.camera import _image_outputs
+
+    W, H = 5, 4
+    rgb8, linear = np.zeros((H, W, 3), np.uint8), np.zeros((H, W, 3), np.float32)
+    assert _image_outputs(rgb8, linear, W, H) == (rgb8.ctypes.data, rgb8.nbytes, linear.ctypes.data)
+    assert _image_outputs(None, None, W, H) == (None, 0, None)
+    with pytest.raises(RaytracerError, match="linear buffer"):  # a view with strides: writing it as contiguous corrupts it
+        _image_outputs(None, np.zeros((H, 2 * W, 3), np.float32)[:, ::2], W, H)
+    with pytest.raises(RaytracerError, match="linear buffer"):
+        _image_outputs(None, np.zeros((H, W, 3), np.float32).transpose(1, 0, 2).copy(order="F"), W, H)
+    with pytest.raises(RaytracerError, match="linear buffer"):
+        _image_outputs(None, linear.astype(np.float64), W, H)
+    with pytest.raises(RaytracerError, match="linear buffer"):
+        _image_outputs(None, linear[:-1], W, H)
+    with pytest.raises(RaytracerError, match="pixel buffer"):
+        _image_outputs(rgb8[:, ::-1], None, W, H)
+    with pytest.raises(RaytracerError, match="pixel buffer"):
+        _image_outputs(rgb8.astype(np.int8), None, W, H)
+
+
 def test_scene_errors_are_reported_before_device_checks():
     from mcp_raytracer_b200 import _native
     from mcp_raytracer_b200.scene_data import FlatScene, merge_render_options, render_opts_struct
