@@ -284,6 +284,17 @@ rt_status rt_denoise(int32_t device, int32_t width, int32_t height, const float*
  * render modes other than RT_MODE_DEFAULT.  Synchronous. */
 rt_status rt_camera_render_denoised(rt_camera* cam, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear_rgb,
                                     const rt_denoise_opts* opts, rt_stats* stats);
+/* rt_camera_render_progressive with a denoised preview: passes, caps, on_pass and stats as that call.  After each pass
+ * rgb8 / linear_rgb hold the region's filtered image of the samples so far, and `moments` (optional HOST [H][W][8], the
+ * layout of rt_camera_render_moments) the render's moments.  The features are computed once, in the first pass, from the
+ * first min(samples, 8) samples; the filter reads the noisy colour, which stays on the device.  The last pass is
+ * bit-identical to rt_camera_render_denoised (rgb8, linear_rgb, stats except device_ms and kernel_launches) and its moments
+ * to rt_camera_render_moments.  Errors as rt_camera_render_denoised, and RT_ERR_INVALID_ARGUMENT for n_passes < 1.
+ * Synchronous. */
+rt_status rt_camera_render_progressive_denoised(rt_camera* cam, const rt_region* region, uint8_t* rgb8, size_t rgb8_len,
+                                                float* linear_rgb, float* moments, int32_t n_passes,
+                                                const rt_denoise_opts* opts, rt_progress_fn on_pass, void* user,
+                                                rt_stats* stats);
 
 /* ---- one process, N GPUs: replaces the worker pool of generateImageBuffer(parallel: true)
  *      (src/raytracer.ts:60-90: N worker_threads over row strips of a SharedArrayBuffer, RenderStats.merge) ----

@@ -109,6 +109,38 @@ def _image_outputs(rgb8: Optional[np.ndarray], linear: Optional[np.ndarray], W: 
             linear.ctypes.data if linear is not None else None)
 
 
+def _moments_output(moments: Optional[np.ndarray], W: int, H: int):
+    """Check the moments output array of a render of a W x H image (None = not wanted): the library writes it through its
+    base pointer as a C-contiguous [H][W][8] float32 array.  Returns its pointer."""
+    if moments is None:
+        return None
+    if moments.dtype != np.float32 or moments.size < W * H * 8 or not moments.flags["C_CONTIGUOUS"]:
+        raise RaytracerError("moments buffer must be a C-contiguous float32 [H][W][8] array")
+    return moments.ctypes.data
+
+
+def _progressive(onPass, call) -> None:
+    """Run the progressive library call `call(fn)` with `fn` the rt_progress_fn that calls
+    onPass(pass, passes, samplesCap, RenderStats) after each pass (None = no callback); a true result stops the render.  An
+    exception in onPass stops the render too, and is raised once the library has returned: it never unwinds through the C
+    frame."""
+    errors: List[BaseException] = []
+
+    @C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.POINTER(rt_stats))
+    def cb(_user, k, n, cap, so_far):
+        if onPass is None:
+            return 0
+        try:
+            return 1 if onPass(int(k), int(n), int(cap), RenderStats.from_struct(so_far.contents)) else 0
+        except BaseException as e:  # noqa: BLE001
+            errors.append(e)
+            return 1
+
+    _check(call(C.cast(cb, C.c_void_p)))
+    if errors:
+        raise errors[0]
+
+
 def _region_struct(region: Optional[Dict[str, int]], W: int, H: int) -> rt_region:
     if region is None:
         return rt_region(0, 0, W, H)
@@ -199,22 +231,8 @@ class Camera:
         bp, bl, lp = _image_outputs(pixelData, linear, W, H)
         reg = _region_struct(region, W, H)
         st = rt_stats()
-        errors: List[BaseException] = []
-
-        @C.CFUNCTYPE(C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.POINTER(rt_stats))
-        def cb(_user, k, n, cap, so_far):
-            if onPass is None:
-                return 0
-            try:
-                return 1 if onPass(int(k), int(n), int(cap), RenderStats.from_struct(so_far.contents)) else 0
-            except BaseException as e:  # noqa: BLE001 — never unwind through the C frame
-                errors.append(e)
-                return 1
-
-        _check(_native.lib().rt_camera_render_progressive(self._h, C.byref(reg), bp, bl, lp, int(passes), C.cast(cb, C.c_void_p), None,
-                                                          C.byref(st)))
-        if errors:
-            raise errors[0]
+        _progressive(onPass, lambda fn: _native.lib().rt_camera_render_progressive(self._h, C.byref(reg), bp, bl, lp, int(passes), fn,
+                                                                                   None, C.byref(st)))
         return RenderStats.from_struct(st)
 
     def renderRegionDevice(self, region, rgb8_ptr: int = 0, linear_ptr: int = 0, moments_ptr: int = 0, stats_ptr: int = 0) -> None:
@@ -259,6 +277,22 @@ class Camera:
         opts = denoise_opts_struct(options)
         st = rt_stats()
         _check(_native.lib().rt_camera_render_denoised(self._h, C.byref(reg), bp, bl, lp, C.byref(opts), C.byref(st)))
+        return RenderStats.from_struct(st)
+
+    def renderProgressiveDenoised(self, pixelData: Optional[np.ndarray], passes: int, onPass=None, region: Optional[Dict[str, int]] = None,
+                                  linear: Optional[np.ndarray] = None, moments: Optional[np.ndarray] = None,
+                                  options: Optional[Dict[str, Any]] = None) -> RenderStats:
+        """`renderProgressive` with a denoised preview (rt_camera_render_progressive_denoised): after each pass `pixelData` /
+        `linear` hold the filtered image of the samples so far and `moments` ([H][W][8], optional) the render's moments,
+        then onPass runs as in `renderProgressive`.  The last pass gives the bytes of `renderDenoised`.  options as there."""
+        W, H = self.imageWidth, self.imageHeight
+        bp, bl, lp = _image_outputs(pixelData, linear, W, H)
+        mp = _moments_output(moments, W, H)
+        reg = _region_struct(region, W, H)
+        opts = denoise_opts_struct(options)
+        st = rt_stats()
+        _progressive(onPass, lambda fn: _native.lib().rt_camera_render_progressive_denoised(
+            self._h, C.byref(reg), bp, bl, lp, mp, int(passes), C.byref(opts), fn, None, C.byref(st)))
         return RenderStats.from_struct(st)
 
     # -- per-function parity hooks (rt_debug_*): one device function of the render path on explicit inputs --

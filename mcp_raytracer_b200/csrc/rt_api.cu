@@ -180,6 +180,7 @@ struct rt_camera {
   float* d_fnrm = nullptr;
   float* d_fdepth = nullptr;
   float* d_dn = nullptr;     // denoiser scratch: dn_floats_per_pixel floats per pixel
+  float* d_dnout = nullptr;  // progressive denoised renders: the filtered [H][W][3] image (d_linear keeps the noisy colour)
   unsigned long long* d_stats = nullptr;
   // work queue of the render kernel: [0] = next item, [1..] = finished chunks per tile
   int* d_queue = nullptr;
@@ -228,7 +229,7 @@ static void free_camera(rt_camera* c) {
   for (void* p : c->allocs) dev_free(p);
   dev_free(c->d_rgb8); dev_free(c->d_linear); dev_free(c->d_moments); dev_free(c->d_ids);
   dev_free(c->d_t); dev_free(c->d_normal); dev_free(c->d_front); dev_free(c->d_falb); dev_free(c->d_fnrm); dev_free(c->d_fdepth);
-  dev_free(c->d_dn); dev_free(c->d_stats); dev_free(c->d_queue); dev_free(c->d_scratch); dev_free(c->d_pixstate); dev_free(c->d_adrec);
+  dev_free(c->d_dn); dev_free(c->d_dnout); dev_free(c->d_stats); dev_free(c->d_queue); dev_free(c->d_scratch); dev_free(c->d_pixstate); dev_free(c->d_adrec);
   wf_release(c);
   if (c->ev0) cudaEventDestroy(c->ev0);
   if (c->ev1) cudaEventDestroy(c->ev1);
@@ -770,6 +771,9 @@ static rt_status timed_render(rt_camera* c, RenderParams& P, cudaEvent_t end, un
 
 static rt_status denoise_band(rt_camera* c, const RenderParams& P, int b0, int b1, const DenoiseParams& opts, const float* color,
                               const float* moments, float* out, uint8_t* rgb8, bool poison, int* launches);
+static rt_status denoise_features(rt_camera* c, const RenderParams& P, int b0, int b1, int iterations, bool poison, int* launches);
+static rt_status denoise_filter(rt_camera* c, const RenderParams& P, int b0, int b1, const DenoiseParams& opts, const float* color,
+                                const float* moments, float* out, uint8_t* rgb8, int* launches);
 
 // Render the region and copy it to the caller's [H][W] arrays.  With `dn`, the colour and moments stay on the device and
 // are filtered in place before ev1 (one band covering the region); RGB8 is written from the filtered image.
@@ -857,8 +861,10 @@ rt_status rt_camera_render_moments(rt_camera* cam, const rt_region* region, uint
 }
 
 // Progressive render: the same image as rt_camera_render_region, delivered in n_passes growing prefixes of the samples.
-rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear, int32_t n_passes,
-                                       rt_progress_fn on_pass, void* user, rt_stats* stats) {
+// With `dn`, every pass also renders the moments and filters the region into d_dnout (see rt_camera_render_progressive_denoised);
+// `moments` (host, optional) receives them after each pass.
+static rt_status progressive_host(rt_camera* c, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear, float* moments,
+                                  int32_t n_passes, rt_progress_fn on_pass, void* user, rt_stats* stats, const DenoiseParams* dn = nullptr) {
   RT_GUARD_BEGIN
   if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
   if (n_passes < 1) return fail(RT_ERR_INVALID_ARGUMENT, "n_passes must be >= 1");
@@ -870,10 +876,15 @@ rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, ui
   RenderParams P0;
   rt_status st = clip_region(c, region, P0);
   if (st != RT_OK) return st;
+  const bool with_moments = moments || dn;
   if (rgb8 && !c->d_rgb8) CU(dev_alloc(&c->d_rgb8, npx * 3));
-  if (linear && !c->d_linear) CU(dev_alloc(&c->d_linear, npx * 3 * sizeof(float)));
+  if ((linear || dn) && !c->d_linear) CU(dev_alloc(&c->d_linear, npx * 3 * sizeof(float)));
+  if (with_moments && !c->d_moments) CU(dev_alloc(&c->d_moments, npx * 8 * sizeof(float)));
+  if (dn && !c->d_dnout) CU(dev_alloc(&c->d_dnout, npx * 3 * sizeof(float)));
   const int S = c->hs->cam.samples;
-  const bool stream = c->hs->cam.adaptive || c->hs->cam.mode != 0;
+  // moments run the pixel stream at fixed spp too (render_needs_full), which counts a pixel in the pass that completes it.
+  // At fixed spp both rules give the same totals (no pixel completes before the last pass), so no test can tell them apart.
+  const bool stream = c->hs->cam.adaptive || c->hs->cam.mode != 0 || with_moments;
   const int batch = c->hs->cam.adaptive ? std::max(1, c->hs->cam.a_batch) : 1;
   rt_stats total = unpack_stats(kStatsInit);
   int prev = 0, passes_run = 0;
@@ -885,15 +896,33 @@ rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, ui
     else cap = S;
     if ((int)cap <= prev && !(S <= 0 && k == n_passes)) continue; // nothing new in this pass (more passes than samples)
     RenderParams P = P0;
-    P.rgb8 = rgb8 ? c->d_rgb8 : nullptr;
-    P.linear = linear ? c->d_linear : nullptr;
-    const ProgPass pass{prev, (int)cap, passes_run == 0};
+    P.rgb8 = rgb8 && !dn ? c->d_rgb8 : nullptr;
+    P.linear = linear || dn ? c->d_linear : nullptr;
+    P.moments = with_moments ? c->d_moments : nullptr;
+    // The filter writes d_dnout, never the noisy colour in d_linear: a pixel that converged in an earlier pass is not
+    // rendered again, and the next pass's filter must read its noisy colour.  The features are a function of (pixel,
+    // sample) only: the first pass computes them, with the sample count of the one-shot call, for every later pass.
+    std::function<rt_status(int*)> denoise;
+    const bool first = passes_run == 0;
+    if (dn)
+      denoise = [&](int* l) {
+        int lf = 0;
+        if (first) {
+          rt_status s = denoise_features(c, P, P.y0, P.y1, dn->iterations, false, &lf);
+          if (s != RT_OK) return s;
+        }
+        rt_status s = denoise_filter(c, P, P.y0, P.y1, *dn, P.linear, P.moments, c->d_dnout, rgb8 ? c->d_rgb8 : nullptr, l);
+        *l += lf;
+        return s;
+      };
+    const ProgPass pass{prev, (int)cap, first};
     int launches = 0;
     unsigned long long raw[kStatCount];
-    st = timed_render(c, P, c->ev1, raw, &launches, (S > 0 && n_passes > 1) ? &pass : nullptr);
+    st = timed_render(c, P, c->ev1, raw, &launches, (S > 0 && n_passes > 1) ? &pass : nullptr, denoise);
     if (st != RT_OK) return st;
     if (rgb8) CU(copy_region(rgb8, c->d_rgb8, 3, P0, W, cudaMemcpyDeviceToHost, c->stream));
-    if (linear) CU(copy_region(linear, c->d_linear, 12, P0, W, cudaMemcpyDeviceToHost, c->stream));
+    if (linear) CU(copy_region(linear, dn ? c->d_dnout : c->d_linear, 12, P0, W, cudaMemcpyDeviceToHost, c->stream));
+    if (moments) CU(copy_region(moments, c->d_moments, 32, P0, W, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     rt_stats ps = unpack_stats(raw);
     ps.kernel_launches = launches;
@@ -915,6 +944,11 @@ rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, ui
   if (stats) *stats = total;
   return RT_OK;
   RT_GUARD_END
+}
+
+rt_status rt_camera_render_progressive(rt_camera* c, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear, int32_t n_passes,
+                                       rt_progress_fn on_pass, void* user, rt_stats* stats) {
+  return progressive_host(c, region, rgb8, rgb8_len, linear, nullptr, n_passes, on_pass, user, stats);
 }
 
 rt_status rt_camera_trace_primary(rt_camera* c, const rt_region* region, int32_t* obj_id, float* t, float* normal,
@@ -979,10 +1013,20 @@ static rt_status features_prepare(rt_camera* c, size_t npx) {
 // fills those buffers with NaN, so that a read outside the computed rows changes the image.
 static rt_status denoise_band(rt_camera* c, const RenderParams& P, int b0, int b1, const DenoiseParams& opts, const float* color,
                               const float* moments, float* out, uint8_t* rgb8, bool poison, int* launches) {
+  int lf = 0;
+  rt_status st = denoise_features(c, P, b0, b1, opts.iterations, poison, &lf);
+  if (st != RT_OK) return st;
+  st = denoise_filter(c, P, b0, b1, opts, color, moments, out, rgb8, launches);
+  *launches += lf;
+  return st;
+}
+
+// Feature step of denoise_band: the first-hit features of the rows a band's filter with `iterations` passes reads, over the
+// one-shot render's first min(samples, 8) camera rays per pixel.
+static rt_status denoise_features(rt_camera* c, const RenderParams& P, int b0, int b1, int iterations, bool poison, int* launches) {
   *launches = 0;
   if (P.x1 <= P.x0 || b1 <= b0) return RT_OK;
-  const int W = c->hs->image_width;
-  const size_t npx = (size_t)W * c->hs->image_height;
+  const size_t npx = (size_t)c->hs->image_width * c->hs->image_height;
   rt_status st = features_prepare(c, npx);
   if (st != RT_OK) return st;
   if (!c->d_dn) CU(dev_alloc(&c->d_dn, npx * kDnFloatsPerPixel * sizeof(float)));
@@ -993,11 +1037,23 @@ static rt_status denoise_band(rt_camera* c, const RenderParams& P, int b0, int b
     CU(cudaMemsetAsync(c->d_dn, 0xff, npx * kDnFloatsPerPixel * sizeof(float), c->stream));
   }
   RenderParams F = P; // the feature rows: one beyond what prepare computes
-  const int hf = dn_halo(opts.iterations, -1) + 1;
+  const int hf = dn_halo(iterations, -1) + 1;
   F.y0 = std::max(P.y0, b0 - hf);
   F.y1 = std::min(P.y1, b1 + hf);
   const int n_feat = std::max(1, std::min(c->hs->cam.samples, 8));
   CU(launch_render_features(c->ds, F, n_feat, c->d_falb, c->d_fnrm, c->d_fdepth, c->stream));
+  *launches = 1;
+  return RT_OK;
+}
+
+// Filter step of denoise_band: prepare, the a-trous passes and finish of the band, on the features denoise_features left.
+static rt_status denoise_filter(rt_camera* c, const RenderParams& P, int b0, int b1, const DenoiseParams& opts, const float* color,
+                                const float* moments, float* out, uint8_t* rgb8, int* launches) {
+  *launches = 0;
+  if (P.x1 <= P.x0 || b1 <= b0) return RT_OK;
+  const int W = c->hs->image_width;
+  const size_t npx = (size_t)W * c->hs->image_height;
+  if (!c->d_dn) CU(dev_alloc(&c->d_dn, npx * kDnFloatsPerPixel * sizeof(float)));
   DenoiseParams D = opts;
   D.width = W;
   D.x0 = P.x0; D.y0 = P.y0; D.x1 = P.x1; D.y1 = P.y1;
@@ -1005,9 +1061,7 @@ static rt_status denoise_band(rt_camera* c, const RenderParams& P, int b0, int b
   dn_scratch(D, c->d_dn, npx);
   D.out = out;
   D.rgb8 = rgb8;
-  int dn_launches = 0;
-  CU(launch_denoise(D, b0, b1, c->stream, &dn_launches));
-  *launches = 1 + dn_launches;
+  CU(launch_denoise(D, b0, b1, c->stream, launches));
   return RT_OK;
 }
 
@@ -1090,6 +1144,24 @@ rt_status rt_camera_render_denoised(rt_camera* c, const rt_region* region, uint8
   if (c->opts.part_count > 1) return fail(RT_ERR_UNSUPPORTED, "denoised renders are not partitioned");
   if (c->hs->cam.mode != RT_MODE_DEFAULT) return fail(RT_ERR_UNSUPPORTED, "denoised renders need the default render mode");
   return render_host(c, region, rgb8, rgb8_len, linear, nullptr, stats, &D);
+  RT_GUARD_END
+}
+
+// Progressive render with a denoised preview after every pass; the last pass is rt_camera_render_denoised's image.
+rt_status rt_camera_render_progressive_denoised(rt_camera* c, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
+                                                float* moments, int32_t n_passes, const rt_denoise_opts* opts, rt_progress_fn on_pass,
+                                                void* user, rt_stats* stats) {
+  RT_GUARD_BEGIN
+  if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
+  if (n_passes < 1) return fail(RT_ERR_INVALID_ARGUMENT, "n_passes must be >= 1");
+  DenoiseParams D{};
+  rt_status st = dn_options(opts, D);
+  if (st != RT_OK) return st;
+  if (rgb8 && rgb8_len < (size_t)c->hs->image_width * c->hs->image_height * 3)
+    return fail(RT_ERR_BUFFER_TOO_SMALL, "rgb8 buffer smaller than width*height*3");
+  if (c->opts.part_count > 1) return fail(RT_ERR_UNSUPPORTED, "denoised renders are not partitioned");
+  if (c->hs->cam.mode != RT_MODE_DEFAULT) return fail(RT_ERR_UNSUPPORTED, "denoised renders need the default render mode");
+  return progressive_host(c, region, rgb8, rgb8_len, linear, moments, n_passes, on_pass, user, stats, &D);
   RT_GUARD_END
 }
 

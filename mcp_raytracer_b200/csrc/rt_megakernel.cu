@@ -980,6 +980,13 @@ __device__ __noinline__ void pixstate_store(PixState* ps, size_t pi, float cx, f
   p.sum_ill = s1; p.sum_ill2 = s2; p.samples = samples; p.bounces = bounces; p.done = done;
   ps[pi] = p;
 }
+// Welford second moment of a pixel a later progressive pass picks up: stream_write_pixel left it in the moments buffer at
+// the end of the previous pass (FP32 in, FP32 out, so the sequence continues as in the one-shot render).  Not in PixState,
+// whose layout k_render_adaptive's 64-bit accessors rely on.  Out of line like pixstate_load.
+__device__ __noinline__ V3 moments_m2_load(const float* moments, size_t pi) {
+  const float* m = moments + pi * 8;
+  return mk3(m[3], m[4], m[5]);
+}
 
 // The warp's pixel stream: lanes named in `want` take the next pixels, in lane order, from the current 8x4 block;
 // when it runs out the next block that belongs to this GPU and touches the region is popped from the queue.
@@ -1036,8 +1043,14 @@ __device__ __noinline__ StreamTake stream_take(unsigned want, int cursor, int bl
 #ifndef RT_STREAM_LIST_BLOCKS
 #define RT_STREAM_LIST_BLOCKS RT_MIN_BLOCKS
 #endif
-template <int KIND, bool SHADOW = false> // SHADOW: the shadow-ray estimator (path_post_shadow)
-__global__ void __launch_bounds__(256, KIND == BVH_LIST ? RT_STREAM_LIST_BLOCKS : RT_MIN_BLOCKS) k_render_stream(const DevScene S, const RenderParams R) {
+// SHADOW: the shadow-ray estimator (path_post_shadow).  RESUME: a later progressive pass (k_render_stream_resume), which
+// picks pixels up from R.pixstate.  Its warps may take only pixels that stopped in earlier passes, so a warp left without a
+// pixel goes on taking until the stream is exhausted; with moments it also reloads each pixel's Welford M2
+// (moments_m2_load).  One-shot renders never take such a pixel, so a warp with no pixel after a take has exhausted the
+// stream.  Separate instantiations keep their kernels as they were: the reload in a shared kernel cost the one-shot
+// moments render 0.3 % and changed the spills of another (profiles/README.md section 9.2).
+template <int KIND, bool SHADOW, bool RESUME>
+__device__ __forceinline__ void render_stream(const DevScene& S, const RenderParams& R) {
   __shared__ ListSmemData sm_data;
   const ListSmem sm = stage_list<KIND>(S, sm_data);
   const ListSmem& L = sm;
@@ -1103,11 +1116,19 @@ __global__ void __launch_bounds__(256, KIND == BVH_LIST ? RT_STREAM_LIST_BLOCKS 
         samples0 = 0; bounces0 = 0;
         if (R.pixstate && R.s0 > 0) { // a later pass (s0 = the previous cap): pick the pixel up where the last pass left it
           if (pixstate_load(R.pixstate, (size_t)j * cam.width + i, color.x, color.y, color.z, sum_ill, sum_ill2, samples, bounces_sum)) have_px = false;
+          else if constexpr (RESUME) {
+            if (R.moments) { const V3 m2 = moments_m2_load(R.moments, (size_t)j * cam.width + i); m2x = m2.x; m2y = m2.y; m2z = m2.z; }
+          }
           samples0 = samples; bounces0 = bounces_sum;
         }
       }
     }
-    if (__all_sync(full, !have_px)) break; // stream exhausted and every pixel written
+    if (__all_sync(full, !have_px)) {
+      if constexpr (RESUME) {
+        if (!(queue_empty && cursor >= 32)) continue; // every pixel taken had stopped in an earlier pass: take more
+      }
+      break; // stream exhausted and every pixel written
+    }
 
     bool stop = have_px && cam.samples <= 0; // while (0 < 0): the pixel gets no sample at all
     bool final_ = stop;
@@ -1157,14 +1178,23 @@ __global__ void __launch_bounds__(256, KIND == BVH_LIST ? RT_STREAM_LIST_BLOCKS 
   flush_stats_range(R, t_pixels, t_smin, t_smax, t_samples, t_bounces, wc.rays, t_bmin, t_bmax);
   flush_work(R, wc);
 }
+template <int KIND, bool SHADOW = false>
+__global__ void __launch_bounds__(256, KIND == BVH_LIST ? RT_STREAM_LIST_BLOCKS : RT_MIN_BLOCKS) k_render_stream(const DevScene S, const RenderParams R) {
+  render_stream<KIND, SHADOW, false>(S, R);
+}
+template <int KIND, bool SHADOW = false>
+__global__ void __launch_bounds__(256, KIND == BVH_LIST ? RT_STREAM_LIST_BLOCKS : RT_MIN_BLOCKS) k_render_stream_resume(const DevScene S, const RenderParams R) {
+  render_stream<KIND, SHADOW, true>(S, R);
+}
 
 // =========================================================================================
 // k_render_stream_trav — k_render_stream for deep SAH trees: the pixel stream of k_render_stream with the
 // resumable traversal of k_render_trav (bursts interleaved with shading), so a lane whose ray finished
 // early shades, takes its next sample or its next pixel while the others still walk the tree.  Per-pixel
-// arithmetic and its order are those of k_render_stream: identical output.
+// arithmetic and its order are those of k_render_stream: identical output.  RESUME as in render_stream.
 // =========================================================================================
-__global__ void __launch_bounds__(256, RT_MIN_BLOCKS) k_render_stream_trav(const DevScene S, const RenderParams R) {
+template <bool RESUME>
+__device__ __forceinline__ void render_stream_trav(const DevScene& S, const RenderParams& R) {
   const DevCamera& cam = S.cam;
   const MixW mw = make_mixw(S);
   const unsigned lane = threadIdx.x & 31u, full = 0xffffffffu;
@@ -1256,12 +1286,20 @@ __global__ void __launch_bounds__(256, RT_MIN_BLOCKS) k_render_stream_trav(const
           skip = pixstate_load(R.pixstate, (size_t)j * cam.width + i, color.x, color.y, color.z, sum_ill, sum_ill2, samples, bounces_sum) != 0;
           samples0 = samples; bounces0 = bounces_sum;
         }
+        if constexpr (RESUME) {
+          if (!skip && R.moments) { const V3 m2 = moments_m2_load(R.moments, (size_t)j * cam.width + i); m2x = m2.x; m2y = m2.y; m2z = m2.z; }
+        }
         if (skip) have_px = false;
         else if (cam.samples <= 0) finish_pixel(true); // while (0 < 0): the pixel gets no sample at all
         else { st = ST_BEGIN; fresh = true; }
       }
     }
-    if (__all_sync(full, st == ST_NONE && !have_px)) break; // stream exhausted and every pixel written
+    if (__all_sync(full, st == ST_NONE && !have_px)) {
+      if constexpr (RESUME) {
+        if (!(queue_empty && cursor >= 32)) continue; // every pixel taken had stopped in an earlier pass: take more
+      }
+      break; // stream exhausted and every pixel written
+    }
 
     // ---- shading phase: finish the bounce of lanes whose ray is done, start the next bounce / sample ----
     if (st == ST_HIT) {
@@ -1303,6 +1341,12 @@ __global__ void __launch_bounds__(256, RT_MIN_BLOCKS) k_render_stream_trav(const
   }
   flush_stats_range(R, t_pixels, t_smin, t_smax, t_samples, t_bounces, wc.rays, t_bmin, t_bmax);
   flush_work(R, wc);
+}
+__global__ void __launch_bounds__(256, RT_MIN_BLOCKS) k_render_stream_trav(const DevScene S, const RenderParams R) {
+  render_stream_trav<false>(S, R);
+}
+__global__ void __launch_bounds__(256, RT_MIN_BLOCKS) k_render_stream_trav_resume(const DevScene S, const RenderParams R) {
+  render_stream_trav<true>(S, R);
 }
 
 // =========================================================================================
@@ -1635,6 +1679,14 @@ static cudaError_t launch_persistent(K kernel, const DevScene& S, const RenderPa
   return cudaGetLastError();
 }
 
+// A later progressive pass picks pixels up from R.pixstate: the _resume kernels (see render_stream).
+static bool stream_resumes(const RenderParams& R) { return R.pixstate && R.s0 > 0; }
+template <int KIND, bool SHADOW = false>
+static cudaError_t launch_stream(const DevScene& S, const RenderParams& R, long long tiles, int sms, cudaStream_t st) {
+  if (stream_resumes(R)) return launch_persistent(k_render_stream_resume<KIND, SHADOW>, S, R, tiles, sms, st);
+  return launch_persistent(k_render_stream<KIND, SHADOW>, S, R, tiles, sms, st);
+}
+
 cudaError_t launch_render_mega(const DevScene& S, const RenderParams& R, int sms, cudaStream_t st) {
   if (R.x1 <= R.x0 || R.y1 <= R.y0) return cudaSuccess;
   const long long tiles = (long long)R.tiles_x * R.tiles_y;
@@ -1644,9 +1696,9 @@ cudaError_t launch_render_mega(const DevScene& S, const RenderParams& R, int sms
     static const bool no_stream_trav = getenv("RT_B200_NO_STREAM_TRAV") != nullptr; // development switch
     if (S.cam.shadow_rays) { // whole-query walks for every tree size: the shadow ray is traced inside the shading step
       switch (S.bvh_kind) {
-        case BVH_LIST: return launch_persistent(k_render_stream<BVH_LIST, true>, S, R, tiles, sms, st);
-        case BVH_SAH: return launch_persistent(k_render_stream<BVH_SAH, true>, S, R, tiles, sms, st);
-        default: return launch_persistent(k_render_stream<BVH_REFERENCE, true>, S, R, tiles, sms, st);
+        case BVH_LIST: return launch_stream<BVH_LIST, true>(S, R, tiles, sms, st);
+        case BVH_SAH: return launch_stream<BVH_SAH, true>(S, R, tiles, sms, st);
+        default: return launch_stream<BVH_REFERENCE, true>(S, R, tiles, sms, st);
       }
     }
     if (R.ad_blocks > 0) { // chosen by render_adaptive_blocks (rt_api.cu sizes adstate / adrec from it)
@@ -1657,11 +1709,12 @@ cudaError_t launch_render_mega(const DevScene& S, const RenderParams& R, int sms
       }
     }
     switch (S.bvh_kind) {
-      case BVH_LIST: return launch_persistent(k_render_stream<BVH_LIST>, S, R, tiles, sms, st);
+      case BVH_LIST: return launch_stream<BVH_LIST>(S, R, tiles, sms, st);
       case BVH_SAH:
-        if (S.n_nodes >= kTravNodes && !no_stream_trav) return launch_persistent(k_render_stream_trav, S, R, tiles, sms, st);
-        return launch_persistent(k_render_stream<BVH_SAH>, S, R, tiles, sms, st);
-      default: return launch_persistent(k_render_stream<BVH_REFERENCE>, S, R, tiles, sms, st);
+        if (S.n_nodes >= kTravNodes && !no_stream_trav)
+          return launch_persistent(stream_resumes(R) ? k_render_stream_trav_resume : k_render_stream_trav, S, R, tiles, sms, st);
+        return launch_stream<BVH_SAH>(S, R, tiles, sms, st);
+      default: return launch_stream<BVH_REFERENCE>(S, R, tiles, sms, st);
     }
   }
   // a tile = 8 warp blocks and a CTA runs 8 warps: `tiles * chunks` CTAs' worth of warp items

@@ -25,7 +25,9 @@ def sass(lib):
     out = subprocess.run(["cuobjdump", "-sass", str(lib)], capture_output=True, text=True, check=True).stdout
     funcs, ident, cur = {}, "", None
     for line in out.splitlines():
-        if line.startswith("identifier = "):
+        if line.startswith("Fatbin "):  # the next ELF's header (it may carry a "compressed" line): no function's code
+            cur = None
+        elif line.startswith("identifier = "):
             ident, cur = line[len("identifier = "):].strip(), None
         elif line.strip().startswith("Function : "):
             key = (ident, line.split("Function : ", 1)[1].strip())
