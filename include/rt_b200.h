@@ -244,6 +244,11 @@ typedef int32_t (*rt_progress_fn)(void* user, int32_t pass, int32_t n_passes, in
 rt_status rt_camera_render_progressive(rt_camera* cam, const rt_region* region, uint8_t* rgb8, size_t rgb8_len,
                                        float* linear_rgb, int32_t n_passes, rt_progress_fn on_pass, void* user,
                                        rt_stats* stats);
+/* Host-only: the sample cap of each of the n_passes passes of every progressive call, for a camera of `samples` per pixel
+ * and `batch` = aBatch when it samples adaptively, 1 otherwise.  caps[k - 1] = the cap passed to on_pass after pass k, or
+ * -1 for a pass with no new samples, which the calls skip (more passes than samples).  Returns the number of passes that
+ * run, or -1 for samples < 0, batch < 1, n_passes < 1 or a null `caps`. */
+int32_t rt_progressive_caps(int32_t samples, int32_t batch, int32_t n_passes, int32_t* caps);
 
 /* ---- parity hook: primary visibility through pixel centres (getRay with no jitter and
  * no defocus, src/camera.ts:176-196) + closest hit over (0.001, inf) (src/camera.ts:249).
@@ -327,6 +332,28 @@ rt_status rt_multi_render_region(rt_multi* multi, const rt_region* region, uint8
  * Synchronous. */
 rt_status rt_multi_render_denoised(rt_multi* multi, const rt_region* region, uint8_t* rgb8, size_t rgb8_len,
                                    float* linear_rgb, const rt_denoise_opts* opts, rt_stats* stats);
+/* Progressive renders on every device.  Pass by pass, each call delivers what its one-camera counterpart
+ * (rt_camera_render_progressive, rt_camera_render_progressive_denoised) delivers on a camera with the same scene, options
+ * and region, for every n_devices and on both paths: the same caps passed to `on_pass`, bit-identical rgb8 / linear_rgb
+ * (/ moments) in the caller's buffers after each pass, and the same `so_far` stats except device_ms and kernel_launches.
+ * Pixels outside the region are never written.  Each pass renders like rt_multi_render_region (the denoised form: like
+ * rt_multi_render_denoised, with the features computed in the first pass only); every device keeps its pixels' state
+ * between the passes.  `on_pass` runs on the calling thread, once per pass, after every device's part of that pass has
+ * landed in the caller's buffers; a non-zero return stops every device after that pass.  The call returns only when no
+ * work of it is left queued on any device.  With n_passes == 1 the result equals rt_multi_render_region /
+ * rt_multi_render_denoised (rgb8, linear_rgb, stats).  Errors as the one-camera calls: RT_ERR_INVALID_ARGUMENT for a null
+ * multi, n_passes < 1 or bad denoise options, RT_ERR_BUFFER_TOO_SMALL, and RT_ERR_UNSUPPORTED from the denoised form for
+ * render modes other than RT_MODE_DEFAULT (the plain form renders every mode).  stats: device_ms = the sum over the
+ * passes of each pass's time as the one-shot multi call counts it (the plain form: the slowest device's render; the
+ * denoised form: device[0]'s span from its render to the last band); kernel_launches = the sum over devices and passes.
+ * Synchronous. */
+rt_status rt_multi_render_progressive(rt_multi* multi, const rt_region* region, uint8_t* rgb8, size_t rgb8_len,
+                                      float* linear_rgb, int32_t n_passes, rt_progress_fn on_pass, void* user,
+                                      rt_stats* stats);
+rt_status rt_multi_render_progressive_denoised(rt_multi* multi, const rt_region* region, uint8_t* rgb8, size_t rgb8_len,
+                                               float* linear_rgb, float* moments, int32_t n_passes,
+                                               const rt_denoise_opts* opts, rt_progress_fn on_pass, void* user,
+                                               rt_stats* stats);
 
 /* ---- one process PER GPU (torch.distributed ranks of one node): a device buffer every rank can write ----
  * Rank 0 creates the framebuffer and hands the 64-byte CUDA IPC handle to the other ranks (any transport);

@@ -26,7 +26,8 @@ EXPORTS = [
     "rt_shared_buffer_create", "rt_shared_buffer_open", "rt_shared_buffer_release",
     "rt_debug_scatter", "rt_debug_get_ray", "rt_debug_light_pdf", "rt_debug_light_random_vec", "rt_debug_diffuse_bounce",
     "rt_camera_render_features", "rt_denoise", "rt_camera_render_denoised", "rt_multi_render_denoised",
-    "rt_camera_render_progressive_denoised",
+    "rt_camera_render_progressive_denoised", "rt_multi_render_progressive", "rt_multi_render_progressive_denoised",
+    "rt_progressive_caps",
 ]
 
 STATUS_NAMES = {
@@ -98,6 +99,11 @@ def lib() -> C.CDLL:
     L.rt_multi_render_denoised.argtypes = [vp, C.POINTER(rt_region), vp, C.c_size_t, vp, C.POINTER(rt_denoise_opts), C.POINTER(rt_stats)]
     L.rt_camera_render_progressive_denoised.argtypes = [vp, C.POINTER(rt_region), vp, C.c_size_t, vp, vp, i32, C.POINTER(rt_denoise_opts),
                                                         vp, vp, C.POINTER(rt_stats)]
+    L.rt_multi_render_progressive.argtypes = [vp, C.POINTER(rt_region), vp, C.c_size_t, vp, i32, vp, vp, C.POINTER(rt_stats)]
+    L.rt_multi_render_progressive_denoised.argtypes = [vp, C.POINTER(rt_region), vp, C.c_size_t, vp, vp, i32, C.POINTER(rt_denoise_opts),
+                                                       vp, vp, C.POINTER(rt_stats)]
+    L.rt_progressive_caps.restype = i32
+    L.rt_progressive_caps.argtypes = [i32, i32, i32, vp]
     _lib = L
     return L
 

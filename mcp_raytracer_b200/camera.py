@@ -415,6 +415,33 @@ class MultiCamera:
         _check(_native.lib().rt_multi_render_denoised(self._h, C.byref(reg), bp, bl, lp, C.byref(opts), C.byref(st)))
         return RenderStats.from_struct(st)
 
+    def renderProgressive(self, pixelData: np.ndarray, passes: int, onPass=None, region: Optional[Dict[str, int]] = None,
+                          linear: Optional[np.ndarray] = None) -> RenderStats:
+        """`Camera.renderProgressive` on every device (rt_multi_render_progressive): the same caps, and after each pass the
+        same bytes as one Camera's.  onPass runs once per pass, after every device's part of it has landed."""
+        W, H = self.imageWidth, self.imageHeight
+        bp, bl, lp = _image_outputs(pixelData, linear, W, H)
+        reg = _region_struct(region, W, H)
+        st = rt_stats()
+        _progressive(onPass, lambda fn: _native.lib().rt_multi_render_progressive(self._h, C.byref(reg), bp, bl, lp, int(passes), fn,
+                                                                                  None, C.byref(st)))
+        return RenderStats.from_struct(st)
+
+    def renderProgressiveDenoised(self, pixelData: Optional[np.ndarray], passes: int, onPass=None, region: Optional[Dict[str, int]] = None,
+                                  linear: Optional[np.ndarray] = None, moments: Optional[np.ndarray] = None,
+                                  options: Optional[Dict[str, Any]] = None) -> RenderStats:
+        """`Camera.renderProgressiveDenoised` on every device (rt_multi_render_progressive_denoised): after each pass the same
+        bytes as one Camera's; each device filters a band of the region's rows, as in `renderDenoised`."""
+        W, H = self.imageWidth, self.imageHeight
+        bp, bl, lp = _image_outputs(pixelData, linear, W, H)
+        mp = _moments_output(moments, W, H)
+        reg = _region_struct(region, W, H)
+        opts = denoise_opts_struct(options)
+        st = rt_stats()
+        _progressive(onPass, lambda fn: _native.lib().rt_multi_render_progressive_denoised(
+            self._h, C.byref(reg), bp, bl, lp, mp, int(passes), C.byref(opts), fn, None, C.byref(st)))
+        return RenderStats.from_struct(st)
+
 
 def createCameraFromSceneData(sceneData: Dict[str, Any], renderOptions: Optional[Dict[str, Any]] = None) -> Camera:
     """src/scenes/scenes.ts:60-104"""

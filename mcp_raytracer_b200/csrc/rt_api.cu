@@ -775,10 +775,40 @@ static rt_status denoise_features(rt_camera* c, const RenderParams& P, int b0, i
 static rt_status denoise_filter(rt_camera* c, const RenderParams& P, int b0, int b1, const DenoiseParams& opts, const float* color,
                                 const float* moments, float* out, uint8_t* rgb8, int* launches);
 
+// Partitioned camera: copy the 8x4 blocks it owns in the region of P from its rgb8 / linear / moments buffers (each
+// optional) into the caller's [H][W] arrays, through host staging of the region's rows.  Synchronises the camera's stream.
+static rt_status copy_owned_blocks(rt_camera* c, const RenderParams& P, uint8_t* rgb8, float* linear, float* moments) {
+  const int W = c->hs->image_width, rh = P.y1 - P.y0;
+  std::vector<uint8_t> hr;
+  std::vector<float> hl, hm;
+  const size_t row0 = (size_t)P.y0 * W;
+  if (rgb8) { hr.resize((size_t)rh * W * 3); CU(cudaMemcpyAsync(hr.data(), c->d_rgb8 + row0 * 3, hr.size(), cudaMemcpyDeviceToHost, c->stream)); }
+  if (linear) { hl.resize((size_t)rh * W * 3); CU(cudaMemcpyAsync(hl.data(), c->d_linear + row0 * 3, hl.size() * 4, cudaMemcpyDeviceToHost, c->stream)); }
+  if (moments) { hm.resize((size_t)rh * W * 8); CU(cudaMemcpyAsync(hm.data(), c->d_moments + row0 * 8, hm.size() * 4, cudaMemcpyDeviceToHost, c->stream)); }
+  CU(cudaStreamSynchronize(c->stream));
+  const int bpr = (W + 7) / 8;
+  for (int y = P.y0; y < P.y1; ++y) {
+    for (int x = P.x0; x < P.x1;) {
+      const int bx = x / 8;
+      const int xe = std::min(P.x1, (bx + 1) * 8);
+      if (block_owner(bx, y / 4, bpr, c->opts.part_count) == c->opts.part_index) {
+        const size_t dst = (size_t)y * W + x, src = (size_t)(y - P.y0) * W + x;
+        const size_t n = (size_t)(xe - x);
+        if (rgb8) std::memcpy(rgb8 + dst * 3, hr.data() + src * 3, n * 3);
+        if (linear) std::memcpy(linear + dst * 3, hl.data() + src * 3, n * 12);
+        if (moments) std::memcpy(moments + dst * 8, hm.data() + src * 8, n * 32);
+      }
+      x = xe;
+    }
+  }
+  return RT_OK;
+}
+
 // Render the region and copy it to the caller's [H][W] arrays.  With `dn`, the colour and moments stay on the device and
-// are filtered in place before ev1 (one band covering the region); RGB8 is written from the filtered image.
+// are filtered in place before ev1 (one band covering the region); RGB8 is written from the filtered image.  `pass`: one
+// pass of a progressive render (the host-merge path of rt_multi_render_progressive*).
 static rt_status render_host(rt_camera* c, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
-                             float* moments, rt_stats* stats, const DenoiseParams* dn = nullptr) {
+                             float* moments, rt_stats* stats, const DenoiseParams* dn = nullptr, const ProgPass* pass = nullptr) {
   RT_GUARD_BEGIN
   if (!c) return fail(RT_ERR_INVALID_ARGUMENT, "null camera");
   const int W = c->hs->image_width, H = c->hs->image_height;
@@ -799,7 +829,7 @@ static rt_status render_host(rt_camera* c, const rt_region* region, uint8_t* rgb
     denoise = [&](int* l) { return denoise_band(c, P, P.y0, P.y1, *dn, P.linear, P.moments, P.linear, rgb8 ? c->d_rgb8 : nullptr, false, l); };
   int launches = 0;
   unsigned long long raw[kStatCount];
-  if ((st = timed_render(c, P, c->ev1, raw, &launches, nullptr, denoise)) != RT_OK) return st;
+  if ((st = timed_render(c, P, c->ev1, raw, &launches, pass, denoise)) != RT_OK) return st;
   const bool whole_tiles = c->opts.part_count <= 1;
   const int rw = P.x1 - P.x0, rh = P.y1 - P.y0;
   if (rw > 0 && rh > 0) {
@@ -810,29 +840,8 @@ static rt_status render_host(rt_camera* c, const rt_region* region, uint8_t* rgb
       if (moments) CU(copy_region(moments, c->d_moments, 32, P, W, cudaMemcpyDeviceToHost, c->stream));
       CU(cudaStreamSynchronize(c->stream));
     } else {
-      // partitioned render: stage the rows, then copy only the tiles this part owns
-      std::vector<uint8_t> hr;
-      std::vector<float> hl, hm;
-      const size_t row0 = (size_t)P.y0 * W;
-      if (rgb8) { hr.resize((size_t)rh * W * 3); CU(cudaMemcpyAsync(hr.data(), c->d_rgb8 + row0 * 3, hr.size(), cudaMemcpyDeviceToHost, c->stream)); }
-      if (linear) { hl.resize((size_t)rh * W * 3); CU(cudaMemcpyAsync(hl.data(), c->d_linear + row0 * 3, hl.size() * 4, cudaMemcpyDeviceToHost, c->stream)); }
-      if (moments) { hm.resize((size_t)rh * W * 8); CU(cudaMemcpyAsync(hm.data(), c->d_moments + row0 * 8, hm.size() * 4, cudaMemcpyDeviceToHost, c->stream)); }
-      CU(cudaStreamSynchronize(c->stream));
-      const int bpr = (W + 7) / 8;
-      for (int y = P.y0; y < P.y1; ++y) {
-        for (int x = P.x0; x < P.x1;) {
-          const int bx = x / 8;
-          const int xe = std::min(P.x1, (bx + 1) * 8);
-          if (block_owner(bx, y / 4, bpr, c->opts.part_count) == c->opts.part_index) {
-            const size_t dst = (size_t)y * W + x, src = (size_t)(y - P.y0) * W + x;
-            const size_t n = (size_t)(xe - x);
-            if (rgb8) std::memcpy(rgb8 + dst * 3, hr.data() + src * 3, n * 3);
-            if (linear) std::memcpy(linear + dst * 3, hl.data() + src * 3, n * 12);
-            if (moments) std::memcpy(moments + dst * 8, hm.data() + src * 8, n * 32);
-          }
-          x = xe;
-        }
-      }
+      // partitioned render: only the blocks this part owns
+      if ((st = copy_owned_blocks(c, P, rgb8, linear, moments)) != RT_OK) return st;
     }
   } else {
     CU(cudaStreamSynchronize(c->stream));
@@ -860,6 +869,42 @@ rt_status rt_camera_render_moments(rt_camera* cam, const rt_region* region, uint
   return render_host(cam, region, rgb8, rgb8_len, linear_rgb, moments, stats);
 }
 
+// The sample cap after each of the n_passes passes of a progressive render of S samples per pixel: ceil(S k / n_passes),
+// rounded up to a multiple of `batch` before the last pass, which ends at S.  The pixel stream stops on batch boundaries
+// only (the convergence check of camera.ts:348-368 runs there, so a pixel's decisions are those of the one-shot render):
+// `batch` is aBatch for adaptive cameras, 1 otherwise.  -1 = a pass with no new samples (more passes than samples), which
+// is skipped; with S = 0 only the last pass runs.
+static std::vector<int> pass_caps(int S, int batch, int n_passes) {
+  std::vector<int> caps((size_t)n_passes, -1);
+  int prev = 0;
+  for (int k = 1; k <= n_passes; ++k) {
+    long long cap = ((long long)S * k + n_passes - 1) / n_passes;
+    if (k < n_passes) cap = std::min<long long>(S, (cap + batch - 1) / batch * batch);
+    else cap = S;
+    if ((int)cap <= prev && !(S <= 0 && k == n_passes)) continue;
+    caps[(size_t)k - 1] = prev = (int)cap;
+  }
+  return caps;
+}
+static std::vector<int> camera_pass_caps(const rt_camera* c, int n_passes) {
+  const DevCamera& cam = c->hs->cam;
+  return pass_caps(cam.samples, cam.adaptive ? std::max(1, cam.a_batch) : 1, n_passes);
+}
+
+// Fold the stats of one pass (`ms` of device time) into the running total of a progressive render: work, launches and
+// device_ms add up.  The pixel stream (`stream`) counts a pixel in the pass that completes it; at fixed spp every pass
+// touches every pixel, and all of them have `cap` samples now.
+static void fold_pass_stats(rt_stats* total, const rt_stats& ps, double ms, bool stream, int cap) {
+  const int32_t samples_min = total->samples_min;
+  merge_stats(total, ps);
+  total->device_ms += ms;
+  if (!stream) {
+    total->pixels = ps.pixels;
+    total->samples_min = ps.pixels ? (int32_t)cap : samples_min;
+    total->samples_max = ps.pixels ? (int32_t)cap : 0;
+  }
+}
+
 // Progressive render: the same image as rt_camera_render_region, delivered in n_passes growing prefixes of the samples.
 // With `dn`, every pass also renders the moments and filters the region into d_dnout (see rt_camera_render_progressive_denoised);
 // `moments` (host, optional) receives them after each pass.
@@ -885,16 +930,12 @@ static rt_status progressive_host(rt_camera* c, const rt_region* region, uint8_t
   // moments run the pixel stream at fixed spp too (render_needs_full), which counts a pixel in the pass that completes it.
   // At fixed spp both rules give the same totals (no pixel completes before the last pass), so no test can tell them apart.
   const bool stream = c->hs->cam.adaptive || c->hs->cam.mode != 0 || with_moments;
-  const int batch = c->hs->cam.adaptive ? std::max(1, c->hs->cam.a_batch) : 1;
+  const std::vector<int> caps = camera_pass_caps(c, n_passes);
   rt_stats total = unpack_stats(kStatsInit);
   int prev = 0, passes_run = 0;
   for (int k = 1; k <= n_passes; ++k) {
-    // prefix of the samples after pass k; the pixel stream stops on batch boundaries only (the convergence check of
-    // camera.ts:348-368 runs there, so a pixel's decisions are those of the one-shot render)
-    long long cap = ((long long)S * k + n_passes - 1) / n_passes;
-    if (k < n_passes) cap = std::min<long long>(S, (cap + batch - 1) / batch * batch);
-    else cap = S;
-    if ((int)cap <= prev && !(S <= 0 && k == n_passes)) continue; // nothing new in this pass (more passes than samples)
+    const int cap = caps[(size_t)k - 1];
+    if (cap < 0) continue;
     RenderParams P = P0;
     P.rgb8 = rgb8 && !dn ? c->d_rgb8 : nullptr;
     P.linear = linear || dn ? c->d_linear : nullptr;
@@ -915,7 +956,7 @@ static rt_status progressive_host(rt_camera* c, const rt_region* region, uint8_t
         *l += lf;
         return s;
       };
-    const ProgPass pass{prev, (int)cap, first};
+    const ProgPass pass{prev, cap, first};
     int launches = 0;
     unsigned long long raw[kStatCount];
     st = timed_render(c, P, c->ev1, raw, &launches, (S > 0 && n_passes > 1) ? &pass : nullptr, denoise);
@@ -928,16 +969,8 @@ static rt_status progressive_host(rt_camera* c, const rt_region* region, uint8_t
     ps.kernel_launches = launches;
     float ms = 0;
     CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-    // over the passes: device_ms adds up; a pixel is counted by the pass that completes it
-    const int32_t samples_min = total.samples_min;
-    merge_stats(&total, ps);
-    total.device_ms += ms;
-    if (!stream) { // fixed spp: every pass touches every pixel; all of them have `cap` samples now
-      total.pixels = ps.pixels;
-      total.samples_min = ps.pixels ? (int32_t)cap : samples_min;
-      total.samples_max = ps.pixels ? (int32_t)cap : 0;
-    }
-    prev = (int)cap;
+    fold_pass_stats(&total, ps, ms, stream, cap);
+    prev = cap;
     ++passes_run;
     if (on_pass && on_pass(user, k, n_passes, (int32_t)cap, &total) != 0) break; // the caller has seen enough
   }
@@ -1298,9 +1331,21 @@ rt_status rt_multi_create(const rt_scene_desc* scene, const rt_render_opts* opts
         if (prev == d) { free_multi(m); return fail(RT_ERR_INVALID_ARGUMENT, "device listed twice"); }
       m->devices.push_back(d);
     }
+    // RT_B200_MULTI_PARTS=n (development switch): n parts dealt to the devices in turn, each with its own camera, stream
+    // and events, so that the partitioned passes, the cross-stream waits and both paths run with several parts on one GPU
+    if (const char* e = getenv("RT_B200_MULTI_PARTS")) {
+      const int parts = atoi(e);
+      if (parts >= 1) {
+        const std::vector<int> given = m->devices;
+        m->devices.clear();
+        for (int k = 0; k < parts; ++k) m->devices.push_back(given[(size_t)k % given.size()]);
+        n_devices = parts;
+      }
+    }
     // every device must be able to write device[0]'s memory, else the host-merge path is used
     m->p2p = true;
     for (int k = 1; k < n_devices && m->p2p; ++k) {
+      if (m->devices[k] == m->devices[0]) continue; // a part on device[0] itself needs no peer mapping
       int can = 0;
       if (cudaDeviceCanAccessPeer(&can, m->devices[k], m->devices[0]) != cudaSuccess || !can) { cudaGetLastError(); m->p2p = false; break; }
       DeviceGuard g(m->devices[k]);
@@ -1419,6 +1464,20 @@ rt_status rt_multi_render_region(rt_multi* m, const rt_region* region, uint8_t* 
   RT_GUARD_END
 }
 
+// The row bands of the denoiser on several parts: one per part, or RT_B200_DENOISE_BANDS=n (development switch) bands dealt
+// to the parts in turn, with `poison` set: their buffers are filled with NaN first (denoise_features).
+static int dn_band_count(int n_parts, bool* poison) {
+  const char* e = getenv("RT_B200_DENOISE_BANDS");
+  *poison = e && atoi(e) >= 1;
+  return *poison ? atoi(e) : n_parts;
+}
+// Band b of n_bands: contiguous rows [b0, b1) of the region of P; some bands are empty when the region has fewer rows.
+static void band_rows(const RenderParams& P, int b, int n_bands, int& b0, int& b1) {
+  const int rh = P.y1 - P.y0;
+  b0 = P.y0 + (int)((long long)b * rh / n_bands);
+  b1 = P.y0 + (int)((long long)(b + 1) * rh / n_bands);
+}
+
 // Denoised render on every device (include/rt_b200.h).  Peer-write path: every device renders its blocks' colour and
 // moments straight into device 0's d_color / d_moments, then, after every device's render, filters its band of the
 // region's rows (dn_halo's ghost zones, recomputed instead of exchanged) with prepare reading the colour and moments over
@@ -1443,14 +1502,9 @@ rt_status rt_multi_render_denoised(rt_multi* m, const rt_region* region, uint8_t
   st = clip_region(c0, region, P0);
   if (st != RT_OK) return st;
   const int rw = P0.x1 - P0.x0, rh = P0.y1 - P0.y0;
-  int n_bands = n;
-  const char* bands_env = getenv("RT_B200_DENOISE_BANDS");
-  const bool poison = bands_env && atoi(bands_env) >= 1;
-  if (poison) n_bands = atoi(bands_env);
-  auto band = [&](int b, int& b0, int& b1) { // contiguous rows; some bands are empty when the region has fewer rows
-    b0 = P0.y0 + (int)((long long)b * rh / n_bands);
-    b1 = P0.y0 + (int)((long long)(b + 1) * rh / n_bands);
-  };
+  bool poison = false;
+  const int n_bands = dn_band_count(n, &poison);
+  auto band = [&](int b, int& b0, int& b1) { band_rows(P0, b, n_bands, b0, b1); };
   {
     DeviceGuard g0(m->devices[0]);
     if (!m->d_color) CU(dev_alloc(&m->d_color, npx * 3 * sizeof(float)));
@@ -1542,6 +1596,210 @@ rt_status rt_multi_render_denoised(rt_multi* m, const rt_region* region, uint8_t
   CU(cudaStreamSynchronize(c0->stream));
   return RT_OK;
   RT_GUARD_END
+}
+
+} // extern "C"
+
+// Progressive render on every device (rt_multi_render_progressive*, include/rt_b200.h): the passes and caps of
+// progressive_host, each pass rendered, filtered (`dn`) and delivered the way rt_multi_render_region and
+// rt_multi_render_denoised deliver a one-shot call.  Each camera keeps its PixelStats and fixed-point sums in its own
+// memory between the passes.  With `dn` the features are computed in the first pass only, and the filter never writes
+// the colour it reads (d_color, or the host-merge path's upload of it): a pixel that converged in an earlier pass is not
+// rendered again, and its noisy colour must survive for the next pass's filter.
+// Ordering between passes: pass k+1's render on any device writes colour rows that other devices' pass-k band filters
+// read (the halos), and framebuffer rows that device 0's pass-k copy reads.  This relies on the host synchronisation that
+// precedes on_pass: device 0's stream waits on every device's `done` event, recorded after that device's last kernel of
+// the pass (the host-merge path synchronises every device's stream), and the host enqueues pass k+1 only after
+// cudaStreamSynchronize of that stream has returned.
+static rt_status multi_progressive(rt_multi* m, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
+                                   float* moments, int32_t n_passes, rt_progress_fn on_pass, void* user, rt_stats* stats,
+                                   const DenoiseParams* dn) {
+  const int n = (int)m->cams.size();
+  rt_camera* c0 = m->cams[0];
+  const int W = c0->hs->image_width, H = c0->hs->image_height;
+  const size_t npx = (size_t)W * H;
+  if (rgb8 && rgb8_len < npx * 3) return fail(RT_ERR_BUFFER_TOO_SMALL, "rgb8 buffer smaller than width*height*3");
+  if (dn && c0->hs->cam.mode != RT_MODE_DEFAULT) return fail(RT_ERR_UNSUPPORTED, "denoised renders need the default render mode");
+  RenderParams P0;
+  rt_status st = clip_region(c0, region, P0);
+  if (st != RT_OK) return st;
+  const bool filter = dn && P0.x1 > P0.x0 && P0.y1 > P0.y0;
+  const bool host_merge = !m->p2p && n > 1;
+  bool poison = false;
+  const int n_bands = dn_band_count(n, &poison);
+  {
+    DeviceGuard g0(m->devices[0]);
+    if (dn && !m->d_color) CU(dev_alloc(&m->d_color, npx * 3 * sizeof(float)));
+    if (dn && !m->d_moments) CU(dev_alloc(&m->d_moments, npx * 8 * sizeof(float)));
+    if ((dn || (linear && !host_merge)) && !m->d_linear) CU(dev_alloc(&m->d_linear, npx * 3 * sizeof(float)));
+    if (rgb8 && (dn || !host_merge) && !m->d_rgb8) CU(dev_alloc(&m->d_rgb8, npx * 3));
+  }
+  uint8_t* out8 = rgb8 ? m->d_rgb8 : nullptr;
+  // Features (first pass) and filter of every band, band b on cams[b % parts].  With the switch's poison, a part's
+  // buffers are filled with NaN before its first band's features only: its later passes filter every band on them.
+  auto filter_bands = [&](int parts, bool first, int* launches) -> rt_status {
+    for (int b = 0; first && b < n_bands; ++b) {
+      rt_camera* c = m->cams[b % parts];
+      DeviceGuard g(c->device);
+      int b0, b1, l = 0;
+      band_rows(P0, b, n_bands, b0, b1);
+      rt_status s = denoise_features(c, P0, b0, b1, dn->iterations, poison && b < parts, &l);
+      if (s != RT_OK) return s;
+      *launches += l;
+    }
+    for (int b = 0; b < n_bands; ++b) {
+      rt_camera* c = m->cams[b % parts];
+      DeviceGuard g(c->device);
+      int b0, b1, l = 0;
+      band_rows(P0, b, n_bands, b0, b1);
+      rt_status s = denoise_filter(c, P0, b0, b1, *dn, m->d_color, m->d_moments, m->d_linear, out8, &l);
+      if (s != RT_OK) return s;
+      *launches += l;
+    }
+    return RT_OK;
+  };
+  // host merge, denoised: every device's blocks of the colour and moments, uploaded to device 0 for the filter
+  std::vector<float> hc, hm;
+  float* h_mom = moments;
+  if (dn && host_merge) {
+    hc.resize(npx * 3);
+    if (!h_mom) { hm.resize(npx * 8); h_mom = hm.data(); }
+  }
+  const int S = c0->hs->cam.samples;
+  const bool stream = c0->hs->cam.adaptive || c0->hs->cam.mode != 0 || dn; // as progressive_host
+  const std::vector<int> caps = camera_pass_caps(c0, n_passes);
+  rt_stats total = unpack_stats(kStatsInit);
+  int prev = 0;
+  bool first = true;
+  for (int k = 1; k <= n_passes; ++k) {
+    const int cap = caps[(size_t)k - 1];
+    if (cap < 0) continue;
+    const ProgPass pass{prev, cap, first};
+    const ProgPass* pp = (S > 0 && n_passes > 1) ? &pass : nullptr;
+    rt_stats ps;
+    double ms = 0;
+    int launches = 0;
+    if (host_merge) {
+      std::vector<rt_stats> dev((size_t)n);
+      st = on_every_device(n, [&](int j) {
+        return dn ? render_host(m->cams[j], region, nullptr, 0, hc.data(), h_mom, &dev[j], nullptr, pp)
+                  : render_host(m->cams[j], region, rgb8, rgb8_len, linear, nullptr, &dev[j], nullptr, pp);
+      });
+      if (st != RT_OK) return st;
+      ps = merge_host_stats(dev);
+      ms = ps.device_ms; // the slowest device
+      launches = ps.kernel_launches;
+      if (dn) { // device 0 filters the region
+        DeviceGuard g0(m->devices[0]);
+        CU(cudaEventRecord(c0->ev0, c0->stream));
+        if (filter) {
+          CU(copy_region(m->d_color, hc.data(), 12, P0, W, cudaMemcpyHostToDevice, c0->stream));
+          CU(copy_region(m->d_moments, h_mom, 32, P0, W, cudaMemcpyHostToDevice, c0->stream));
+          if ((st = filter_bands(1, first, &launches)) != RT_OK) return st;
+        }
+        CU(cudaEventRecord(c0->ev1, c0->stream));
+        if (rgb8) CU(copy_region(rgb8, m->d_rgb8, 3, P0, W, cudaMemcpyDeviceToHost, c0->stream));
+        if (linear) CU(copy_region(linear, m->d_linear, 12, P0, W, cudaMemcpyDeviceToHost, c0->stream));
+        CU(cudaStreamSynchronize(c0->stream));
+        float f = 0;
+        CU(cudaEventElapsedTime(&f, c0->ev0, c0->ev1));
+        ms += f; // the slowest render, then the upload and the filter
+      }
+    } else {
+      // ---- peer-write path: every device writes its blocks into device 0's buffers ----
+      for (int j = 0; j < n; ++j) {
+        rt_camera* c = m->cams[j];
+        DeviceGuard g(c->device);
+        RenderParams P;
+        if ((st = clip_region(c, region, P)) != RT_OK) return st;
+        P.rgb8 = rgb8 && !dn ? m->d_rgb8 : nullptr; // the denoised form writes RGB8 from the filtered image
+        P.linear = dn ? m->d_color : linear ? m->d_linear : nullptr;
+        P.moments = dn ? m->d_moments : nullptr;
+        int l = 0;
+        if ((st = timed_render(c, P, dn ? m->rendered[j] : c->ev1, m->h_stats + (size_t)j * kStatCount, &l, pp)) != RT_OK) return st;
+        launches += l;
+        if (!dn) CU(cudaEventRecord(m->done[j], c->stream));
+      }
+      if (dn) {
+        if (filter) {
+          for (int j = 0; j < n; ++j) { // a band's passes read rows other devices rendered
+            DeviceGuard g(m->cams[j]->device);
+            for (int i = 0; i < n; ++i)
+              if (i != j) CU(cudaStreamWaitEvent(m->cams[j]->stream, m->rendered[i], 0));
+          }
+          if ((st = filter_bands(n, first, &launches)) != RT_OK) return st;
+        }
+        for (int j = 1; j < n; ++j) {
+          DeviceGuard g(m->cams[j]->device);
+          CU(cudaEventRecord(m->done[j], m->cams[j]->stream));
+        }
+      }
+      DeviceGuard g0(m->devices[0]);
+      for (int j = 1; j < n; ++j) CU(cudaStreamWaitEvent(c0->stream, m->done[j], 0)); // every device's part of the pass has landed
+      if (dn) CU(cudaEventRecord(c0->ev1, c0->stream));
+      if (rgb8) CU(copy_region(rgb8, m->d_rgb8, 3, P0, W, cudaMemcpyDeviceToHost, c0->stream));
+      if (linear) CU(copy_region(linear, m->d_linear, 12, P0, W, cudaMemcpyDeviceToHost, c0->stream));
+      if (moments) CU(copy_region(moments, m->d_moments, 32, P0, W, cudaMemcpyDeviceToHost, c0->stream));
+      CU(cudaStreamSynchronize(c0->stream));
+      if (dn) { // device 0, from its render to the last band's last kernel
+        float f = 0;
+        CU(cudaEventElapsedTime(&f, c0->ev0, c0->ev1));
+        ms = f;
+      } else { // the slowest device
+        for (int j = 0; j < n; ++j) {
+          DeviceGuard g(m->cams[j]->device);
+          float f = 0;
+          CU(cudaEventElapsedTime(&f, m->cams[j]->ev0, m->cams[j]->ev1));
+          ms = std::max(ms, (double)f);
+        }
+      }
+      ps = merge_raw_stats(m);
+    }
+    ps.kernel_launches = launches;
+    fold_pass_stats(&total, ps, ms, stream, cap);
+    prev = cap;
+    first = false;
+    if (on_pass && on_pass(user, k, n_passes, (int32_t)cap, &total) != 0) break; // every device stops after this pass
+  }
+  if (stats) *stats = total;
+  return RT_OK;
+}
+
+extern "C" {
+
+rt_status rt_multi_render_progressive(rt_multi* m, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
+                                      int32_t n_passes, rt_progress_fn on_pass, void* user, rt_stats* stats) {
+  RT_GUARD_BEGIN
+  if (!m || m->cams.empty()) return fail(RT_ERR_INVALID_ARGUMENT, "null argument");
+  if (n_passes < 1) return fail(RT_ERR_INVALID_ARGUMENT, "n_passes must be >= 1");
+  return multi_progressive(m, region, rgb8, rgb8_len, linear, nullptr, n_passes, on_pass, user, stats, nullptr);
+  RT_GUARD_END
+}
+
+rt_status rt_multi_render_progressive_denoised(rt_multi* m, const rt_region* region, uint8_t* rgb8, size_t rgb8_len, float* linear,
+                                               float* moments, int32_t n_passes, const rt_denoise_opts* opts, rt_progress_fn on_pass,
+                                               void* user, rt_stats* stats) {
+  RT_GUARD_BEGIN
+  if (!m || m->cams.empty()) return fail(RT_ERR_INVALID_ARGUMENT, "null argument");
+  if (n_passes < 1) return fail(RT_ERR_INVALID_ARGUMENT, "n_passes must be >= 1");
+  DenoiseParams D{};
+  rt_status st = dn_options(opts, D);
+  if (st != RT_OK) return st;
+  return multi_progressive(m, region, rgb8, rgb8_len, linear, moments, n_passes, on_pass, user, stats, &D);
+  RT_GUARD_END
+}
+
+int32_t rt_progressive_caps(int32_t samples, int32_t batch, int32_t n_passes, int32_t* caps) {
+  if (samples < 0 || batch < 1 || n_passes < 1 || !caps) return -1;
+  try {
+    const std::vector<int> v = pass_caps(samples, batch, n_passes);
+    int32_t run = 0;
+    for (int k = 0; k < n_passes; ++k) {
+      caps[k] = v[(size_t)k];
+      run += v[(size_t)k] >= 0;
+    }
+    return run;
+  } catch (const std::exception&) { return -1; }
 }
 
 // ---- framebuffer shared between the one-process-per-GPU ranks of a node (CUDA IPC) ----
